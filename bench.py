@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on BASELINE.json's config.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric: audio-seconds rendered per wall-second ("x realtime") of the batched single-band STFT
@@ -11,6 +11,10 @@ pre-quant -> wavefold -> post-quant -> limiter, quantize_mode="spectral_bins").
 One "step" = one render of the whole per-GPU batch.  `value` is timed with the batch already in
 HBM; `e2e` is the same render through the public API (`process_batch`) from pinned HOST buffers,
 host<->device copies inside the timed region.  One JSON line is printed by rank 0.
+
+--dump-outputs DIR writes what the last timed step returned, as DIR/y.npy (float32 [clips, samples]): the rendered
+clips of a fixed, seeded sample of DUMP_CLIPS clips of rank 0's batch (61 MB).  The inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -23,6 +27,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it
 
 SR = 48000
 CLIP_SECONDS = 10
@@ -33,6 +38,7 @@ WORKLOAD_MB = "configs[2]: 4096 synthetic 10 s mono clips/GPU, multiband: LR4 cr
 RENDER_KW = {"quantize_mode": "spectral_bins"}   # process_audio keyword arguments of the selected workload (the STFT path)
 METRIC = "audio-seconds/sec for batched STFT quantize+distort pipeline"
 UNIT = "audio-s/s"
+DUMP_CLIPS = 32
 
 
 def _peaks():
@@ -243,6 +249,15 @@ def other_configs(qd, x, clips: int):
     return out
 
 
+def dump_outputs(out_dir: str, y) -> None:
+    """DIR/y.npy: the rendered clips of a fixed, seeded sample of the batch, in ascending clip order."""
+    import numpy as np
+    import torch
+    clips = np.sort(np.random.default_rng(0).choice(y.shape[0], min(DUMP_CLIPS, y.shape[0]), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "y.npy"), y[torch.from_numpy(clips).to(y.device)].cpu().numpy())
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -298,6 +313,8 @@ def run_ours(args):
     barrier()
     ms_dev = max_over_ranks(ev0.elapsed_time(ev1)) / args.steps
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, y)
     timing = r.read_timing()
     launches = sum(v["launches"] for v in timing.values())
     audio_s = B * CLIP_SECONDS * world
@@ -546,7 +563,11 @@ def main():
     ap.add_argument("--other-clips", type=int, default=1024, help="clips for the device-resident numbers of the other BASELINE configs (0 = skip)")
     ap.add_argument("--workload", default="single_band", choices=["single_band", "multiband"],
                     help="single_band = BASELINE configs[1] (the bench line); multiband = configs[2], for the record")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help=f"write the last timed step's output (a seeded sample of {DUMP_CLIPS} clips) to DIR/y.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.workload == "multiband":
         global WORKLOAD
         WORKLOAD = WORKLOAD_MB

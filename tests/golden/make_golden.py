@@ -53,7 +53,7 @@ def gen_pipeline():
         out[f"{name}/pre_quant"] = taps["pre_quant"].astype(np.float32)
         out[f"{name}/post_dist"] = taps["post_dist"].astype(np.float32)
         print(f"pipeline {name}: n={n} peak={np.max(np.abs(y)):.4f}")
-    np.savez_compressed(os.path.join(HERE, "pipeline.npz"), **out)
+    qd_cases.save_golden("pipeline", out)
 
 
 def gen_tables():
@@ -73,7 +73,7 @@ def gen_tables():
         out[f"htb/{f0}"] = ref_q.build_harmonic_target_bins(freqs, f0).astype(np.int64)
     # reference KAT (tests/test_quantizer.py:10-23)
     out["tb/kat4"] = ref_q.build_target_bins_for_freqs(np.array([0.0, 430.0, 440.0, 450.0]), "A", "minor")
-    np.savez_compressed(os.path.join(HERE, "tables.npz"), **out)
+    qd_cases.save_golden("tables", out)
     print("tables:", len(out))
 
 
@@ -86,7 +86,7 @@ def gen_analysis():
         avg, per = avg_cents_offset_from_scale(x, sr, key, scale, **kw)
         out[f"{name}/x"], out[f"{name}/avg"], out[f"{name}/per_peak"] = x, np.float64(avg), per
         print(f"analysis {name}: avg {avg:.3f} cents over {len(per)} peaks")
-    np.savez_compressed(os.path.join(HERE, "analysis.npz"), **out)
+    qd_cases.save_golden("analysis", out)
 
 
 def gen_autotune():
@@ -120,7 +120,7 @@ def gen_autotune():
         out[f"{name}/x"], out[f"{name}/y"] = xx, y
         out[f"{name}/pre_quant"], out[f"{name}/post_dist"] = taps["pre_quant"].astype(np.float32), taps["post_dist"].astype(np.float32)
         print(f"autotune {name}: n={n} peak={np.max(np.abs(y)):.4f} moved={np.max(np.abs(y - xx)):.4f}")
-    np.savez_compressed(os.path.join(HERE, "autotune.npz"), **out)
+    qd_cases.save_golden("autotune", out)
 
 
 def gen_stages():
@@ -194,7 +194,7 @@ def gen_stages():
     sl, sh = design_linkwitz_riley_sos(sr, 300.0)
     out["td/xo/sos_low"], out["td/xo/sos_high"] = sl, sh
     out["td/sat"] = saturate_lowband(lo, drive=2.5)
-    np.savez_compressed(os.path.join(HERE, "stages.npz"), **out)
+    qd_cases.save_golden("stages", out)
     print("stages:", len(out))
 
 
@@ -206,7 +206,7 @@ def gen_frontend():
         y, taps = quiet(ref_pipeline.process_audio, x, sr, quantize_mode="spectral_bins", config=cfg, **kw)
         out[f"{name}/x"], out[f"{name}/y"] = x, y
         print(f"ui {name}: peak={np.max(np.abs(y)):.4f}")
-    np.savez_compressed(os.path.join(HERE, "frontend.npz"), **out)
+    qd_cases.save_golden("frontend", out)
 
 
 def _run_case(x, sr, n_fft, rng_seed, kw, mode="spectral_bins"):
@@ -274,7 +274,7 @@ def gen_round2():
         m, ph = ref_fx.phase_dispersal(np.ones(1025), np.zeros(1025), thresh=0.0, amount=0.0, randomized=True, rand_amt=1.0)
         jit.append(ph)
     out["scr/1025/jitter"] = np.array(jit)
-    np.savez_compressed(os.path.join(HERE, "round2.npz"), **out)
+    qd_cases.save_golden("round2", out)
     print("round2:", len(out), os.path.getsize(os.path.join(HERE, "round2.npz")) // 1024, "KiB")
 
 
@@ -300,7 +300,9 @@ def gen_refwav():
                 sr2, k = wavfile.read(pth)
                 assert sr2 == sr and k.dtype == np.int16
                 out[f"{name}/kat_{suffix}"] = k
-    np.savez_compressed(os.path.join(HERE, "refwav.npz"), **out)
+    inputs = {k: v for k, v in out.items() if k.endswith(("/x16", "/sr"))}
+    qd_cases.save_golden("refwav", inputs)
+    qd_cases.save_golden("refwav_renders", {k: v for k, v in out.items() if k not in inputs})
     print("refwav:", len(out), os.path.getsize(os.path.join(HERE, "refwav.npz")) // 1024, "KiB")
 
 
@@ -319,7 +321,7 @@ def gen_scenarios():
         out[f"{name}/pre_quant"] = np.asarray(taps["pre_quant"], dtype=np.float32)
         out[f"{name}/post_dist"] = np.asarray(taps["post_dist"], dtype=np.float32)
         print(f"scenario {name} ({cite}): n={len(x)} peak={np.max(np.abs(y)):.4f} moved={np.max(np.abs(y - x[:len(y)])):.4f}")
-    np.savez_compressed(os.path.join(HERE, "scenarios.npz"), **out)
+    qd_cases.save_golden("scenarios", out)
     print("scenarios:", len(out), os.path.getsize(os.path.join(HERE, "scenarios.npz")) // 1024, "KiB")
 
 
@@ -379,7 +381,7 @@ def gen_scripts():
             assert sr2 == sr and y16.dtype == np.int16 and y16.shape == x16.shape
             out[f"{name}/y16"] = y16
             print(f"harness {name} ({cite}): n={len(x16)} peak={np.max(np.abs(y16.astype(np.int32)))}")
-    np.savez_compressed(os.path.join(HERE, "scripts.npz"), **out)
+    qd_cases.save_golden("scripts", out)
     print("scripts:", len(out), os.path.getsize(os.path.join(HERE, "scripts.npz")) // 1024, "KiB")
 
 

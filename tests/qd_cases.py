@@ -5,9 +5,101 @@ process_audio).  quantize_mode="spectral_bins" is always passed (SURVEY.md secti
 """
 from __future__ import annotations
 
+import fnmatch
+import hashlib
 import os
 
 import numpy as np
+
+GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+# ---------------------------------------------------------------- fixture files (tests/golden/*.npz)
+# Whole renders of every case would make the fixtures tens of megabytes.  An array larger than GOLDEN_SAMPLE elements is
+# therefore stored as the SHA-256 digest of the whole array (exact comparisons stay exact) plus its values at
+# GOLDEN_SAMPLE fixed positions drawn with a seed (toleranced comparisons); the positions are stored too, one set per
+# array size.  Arrays the tests feed back into the code as inputs are kept whole (GOLDEN_WHOLE).
+GOLDEN_SAMPLE = 1024
+GOLDEN_WHOLE = {
+    "tables": ("*",),
+    "refwav": ("*",),                                     # the reference's own WAV files: cannot be regenerated
+    "stages": ("q/mags", "q/phases", "fx/mag", "fx/phase", "fx/formant/zeros_in", "fx/formant/in257", "stft/x", "td/*"),
+    "autotune": ("st/x", "st/body", "st/det", "st/ratio_track", "st/ratio_manual"),
+    "round2": ("scr/*",),
+    "pipeline": ("sb_wide_mask/post_dist",),
+    "scenarios": ("formant_six/*",),
+}
+
+
+def _digest(a: np.ndarray) -> str:
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+def save_golden(name: str, arrays: dict) -> str:
+    """Write tests/golden/<name>.npz in the form Golden reads."""
+    whole = GOLDEN_WHOLE.get(name, ())
+    out = {}
+    for key, a in arrays.items():
+        a = np.asarray(a)
+        if a.size <= GOLDEN_SAMPLE or any(fnmatch.fnmatchcase(key, p) for p in whole):
+            out[key] = a
+            continue
+        ik = f"#idx/{a.size}"
+        if ik not in out:
+            out[ik] = np.sort(np.random.default_rng(a.size).choice(a.size, GOLDEN_SAMPLE, replace=False)).astype(np.uint32)
+        out[f"{key}#sha"] = np.array(_digest(a))
+        out[f"{key}#shape"] = np.array(a.shape, dtype=np.int64)
+        out[f"{key}#v"] = a.reshape(-1)[out[ik]]
+    path = os.path.join(GOLDEN_DIR, f"{name}.npz")
+    np.savez_compressed(path, **out)
+    return path
+
+
+class Golden:
+    """One fixture file: `g[key]` is an array stored whole; `matches` compares a whole array exactly, `at` returns the
+    values to compare at the stored positions."""
+
+    def __init__(self, name: str):
+        self._z = np.load(os.path.join(GOLDEN_DIR, f"{name}.npz"))
+        self._files = set(self._z.files)
+
+    def __getitem__(self, key):
+        if key not in self._files:
+            raise KeyError(f"{key} is not stored whole (use Golden.matches / Golden.at)")
+        return self._z[key]
+
+    def shape(self, key):
+        return self._z[key].shape if key in self._files else tuple(int(s) for s in self._z[f"{key}#shape"])
+
+    def matches(self, key, got) -> bool:
+        """np.array_equal(got, <the whole fixture array>)."""
+        got = np.asarray(got)
+        if key in self._files:
+            return bool(np.array_equal(got, self._z[key]))
+        v = self._z[f"{key}#v"]
+        if got.shape != self.shape(key):
+            return False
+        cast = got.astype(v.dtype)
+        return bool(np.array_equal(cast, got)) and _digest(cast) == str(self._z[f"{key}#sha"])
+
+    def at(self, key, got):
+        """(got, fixture) at the stored positions, after checking that `got` has the fixture's shape."""
+        got = np.asarray(got)
+        assert got.shape == self.shape(key), (key, got.shape, self.shape(key))
+        if key in self._files:
+            return got, self._z[key]
+        idx = self._z[f"#idx/{int(np.prod(got.shape))}"]
+        return got.reshape(-1)[idx], self._z[f"{key}#v"]
+
+    def max_abs_err(self, key, got) -> float:
+        a, b = self.at(key, got)
+        return float(np.max(np.abs(a.astype(np.result_type(a, np.float64)) - b))) if b.size else 0.0
+
+    def input(self, name, x):
+        """`x`, regenerated from its seed, after checking that it is the input of the fixture's case `name`."""
+        assert self.matches(f"{name}/x", x), f"{name}: input drifted from the fixture"
+        return x
+
 
 GROWL = dict(key="F", scale="minor", snap_strength=0.9, smear=0.3, bin_smoothing=True,
              pre_quant=True, post_quant=True, distortion_mode="wavefold",

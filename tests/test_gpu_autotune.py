@@ -1,6 +1,5 @@
 """GPU (B200): quantize_mode="autotune_v1" through the C ABI vs the live-reference fixtures (tests/golden/autotune.npz)
 and the oracle (oracle/qd_autotune.py).  Same bar as the STFT path: max abs error <= 1e-4, null <= -80 dBFS."""
-import os
 
 import numpy as np
 import pytest
@@ -9,7 +8,6 @@ import qd_cases
 from oracle import qd_autotune as at
 from oracle import qd_oracle as orc
 
-G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 MAX_ABS = 1e-4
 NULL_DB = -80.0
 
@@ -24,7 +22,7 @@ def qd():
 
 @pytest.fixture(scope="module")
 def gold():
-    return np.load(os.path.join(G, "autotune.npz"))
+    return qd_cases.Golden("autotune")
 
 
 def _check(got, ref, what, max_abs=MAX_ABS):
@@ -48,7 +46,7 @@ def test_autotune_stages_vs_reference(qd, gold):
     y, taps, dbg = r.render_device(torch.from_numpy(x[None, :]).cuda(), want_taps=True, debug=True)
     d = {k: v[0].cpu().numpy() for k, v in dbg.items()}
     for k in ("sub", "body", "air", "det"):          # float64 IIR sweeps in the reference's operation order
-        assert np.max(np.abs(d[k].astype(np.float64) - gold[f"st/{k}"])) <= 2e-7, k
+        assert gold.max_abs_err(f"st/{k}", d[k]) <= 2e-7, k
     f, gf = d["features"], gold["st/features"]
     assert f.shape == gf.shape
     assert np.allclose(f[:, 0], gf[:, 0], rtol=1e-5, atol=1e-8)            # rms (float32 mean)
@@ -60,20 +58,20 @@ def test_autotune_stages_vs_reference(qd, gold):
     assert np.allclose(f[voiced, 2], gf[voiced, 2], rtol=1e-7, atol=0.0)   # YIN pitch (float64)
     assert np.allclose(f[:, 3], gf[:, 3], rtol=0.0, atol=1e-7)
     assert np.max(np.abs(d["ratio_track"].astype(np.float64) - gold["st/ratio_track"])) <= 1e-6
-    _check(d["corrected"], gold["st/corrected"], "corrected body", 2e-5)
-    _check(d["sub_layer"], gold["st/sub_layer"], "sub layer", 2e-6)
-    _check(taps["pre_quant"][0].cpu().numpy(), gold["st/output"], "autotune output", 2e-5)
+    _check(*gold.at("st/corrected", d["corrected"]), "corrected body", 2e-5)
+    _check(*gold.at("st/sub_layer", d["sub_layer"]), "sub layer", 2e-6)
+    _check(*gold.at("st/output", taps["pre_quant"][0].cpu().numpy()), "autotune output", 2e-5)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", list(qd_cases.AUTOTUNE_CASES))
 def test_autotune_pipeline_vs_reference_fixtures(qd, gold, name):
     kind, seed, n, sr, kw = qd_cases.AUTOTUNE_CASES[name]
-    x = gold[f"{name}/x"]
+    x = gold.input(name, qd_cases.make_signal(kind, seed, n, sr))
     y, taps = qd.process_audio(x, sr, quantize_mode="autotune_v1", **kw)
-    _check(y, gold[f"{name}/y"], f"{name}/y")
-    _check(taps["pre_quant"], gold[f"{name}/pre_quant"], f"{name}/pre_quant")
-    _check(taps["post_dist"], gold[f"{name}/post_dist"], f"{name}/post_dist")
+    _check(*gold.at(f"{name}/y", y), f"{name}/y")
+    _check(*gold.at(f"{name}/pre_quant", taps["pre_quant"]), f"{name}/pre_quant")
+    _check(*gold.at(f"{name}/post_dist", taps["post_dist"]), f"{name}/post_dist")
     assert np.array_equal(taps["input"], x) and np.array_equal(taps["output"], y)
 
 

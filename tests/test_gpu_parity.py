@@ -33,7 +33,7 @@ def qd():
 
 @pytest.fixture(scope="module")
 def pipe():
-    return np.load(os.path.join(G, "pipeline.npz"))
+    return qd_cases.Golden("pipeline")
 
 
 def _check(got, ref, what, max_abs=MAX_ABS):
@@ -50,14 +50,14 @@ def _check(got, ref, what, max_abs=MAX_ABS):
 @pytest.mark.parametrize("name", list(qd_cases.CASES))
 def test_pipeline_vs_reference_fixtures(qd, pipe, name):
     kind, seed, n, sr, n_fft, rng_seed, kw = qd_cases.CASES[name]
-    x = pipe[f"{name}/x"]
+    x = pipe.input(name, qd_cases.make_signal(kind, seed, n, sr))
     if rng_seed is not None:
         np.random.seed(rng_seed)  # the random spectral FX replay the global np.random state like the reference
     y, taps = qd.process_audio(x, sr, n_fft=n_fft, **SB, **kw)
     # precision="auto": float32 kernels, except sb_wide_mask (fan-in > 64) and nfft8192, which run in float64
-    _check(y, pipe[f"{name}/y"], f"{name}/y")
-    _check(taps["pre_quant"], pipe[f"{name}/pre_quant"], f"{name}/pre_quant")
-    _check(taps["post_dist"], pipe[f"{name}/post_dist"], f"{name}/post_dist")
+    _check(*pipe.at(f"{name}/y", y), f"{name}/y")
+    _check(*pipe.at(f"{name}/pre_quant", taps["pre_quant"]), f"{name}/pre_quant")
+    _check(*pipe.at(f"{name}/post_dist", taps["post_dist"]), f"{name}/post_dist")
     assert np.array_equal(taps["input"], x) and np.array_equal(taps["output"], y)
 
 
@@ -253,9 +253,10 @@ def test_float64_kernels_vs_reference_fixtures(qd, pipe, name):
     kind, seed, n, sr, n_fft, rng_seed, kw = qd_cases.CASES[name]
     if rng_seed is not None:
         np.random.seed(rng_seed)
-    y, taps = qd.process_audio(pipe[f"{name}/x"], sr, n_fft=n_fft, precision="float64", **SB, **kw)
-    _check(y, pipe[f"{name}/y"], f"{name}/y f64", 2e-6)
-    _check(taps["pre_quant"], pipe[f"{name}/pre_quant"], f"{name}/pre_quant f64", 2e-6)
+    x = pipe.input(name, qd_cases.make_signal(kind, seed, n, sr))
+    y, taps = qd.process_audio(x, sr, n_fft=n_fft, precision="float64", **SB, **kw)
+    _check(*pipe.at(f"{name}/y", y), f"{name}/y f64", 2e-6)
+    _check(*pipe.at(f"{name}/pre_quant", taps["pre_quant"]), f"{name}/pre_quant f64", 2e-6)
 
 
 def test_auto_precision_rule():
@@ -272,11 +273,12 @@ def test_auto_precision_rule():
 @pytest.mark.parametrize("name", list(qd_cases.UI_CASES))
 def test_ui_config_dict_vs_reference_fixtures(qd, name):
     """Streamlit V2 nested config dict (dsp/pipeline.py:923-1008) through process_audio(config=...)."""
-    g = np.load(os.path.join(G, "frontend.npz"))
+    g = qd_cases.Golden("frontend")
     kind, seed, n, sr, rng_seed, cfg, kw = qd_cases.UI_CASES[name]
+    x = g.input(name, qd_cases.make_signal(kind, seed, n, sr))
     np.random.seed(rng_seed)
-    y, _ = qd.process_audio(g[f"{name}/x"], sr, config=cfg, **SB, **kw)
-    _check(y, g[f"{name}/y"], name)
+    y, _ = qd.process_audio(x, sr, config=cfg, **SB, **kw)
+    _check(*g.at(f"{name}/y", y), name)
 
 
 @pytest.mark.gpu
@@ -330,9 +332,9 @@ def test_cents_metric_vs_reference_fixtures(qd, name):
     """avg_cents_offset_from_scale (dsp/analyses.py:53-142): the peak bins come from the CUDA STFT (float64 kernels
     by default), the cents from the host table -> the reference's per-peak values bit for bit."""
     from quantumdistortion_b200 import analyses
-    g = np.load(os.path.join(G, "analysis.npz"))
+    g = qd_cases.Golden("analysis")
     kind, seed, n, sr, key, scale, kw = qd_cases.ANALYSIS_CASES[name]
-    x = g[f"{name}/x"]
+    x = g.input(name, qd_cases.make_signal(kind, seed, n, sr))
     avg, per = analyses.avg_cents_offset_from_scale(x, sr, key, scale, **kw)
     assert np.array_equal(per, g[f"{name}/per_peak"]), name
     assert avg == float(g[f"{name}/avg"])
@@ -372,11 +374,11 @@ def test_cents_metric_batch_of_renders(qd):
 def test_formant_shift_float64_kernels(qd, pipe, name):
     """precision="float64": the cepstral FFTs of the formant shift run in float64 like the rest of the pass."""
     kind, seed, n, sr, n_fft, rng_seed, kw = qd_cases.CASES[name]
-    x = pipe[f"{name}/x"]
+    x = pipe.input(name, qd_cases.make_signal(kind, seed, n, sr))
     if rng_seed is not None:
         np.random.seed(rng_seed)
     y, _ = qd.process_audio(x, sr, n_fft=n_fft, precision="float64", **SB, **kw)
-    _check(y, pipe[f"{name}/y"], f"{name}/y float64", 5e-6)
+    _check(*pipe.at(f"{name}/y", y), f"{name}/y float64", 5e-6)
 
 
 @pytest.mark.gpu

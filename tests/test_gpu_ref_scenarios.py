@@ -6,7 +6,6 @@ there.  Each case is checked twice: against the LIVE reference's output and taps
 generator tests/golden/make_golden.py scenarios) at the north-star tolerance, and against the assertion the
 reference's test makes (qd_cases.check_scenario_property), evaluated on OUR output.
 """
-import os
 
 import numpy as np
 import pytest
@@ -14,7 +13,6 @@ import pytest
 import qd_cases
 from oracle import qd_oracle as orc
 
-G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 MAX_ABS = 1e-4
 NULL_DB = -80.0
 
@@ -31,7 +29,7 @@ def qd():
 
 @pytest.fixture(scope="module")
 def sc():
-    return np.load(os.path.join(G, "scenarios.npz"))
+    return qd_cases.Golden("scenarios")
 
 
 @pytest.fixture(scope="module")
@@ -41,7 +39,7 @@ def rendered(qd, sc):
     for name, (spec, sr, rng_seed, kw, prop, cite) in qd_cases.REF_SCENARIOS.items():
         if rng_seed is not None:
             np.random.seed(rng_seed)   # the random spectral FX replay the global np.random state like the reference
-        out[name] = qd.process_audio(sc[f"{name}/x"], sr=sr, **kw)
+        out[name] = qd.process_audio(sc.input(name, qd_cases.scenario_signal(spec, sr)), sr=sr, **kw)
     return out
 
 
@@ -49,14 +47,14 @@ def rendered(qd, sc):
 @pytest.mark.parametrize("name", list(qd_cases.REF_SCENARIOS))
 def test_reference_test_scenarios(rendered, sc, name):
     spec, sr, rng_seed, kw, prop, cite = qd_cases.REF_SCENARIOS[name]
-    x = sc[f"{name}/x"]
+    x = sc.input(name, qd_cases.scenario_signal(spec, sr))
     y, taps = rendered[name]
     assert set(taps.keys()) == {"input", "pre_quant", "post_dist", "output"}, cite
     assert np.array_equal(taps["input"], x) and np.array_equal(taps["output"], y)
     for got, key in ((y, "y"), (taps["pre_quant"], "pre_quant"), (taps["post_dist"], "post_dist")):
-        ref = sc[f"{name}/{key}"]
         what = f"{name}/{key} ({cite})"
-        assert got.dtype == np.float32 and got.shape == ref.shape == x.shape, what
+        assert got.dtype == np.float32 and got.shape == sc.shape(f"{name}/{key}") == x.shape, what
+        got, ref = sc.at(f"{name}/{key}", got)
         err = float(np.max(np.abs(got.astype(np.float64) - ref)))
         if key == "y" and name in qd_cases.REF_SCENARIO_Y_TOL:   # the reference itself is ill-conditioned there
             assert err <= qd_cases.REF_SCENARIO_Y_TOL[name], f"{what}: max abs err {err:.3e}"
@@ -69,11 +67,11 @@ def test_reference_test_scenarios(rendered, sc, name):
 # ---------------------------------------------------------------- the reference's scripts (tests/golden/scripts.npz)
 @pytest.fixture(scope="module")
 def scr():
-    return np.load(os.path.join(G, "scripts.npz"))
+    return qd_cases.Golden("scripts")
 
 
 def _wav_slice(name, seconds):
-    d = np.load(os.path.join(G, "refwav.npz"))
+    d = qd_cases.Golden("refwav")
     sr = int(d[f"{name}/sr"])
     return d[f"{name}/x16"][: int(sr * seconds)], sr
 
@@ -90,9 +88,9 @@ def test_reference_script_calls(qd, scr, name):
         np.random.seed(rng_seed)
     y, taps = qd.process_audio(audio=x, sr=sr, **qd_cases.script_scenario_kwargs(name))
     for got, key in ((y, "y"), (taps["pre_quant"], "pre_quant"), (taps["post_dist"], "post_dist")):
-        ref = scr[f"{name}/{key}"]
         what = f"{name}/{key} ({cite})"
-        assert got.dtype == np.float32 and got.shape == ref.shape, what
+        assert got.dtype == np.float32 and got.shape == scr.shape(f"{name}/{key}"), what
+        got, ref = scr.at(f"{name}/{key}", got)
         err = float(np.max(np.abs(got.astype(np.float64) - ref)))
         assert err <= MAX_ABS, f"{what}: max abs err {err:.3e}"
         assert orc.null_test_db(got, ref) <= NULL_DB, what
@@ -112,7 +110,7 @@ def test_reference_harness_renders(qd, scr, name, tmp_path):
         np.random.seed(rng_seed)
     qd.process_file_to_file(src, dst, preset=preset, extra_params=qd_cases.harness_extra_params(name))
     sr2, y16 = wavfile.read(str(dst))
-    ref = scr[f"{name}/y16"]
-    assert sr2 == sr and y16.dtype == np.int16 and y16.shape == ref.shape
+    assert sr2 == sr and y16.dtype == np.int16 and y16.shape == scr.shape(f"{name}/y16")
+    y16, ref = scr.at(f"{name}/y16", y16)
     d = int(np.max(np.abs(y16.astype(np.int32) - ref.astype(np.int32))))
     assert d <= 4, f"{name} ({cite}): {d} PCM16 steps"

@@ -8,7 +8,6 @@
 
 Tolerance: the north-star's max-abs <= 1e-4 and null <= -80 dBFS unless a tighter bound is written at the call.
 """
-import os
 
 import numpy as np
 import pytest
@@ -16,7 +15,6 @@ import pytest
 import qd_cases
 from oracle import qd_oracle as orc
 
-G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 MAX_ABS = 1e-4
 NULL_DB = -80.0
 SB = {"quantize_mode": "spectral_bins"}
@@ -34,17 +32,22 @@ def qd():
 
 @pytest.fixture(scope="module")
 def r2():
-    return np.load(os.path.join(G, "round2.npz"))
+    return qd_cases.Golden("round2")
 
 
 @pytest.fixture(scope="module")
 def pipe():
-    return np.load(os.path.join(G, "pipeline.npz"))
+    return qd_cases.Golden("pipeline")
 
 
 @pytest.fixture(scope="module")
 def wav():
-    return np.load(os.path.join(G, "refwav.npz"))
+    return qd_cases.Golden("refwav")
+
+
+@pytest.fixture(scope="module")
+def renders():
+    return qd_cases.Golden("refwav_renders")
 
 
 def _check(got, ref, what, max_abs=MAX_ABS):
@@ -61,13 +64,13 @@ def _check(got, ref, what, max_abs=MAX_ABS):
 @pytest.mark.parametrize("name", list(qd_cases.CASES_R2))
 def test_round2_cases_vs_reference_fixtures(qd, r2, name):
     kind, seed, n, sr, n_fft, rng_seed, kw = qd_cases.CASES_R2[name]
-    x = r2[f"{name}/x"]
+    x = r2.input(name, qd_cases.make_signal(kind, seed, n, sr))
     if rng_seed is not None:
         np.random.seed(rng_seed)
     y, taps = qd.process_audio(x, sr, n_fft=n_fft, **SB, **kw)   # precision="auto"
-    _check(y, r2[f"{name}/y"], f"{name}/y")
-    _check(taps["pre_quant"], r2[f"{name}/pre_quant"], f"{name}/pre_quant")
-    _check(taps["post_dist"], r2[f"{name}/post_dist"], f"{name}/post_dist")
+    _check(*r2.at(f"{name}/y", y), f"{name}/y")
+    _check(*r2.at(f"{name}/pre_quant", taps["pre_quant"]), f"{name}/pre_quant")
+    _check(*r2.at(f"{name}/post_dist", taps["post_dist"]), f"{name}/post_dist")
 
 
 @pytest.mark.gpu
@@ -78,9 +81,10 @@ def test_float64_fx_kernels_vs_reference_fixtures(qd, r2, pipe, name):
     kind, seed, n, sr, n_fft, rng_seed, kw = cases[name]
     if rng_seed is not None:
         np.random.seed(rng_seed)
-    y, taps = qd.process_audio(fix[f"{name}/x"], sr, n_fft=n_fft, precision="float64", **SB, **kw)
-    _check(y, fix[f"{name}/y"], f"{name}/y f64", 5e-6)
-    _check(taps["pre_quant"], fix[f"{name}/pre_quant"], f"{name}/pre_quant f64", 5e-6)
+    x = fix.input(name, qd_cases.make_signal(kind, seed, n, sr))
+    y, taps = qd.process_audio(x, sr, n_fft=n_fft, precision="float64", **SB, **kw)
+    _check(*fix.at(f"{name}/y", y), f"{name}/y f64", 5e-6)
+    _check(*fix.at(f"{name}/pre_quant", taps["pre_quant"]), f"{name}/pre_quant f64", 5e-6)
 
 
 def test_auto_precision_never_picks_a_path_outside_tolerance():
@@ -98,11 +102,12 @@ def test_auto_precision_never_picks_a_path_outside_tolerance():
 def test_autotune_kept_inside_multiband_snap0(qd, r2, name):
     """dsp/pipeline.py:1326-1327, :1076, :537-601: default mode + use_multiband + snap_strength = 0."""
     kind, seed, n, sr, kw = qd_cases.AT_MB_CASES[name]
-    y, taps = qd.process_audio(r2[f"{name}/x"], sr, **kw)
-    _check(y, r2[f"{name}/y"], f"{name}/y", 2e-6)
-    _check(taps["pre_quant"], r2[f"{name}/pre_quant"], f"{name}/pre_quant", 2e-6)
-    _check(taps["post_dist"], r2[f"{name}/post_dist"], f"{name}/post_dist", 2e-6)
-    yb, _ = qd.process_batch(np.stack([r2[f"{name}/x"]] * 3), sr, **kw)        # host pipeline, no taps
+    x = r2.input(name, qd_cases.make_signal(kind, seed, n, sr))
+    y, taps = qd.process_audio(x, sr, **kw)
+    _check(*r2.at(f"{name}/y", y), f"{name}/y", 2e-6)
+    _check(*r2.at(f"{name}/pre_quant", taps["pre_quant"]), f"{name}/pre_quant", 2e-6)
+    _check(*r2.at(f"{name}/post_dist", taps["post_dist"]), f"{name}/post_dist", 2e-6)
+    yb, _ = qd.process_batch(np.stack([x] * 3), sr, **kw)        # host pipeline, no taps
     assert np.array_equal(yb[2], y)
 
 
@@ -110,19 +115,20 @@ def test_autotune_kept_inside_multiband_snap0(qd, r2, name):
 @pytest.mark.parametrize("name", list(qd_cases.UI_AT_CASES))
 def test_ui_dict_keeps_autotune_and_its_sub_keys(qd, r2, name):
     kind, seed, n, sr, _rng, cfg, kw = qd_cases.UI_AT_CASES[name]
-    y, _ = qd.process_audio(r2[f"{name}/x"], sr, config=cfg, **kw)
-    _check(y, r2[f"{name}/y"], name)
+    y, _ = qd.process_audio(r2.input(name, qd_cases.make_signal(kind, seed, n, sr)), sr, config=cfg, **kw)
+    _check(*r2.at(f"{name}/y", y), name)
 
 
 @pytest.mark.gpu
 def test_bare_call_is_the_reference_default(qd):
     """process_audio(x, sr), PipelineConfig(), from_preset() and the file harness without overrides run
     quantize_mode="autotune_v1" (config.py:44, :77, :140) -- compared with the live-reference fixture."""
-    g = np.load(os.path.join(G, "autotune.npz"))
-    x, ref = g["at_tone_default/x"], g["at_tone_default/y"]
+    g = qd_cases.Golden("autotune")
+    kind, seed, n, sr, _kw = qd_cases.AUTOTUNE_CASES["at_tone_default"]
+    x = g.input("at_tone_default", qd_cases.make_signal(kind, seed, n, sr))
     y, taps = qd.process_audio(x, 48000)
-    _check(y, ref, "bare process_audio")
-    _check(taps["pre_quant"], g["at_tone_default/pre_quant"], "bare process_audio pre_quant")
+    _check(*g.at("at_tone_default/y", y), "bare process_audio")
+    _check(*g.at("at_tone_default/pre_quant", taps["pre_quant"]), "bare process_audio pre_quant")
     y2, _ = qd.process_audio(x, 48000, pipeline_config=qd.PipelineConfig())
     assert np.array_equal(y, y2)
     yb, _ = qd.process_batch(x[None, :], 48000)
@@ -136,18 +142,18 @@ def _wav_input(wav, name):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", list(qd_cases.REF_WAVS))
-def test_reference_files_both_modes(qd, wav, name):
+def test_reference_files_both_modes(qd, wav, renders, name):
     """BASELINE configs[0]: examples/example_bass.wav (and tests/data/*.wav) through process_audio -- the literal
     scripts/render_cli.py:32 call (default mode) and the STFT path."""
     x, sr = _wav_input(wav, name)
     y, _ = qd.process_audio(x, sr)
-    _check(y, wav[f"{name}/y_default"], f"{name} default mode")
+    _check(*renders.at(f"{name}/y_default", y), f"{name} default mode")
     y, _ = qd.process_audio(x, sr, **SB)
-    _check(y, wav[f"{name}/y_spectral_bins"], f"{name} spectral_bins")
+    _check(*renders.at(f"{name}/y_spectral_bins", y), f"{name} spectral_bins")
 
 
 @pytest.mark.gpu
-def test_render_cli_semantics_on_example_bass(qd, wav, tmp_path):
+def test_render_cli_semantics_on_example_bass(qd, wav, renders, tmp_path):
     """scripts/render_cli.py: load_audio -> process_audio(audio, sr) -> save_audio, here through the file harness with
     no preset and no overrides; the written PCM16 file against the reference's float output."""
     from quantumdistortion_b200.audio_io import float_to_pcm16, load_audio, save_audio
@@ -158,23 +164,26 @@ def test_render_cli_semantics_on_example_bass(qd, wav, tmp_path):
     qd.process_file_to_file(src, dst)
     got, sr2 = load_audio(dst)
     assert sr2 == sr
-    lsb = np.abs(np.rint(got * 32768.0) - float_to_pcm16(wav["example_bass/y_default"]).astype(np.float64))
+    got, ref = renders.at("example_bass/y_default", got)
+    lsb = np.abs(np.rint(got * 32768.0) - float_to_pcm16(ref).astype(np.float64))
     assert lsb.max() <= 4, lsb.max()     # 1e-4 = 3.3 steps of 16-bit PCM
     del save_audio
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", [n for n in qd_cases.REF_WAVS if n != "example_bass"])
-def test_reference_processed_renders_kat(qd, wav, name):
+def test_reference_processed_renders_kat(qd, wav, renders, name):
     """SURVEY.md section 4: the reference's committed *_multiband.wav / *_multiband_bitcrush.wav renders, <= 6 PCM16 steps."""
     from quantumdistortion_b200.audio_io import float_to_pcm16
     x, sr = _wav_input(wav, name)
     kw = dict(SB, use_multiband=True, crossover_hz=300.0, sub_cut_hz=0.0, air_cut_hz=0.0)
     y, _ = qd.process_audio(x, sr, **kw)
-    d = np.abs(float_to_pcm16(y).astype(np.int32) - wav[f"{name}/kat_multiband"].astype(np.int32))
+    got, ref = renders.at(f"{name}/kat_multiband", float_to_pcm16(y))
+    d = np.abs(got.astype(np.int32) - ref.astype(np.int32))
     assert int(d.max()) <= 6, int(d.max())
     y, _ = qd.process_audio(x, sr, spectral_fx_mode="bitcrush", spectral_fx_strength=0.5, **kw)
-    d = np.abs(float_to_pcm16(y).astype(np.int32) - wav[f"{name}/kat_multiband_bitcrush"].astype(np.int32))
+    got, ref = renders.at(f"{name}/kat_multiband_bitcrush", float_to_pcm16(y))
+    d = np.abs(got.astype(np.int32) - ref.astype(np.int32))
     assert int(d.max()) <= 6, int(d.max())
 
 

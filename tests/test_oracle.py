@@ -19,12 +19,12 @@ def tables():
 
 @pytest.fixture(scope="module")
 def stages():
-    return np.load(os.path.join(G, "stages.npz"))
+    return qd_cases.Golden("stages")
 
 
 @pytest.fixture(scope="module")
 def pipe():
-    return np.load(os.path.join(G, "pipeline.npz"))
+    return qd_cases.Golden("pipeline")
 
 
 def test_target_bins_and_masks_bit_exact(tables):
@@ -78,16 +78,16 @@ def test_quantize_frames_matches_reference(stages):
            "smear0": (1.0, 0.0, True, mask), "smear1": (0.5, 1.0, True, mask)}
     for tag, (snap, smear, smooth, m) in cfg.items():
         nm, nph = orc.quantize_frames(stages["q/mags"], stages["q/phases"], tb, m, snap, smear, smooth)
-        assert np.array_equal(nm, stages[f"q/{tag}/mags"]), tag
-        assert np.array_equal(nph, stages[f"q/{tag}/phases"]), tag
+        assert stages.matches(f"q/{tag}/mags", nm), tag
+        assert stages.matches(f"q/{tag}/phases", nph), tag
 
 
 def test_stft_istft_matches_reference(stages):
     x = stages["stft/x"]
     for nf in (512, 2048):
         S, _ = orc.stft(x, 48000, n_fft=nf)
-        assert np.array_equal(S, stages[f"stft/{nf}/S"])
-        assert np.array_equal(orc.istft(S, 48000, n_fft=nf, length=len(x)), stages[f"stft/{nf}/y"])
+        assert stages.matches(f"stft/{nf}/S", S)
+        assert stages.matches(f"stft/{nf}/y", orc.istft(S, 48000, n_fft=nf, length=len(x)))
 
 
 def test_spectral_fx_matches_reference(stages):
@@ -97,20 +97,19 @@ def test_spectral_fx_matches_reference(stages):
            "scr055": ("bin_scramble", 0.55), "scr03": ("bin_scramble", 0.3), "scr09": ("bin_scramble", 0.9)}
     for tag, (mode, s) in cfg.items():
         np.random.seed(99)
-        for t in range(3):
-            a, b = orc.apply_spectral_fx(fm.copy(), fp.copy(), mode, s, {})
-            assert np.array_equal(a, stages[f"fx/{tag}/mag"][t]), tag
-            assert np.array_equal(b, stages[f"fx/{tag}/phase"][t]), tag
+        frames = [orc.apply_spectral_fx(fm.copy(), fp.copy(), mode, s, {}) for t in range(3)]
+        assert stages.matches(f"fx/{tag}/mag", np.array([a for a, _ in frames])), tag
+        assert stages.matches(f"fx/{tag}/phase", np.array([b for _, b in frames])), tag
     a, _ = orc.fx_bitcrush(fm, fp, method="uniform", step=0.07, threshold=0.01)
-    assert np.array_equal(a, stages["fx/uniform/mag"])
+    assert stages.matches("fx/uniform/mag", a)
 
 
 def test_formant_shift_matches_reference(stages):
     fm = stages["fx/mag"]
     for st in (3.0, -5.0, 12.0, -0.5):
-        assert np.array_equal(orc.formant_shift_frame(fm, st), stages[f"fx/formant/{st}"]), st
-        assert np.array_equal(orc.formant_shift_frame(stages["fx/formant/zeros_in"], st), stages[f"fx/formant/zeros/{st}"]), st
-        assert np.array_equal(orc.formant_shift_frame(stages["fx/formant/in257"], st), stages[f"fx/formant/257/{st}"]), st
+        assert stages.matches(f"fx/formant/{st}", orc.formant_shift_frame(fm, st)), st
+        assert stages.matches(f"fx/formant/zeros/{st}", orc.formant_shift_frame(stages["fx/formant/zeros_in"], st)), st
+        assert stages.matches(f"fx/formant/257/{st}", orc.formant_shift_frame(stages["fx/formant/in257"], st)), st
     assert np.array_equal(orc.formant_shift_frame(fm, 0.0), fm)
 
 
@@ -145,15 +144,14 @@ def test_sosfilt_matches_scipy():
 def test_pipeline_matches_reference(pipe, name):
     kind, seed, n, sr, n_fft, rng_seed, kw = qd_cases.CASES[name]
     x = qd_cases.make_signal(kind, seed, n, sr)
-    assert np.array_equal(x, pipe[f"{name}/x"]), "synthetic input drifted from the fixture"
+    assert pipe.matches(f"{name}/x", x), "synthetic input drifted from the fixture"
     if rng_seed is not None:
         np.random.seed(rng_seed)
     y, taps = orc.process_audio(x, sr, n_fft=n_fft, **kw)
     assert y.dtype == np.float32 and y.shape == x.shape
     for got, key in ((y, "y"), (taps["pre_quant"], "pre_quant"), (taps["post_dist"], "post_dist")):
-        ref = pipe[f"{name}/{key}"]
-        err = float(np.max(np.abs(got.astype(np.float64) - ref))) if len(ref) else 0.0
-        assert np.array_equal(got, ref), f"{name}/{key}: max abs diff {err:.3e}"
+        err = pipe.max_abs_err(f"{name}/{key}", got)
+        assert pipe.matches(f"{name}/{key}", got), f"{name}/{key}: max abs diff {err:.3e}"
 
 
 def test_null_test_definition():
@@ -165,10 +163,10 @@ def test_null_test_definition():
 @pytest.mark.parametrize("name", list(qd_cases.ANALYSIS_CASES))
 def test_cents_metric_matches_reference(name):
     """avg_cents_offset_from_scale (dsp/analyses.py:53-142): oracle and the host cents table vs the live reference."""
-    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "analysis.npz"))
+    g = qd_cases.Golden("analysis")
     kind, seed, n, sr, key, scale, kw = qd_cases.ANALYSIS_CASES[name]
     x = qd_cases.make_signal(kind, seed, n, sr)
-    assert np.array_equal(x, g[f"{name}/x"])
+    assert g.matches(f"{name}/x", x)
     avg, per, bins = orc.avg_cents_offset_from_scale(x, sr, key, scale, return_bins=True, **kw)
     assert np.array_equal(per, g[f"{name}/per_peak"])
     assert (np.isnan(avg) and np.isnan(g[f"{name}/avg"])) or avg == float(g[f"{name}/avg"])

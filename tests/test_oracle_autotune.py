@@ -1,6 +1,5 @@
 """CPU: the autotune_v1 oracle (oracle/qd_autotune.py) against outputs of the LIVE reference stored in
 tests/golden/autotune.npz (tests/golden/make_golden.py autotune).  Bit-exact on every stage and on whole renders."""
-import os
 
 import numpy as np
 import pytest
@@ -9,18 +8,16 @@ import scipy.signal
 import qd_cases
 from oracle import qd_autotune as at
 
-G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-
 
 @pytest.fixture(scope="module")
 def gold():
-    return np.load(os.path.join(G, "autotune.npz"))
+    return qd_cases.Golden("autotune")
 
 
 def test_band_split_and_detector(gold):
     x = gold["st/x"]
     sub, body, air = at.split_sub_body_air(x, 48000, 110.0, 5000.0)
-    assert np.array_equal(sub, gold["st/sub"]) and np.array_equal(body, gold["st/body"]) and np.array_equal(air, gold["st/air"])
+    assert gold.matches("st/sub", sub) and gold.matches("st/body", body) and gold.matches("st/air", air)
     assert np.array_equal(at.detector_sidechain(body, 48000, 110.0, 3000.0), gold["st/det"])
 
 
@@ -47,26 +44,25 @@ def test_frame_features_and_ratio_track(gold):
 
 
 def test_granular_shifter(gold):
-    assert np.array_equal(at.granular_pitch_shift(gold["st/body"], gold["st/ratio_track"]), gold["st/corrected"])
-    assert np.array_equal(at.granular_pitch_shift(gold["st/body"], gold["st/ratio_manual"]), gold["st/shift_manual"])
+    assert gold.matches("st/corrected", at.granular_pitch_shift(gold["st/body"], gold["st/ratio_track"]))
+    assert gold.matches("st/shift_manual", at.granular_pitch_shift(gold["st/body"], gold["st/ratio_manual"]))
     ones = np.ones(100, dtype=np.float32)
     assert np.array_equal(at.granular_pitch_shift(gold["st/body"][:100], ones), gold["st/body"][:100])  # early out, no latency
 
 
 def test_sub_layer_and_mode_output(gold):
     x = gold["st/x"]
-    assert np.array_equal(at.envelope_follow(x, 48000), gold["st/env"])
-    assert np.array_equal(at.sub_layer(x, 48000, at.AutotuneConfig()), gold["st/sub_layer"])
-    assert np.array_equal(at.apply_autotune_v1(x, 48000, at.AutotuneConfig())["output"], gold["st/output"])
+    assert gold.matches("st/env", at.envelope_follow(x, 48000))
+    assert gold.matches("st/sub_layer", at.sub_layer(x, 48000, at.AutotuneConfig()))
+    assert gold.matches("st/output", at.apply_autotune_v1(x, 48000, at.AutotuneConfig())["output"])
 
 
 @pytest.mark.parametrize("name", list(qd_cases.AUTOTUNE_CASES))
 def test_autotune_pipeline_matches_reference(gold, name):
     kind, seed, n, sr, kw = qd_cases.AUTOTUNE_CASES[name]
     x = qd_cases.make_signal(kind, seed, n, sr)
-    assert np.array_equal(x, gold[f"{name}/x"])
+    assert gold.matches(f"{name}/x", x)
     y, taps = at.process_audio_autotune(x, sr, **{k: v for k, v in kw.items()
                                                   if k not in ("smear", "bin_smoothing", "post_quant")})
     for got, key in ((y, "y"), (taps["pre_quant"], "pre_quant"), (taps["post_dist"], "post_dist")):
-        ref = gold[f"{name}/{key}"]
-        assert np.array_equal(got, ref), f"{name}/{key}: max abs diff {np.max(np.abs(got.astype(float) - ref)):.3e}"
+        assert gold.matches(f"{name}/{key}", got), f"{name}/{key}: max abs diff {gold.max_abs_err(f'{name}/{key}', got):.3e}"

@@ -6,7 +6,6 @@ The signals and keyword arguments are the ones the reference's test suite passes
 test_m12_quantum_fx.py, test_quantization_integration.py); quantize_mode stays at the reference default wherever
 the reference test leaves it there, so these cases also pin the mode-resolution rules of dsp/pipeline.py:1315-1327.
 """
-import os
 
 import numpy as np
 import pytest
@@ -15,7 +14,6 @@ import qd_cases
 from oracle import qd_autotune as at
 from oracle import qd_oracle as orc
 
-G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 _AT_DROP = ("smear", "bin_smoothing", "post_quant", "use_multiband", "crossover_hz", "lowband_drive", "quantize_mode",
             # options the reference test passes at their "off" value: they do not leave autotune_v1 (:1315-1324)
             "spectral_fx_mode", "spectral_fx_strength", "spectral_freeze", "formant_shift", "harmonic_lock_hz")
@@ -23,7 +21,7 @@ _AT_DROP = ("smear", "bin_smoothing", "post_quant", "use_multiband", "crossover_
 
 @pytest.fixture(scope="module")
 def sc():
-    return np.load(os.path.join(G, "scenarios.npz"))
+    return qd_cases.Golden("scenarios")
 
 
 def oracle_render(x, sr, kw):
@@ -43,22 +41,28 @@ def oracle_render(x, sr, kw):
 def test_oracle_on_reference_test_scenarios(sc, name):
     spec, sr, rng_seed, kw, prop, cite = qd_cases.REF_SCENARIOS[name]
     x = qd_cases.scenario_signal(spec, sr)
-    assert np.array_equal(x, sc[f"{name}/x"]), "scenario signal drifted from the fixture"
+    assert sc.matches(f"{name}/x", x), "scenario signal drifted from the fixture"
     if rng_seed is not None:
         np.random.seed(rng_seed)
     y, taps = oracle_render(x, sr, kw)
     for got, key in ((y, "y"), (taps["pre_quant"], "pre_quant"), (taps["post_dist"], "post_dist")):
-        ref = sc[f"{name}/{key}"]
         got = np.asarray(got, dtype=np.float32)
-        assert got.shape == ref.shape, f"{name}/{key} ({cite})"
-        err = float(np.max(np.abs(got.astype(np.float64) - ref))) if ref.size else 0.0
+        assert got.shape == sc.shape(f"{name}/{key}"), f"{name}/{key} ({cite})"
+        err = sc.max_abs_err(f"{name}/{key}", got)
         assert err <= 2e-7, f"{name}/{key} ({cite}): max abs err {err:.3e}"
 
 
 def test_reference_assertions_hold_on_the_fixtures(sc):
-    """The fixtures themselves satisfy what the reference's tests assert (a guard for the generator)."""
-    for name in qd_cases.REF_SCENARIOS:
-        qd_cases.check_scenario_property(name, sc[f"{name}/x"], sc[f"{name}/y"], lambda other: sc[f"{other}/y"])
+    """What the reference's tests assert holds on the reference's renders (a guard for the generator).  The fixtures keep
+    a sample of each render, so the assertions run on the oracle's renders, checked against those samples first."""
+    ys = {}
+    for name, (spec, sr, rng_seed, kw, _prop, _cite) in qd_cases.REF_SCENARIOS.items():
+        if rng_seed is not None:
+            np.random.seed(rng_seed)
+        ys[name] = np.asarray(oracle_render(qd_cases.scenario_signal(spec, sr), sr, kw)[0], dtype=np.float32)
+        assert sc.max_abs_err(f"{name}/y", ys[name]) <= 2e-7, name
+    for name, (spec, sr, *_rest) in qd_cases.REF_SCENARIOS.items():
+        qd_cases.check_scenario_property(name, qd_cases.scenario_signal(spec, sr), ys[name], ys.get)
 
 
 def test_reference_formant_second_pass_is_ill_conditioned(sc):
@@ -75,7 +79,7 @@ def test_reference_formant_second_pass_is_ill_conditioned(sc):
         return orc.istft(Sq, sr, 2048, length=len(sig)).astype(np.float32)
 
     y0 = second_pass(x)
-    assert np.array_equal(y0, sc[f"{name}/y"])   # limiter idle (peak 0.07): the pass output is the render
+    assert sc.matches(f"{name}/y", y0)   # limiter idle (peak 0.07): the pass output is the render
     rng = np.random.default_rng(0)
     y1 = second_pass(x.astype(np.float64) + 1e-9 * rng.standard_normal(len(x)))
     assert float(np.max(np.abs(y1 - y0))) > 1e-4
@@ -86,7 +90,7 @@ def test_reference_freeze_needs_a_float64_fft(sc):
     FFT's level (1e-7 of the frame's strongest bin) moves the reference's frozen pass by more than the 1e-4 bound on the
     reference's own test signal, noise at the float64 level does not."""
     name, sr = "freeze_multiband", 44100
-    _, high = orc.linkwitz_riley_split(sc[f"{name}/x"], sr, 300.0)
+    _, high = orc.linkwitz_riley_split(qd_cases.scenario_signal(qd_cases.REF_SCENARIOS[name][0], sr), sr, 300.0)
     S, freqs = orc.stft(high.astype(np.float32), sr, 2048)
 
     def frozen_pass(Sx):
@@ -104,11 +108,11 @@ def test_reference_freeze_needs_a_float64_fft(sc):
 # ---------------------------------------------------------------- the reference's scripts (tests/golden/scripts.npz)
 @pytest.fixture(scope="module")
 def scr():
-    return np.load(os.path.join(G, "scripts.npz"))
+    return qd_cases.Golden("scripts")
 
 
 def _wav_slice(name, seconds):
-    d = np.load(os.path.join(G, "refwav.npz"))
+    d = qd_cases.Golden("refwav")
     sr = int(d[f"{name}/sr"])
     return d[f"{name}/x16"][: int(sr * seconds)], sr
 
@@ -122,8 +126,7 @@ def test_oracle_on_reference_script_calls(scr, name):
         np.random.seed(rng_seed)
     y, taps = oracle_render(x, sr, qd_cases.script_scenario_kwargs(name))
     for got, key in ((y, "y"), (taps["pre_quant"], "pre_quant"), (taps["post_dist"], "post_dist")):
-        ref = scr[f"{name}/{key}"]
-        err = float(np.max(np.abs(np.asarray(got, dtype=np.float64) - ref)))
+        err = scr.max_abs_err(f"{name}/{key}", np.asarray(got, dtype=np.float64))
         assert err <= 2e-7, f"{name}/{key} ({cite}): max abs err {err:.3e}"
 
 
@@ -143,6 +146,6 @@ def test_oracle_on_reference_harness_renders(scr, name):
     if rng_seed is not None:
         np.random.seed(rng_seed)
     y, _ = oracle_render(x, sr, kw)
-    pcm = np.clip(np.rint(y.astype(np.float64) * 32767.0), -32768, 32767).astype(np.int32)
-    d = int(np.max(np.abs(pcm - scr[f"{name}/y16"].astype(np.int32))))
+    pcm, ref = scr.at(f"{name}/y16", np.clip(np.rint(y.astype(np.float64) * 32767.0), -32768, 32767).astype(np.int32))
+    d = int(np.max(np.abs(pcm - ref.astype(np.int32))))
     assert d <= 1, f"{name} ({cite}): {d} PCM16 steps"
