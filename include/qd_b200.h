@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define QD_ABI_VERSION 5
+#define QD_ABI_VERSION 6
 
 typedef enum qd_status {
     QD_OK = 0,
@@ -61,7 +61,7 @@ typedef struct qd_params {
     uint32_t struct_size;        /* sizeof(qd_params), for ABI checks */
     int32_t  sample_rate;
     int32_t  n_fft;              /* dsp/pipeline.py:149 N_FFT_DEFAULT; hop = n_fft/4 */
-    int32_t  n_samples;          /* samples per clip (all clips of a batch share it) */
+    int32_t  n_samples;          /* samples per clip (all clips of a batch share it); longest clip for ragged renders */
 
     int32_t  passthrough;        /* dsp/pipeline.py:477-535 */
     int32_t  pre_quant;          /* pre_quant  and snap_strength > 0  (:635) */
@@ -139,8 +139,8 @@ typedef struct qd_tables {
 
 /* Optional extra outputs (dsp/pipeline.py:914-918, 1104-1109); NULL = not wanted. */
 typedef struct qd_taps {
-    float *pre_quant;   /* [batch, n_samples] */
-    float *post_dist;   /* [batch, n_samples] */
+    float *pre_quant;   /* [batch, n_samples], or packed like x in a ragged render */
+    float *post_dist;   /* [batch, n_samples], or packed like x in a ragged render */
 } qd_taps;
 
 typedef struct qd_plan qd_plan;
@@ -214,6 +214,30 @@ int qd_render_host_pcm16(qd_plan *plan, const int16_t *x_host, int16_t *y_host, 
 #define QD_SAMPLE_PCM16 1
 int qd_render_host_ex(qd_plan *plan, const void *x_host, void *y_host, int64_t batch, int64_t chunk_clips,
                       int32_t in_format, int32_t out_format);
+
+/*
+ * Ragged batch: clips of different lengths in one render.  Clip c occupies x[starts[c] - starts[0] ... + lengths[c])
+ * and the same span of y and of each tap.  starts: int64[batch], non-decreasing, spans do not overlap (gaps allowed:
+ * the Python packer aligns every start to 16 bytes); lengths: int32[batch], each <= the plan's n_samples (the plan's
+ * n_samples is the longest clip it accepts, and sizes its FX tables).  Offsets are relative to starts[0], so a
+ * sub-range of clips is addressed by advancing x, y, starts and lengths together.  Samples in the gaps of y and of
+ * the taps are unspecified.
+ *   span_samples  packed extent, starts[batch-1] - starts[0] + lengths[batch-1]: sizes the workspace, whose
+ *                 intermediates are packed like x
+ *   max_samples   the longest clip of the batch (<= n_samples): sizes the grid
+ * qd_render_device_varlen never reads `starts` / `lengths` on the host (device arrays; the caller validates them);
+ * qd_render_host_varlen takes host arrays, validates them (QD_ERR_INVALID_ARG), uploads them once per call and cuts
+ * the batch into clip ranges whose packed span fits `chunk_samples` (a longer clip gets a chunk of its own).  The
+ * uniform entry points above are the special case starts[c] = c * n_samples, lengths[c] = n_samples.
+ */
+size_t qd_plan_workspace_bytes_varlen(const qd_plan *plan, int64_t batch, int64_t span_samples);
+int qd_render_device_varlen(qd_plan *plan, const float *x, float *y, const int64_t *starts /* device */,
+                            const int32_t *lengths /* device */, int64_t batch, int64_t span_samples,
+                            int32_t max_samples, const qd_taps *taps, void *workspace, size_t workspace_bytes,
+                            void *stream);
+int qd_render_host_varlen(qd_plan *plan, const void *x_host, void *y_host, const int64_t *starts /* host */,
+                          const int32_t *lengths /* host */, int64_t batch, int64_t chunk_samples,
+                          int32_t in_format, int32_t out_format);
 
 /* Stage-level entry points (parity ladder, SURVEY.md section 7.3b). All async on `stream`. */
 /* dsp/limiter.py:14-80 on [batch, n] */

@@ -7,7 +7,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "csrc", "libqd_b200.so")
 
-QD_ABI_VERSION = 5
+QD_ABI_VERSION = 6
 QD_FX = {"none": 0, "bitcrush_log": 1, "bitcrush_uniform": 2, "phase_dispersal": 3,
          "scramble_pick": 4, "scramble_swap": 5}
 
@@ -86,6 +86,10 @@ def load() -> C.CDLL:
     lib.qd_render_host.argtypes = [vp, vp, vp, i64, i64]
     lib.qd_render_host_pcm16.argtypes = [vp, vp, vp, i64, i64]
     lib.qd_render_host_ex.argtypes = [vp, vp, vp, i64, i64, i32, i32]
+    lib.qd_plan_workspace_bytes_varlen.argtypes = [vp, i64, i64]
+    lib.qd_plan_workspace_bytes_varlen.restype = C.c_size_t
+    lib.qd_render_device_varlen.argtypes = [vp, vp, vp, vp, vp, i64, i64, i32, C.POINTER(QdTaps), vp, C.c_size_t, vp]
+    lib.qd_render_host_varlen.argtypes = [vp, vp, vp, vp, vp, i64, i64, i32, i32]
     lib.qd_limiter_device.argtypes = [vp, vp, i64, i64, i32, dbl, dbl, vp]
     lib.qd_crossover_device.argtypes = [vp, vp, vp, i64, i64, C.POINTER((dbl * 6) * 2), C.POINTER((dbl * 6) * 2), vp]
     lib.qd_distort_device.argtypes = [vp, vp, i64, i32, dbl, dbl, flt, flt, vp]

@@ -42,7 +42,11 @@ cudaError_t upload(const std::vector<T> &h, T **d) {
 }
 
 struct HostPipe {   // resources of qd_render_host* (qd_host_pipe.inc)
-    int64_t chunk = 0;
+    int64_t cap = 0;         // samples per device buffer (the longest chunk's packed span)
+    int64_t cap_clips = 0;   // clips per chunk the workspace is sized for
+    int64_t *d_starts = nullptr;   // ragged calls: the caller's starts / lengths, uploaded once per call
+    int32_t *d_lengths = nullptr;
+    int64_t d_clips = 0;
     float *dx[2] = {nullptr, nullptr};
     float *dy[2] = {nullptr, nullptr};
     int16_t *dxr[2] = {nullptr, nullptr};   // PCM16 transport: raw input / output chunks on the device
@@ -88,6 +92,17 @@ struct qd_plan {
 };
 
 namespace {
+// How the clips of one render sit in their buffers: uniform (starts == null: clip c at c * n_samples) or a ragged batch
+// (device arrays, offsets relative to starts[0]).  span = packed extent in samples; max_n = the longest clip.
+struct Packing {
+    const int64_t *starts = nullptr;
+    const int32_t *lengths = nullptr;
+    int64_t span = 0;
+    int max_n = 0;
+};
+// intermediates of a render ([x_dist], [low], [high]) use the packing of x, each padded to 256 bytes
+size_t padded_span(int64_t span) { return ((size_t)span + 63) & ~(size_t)63; }
+
 struct TimeScope {  // brackets the launches of one kernel class with events on the launch stream
     qd_plan *pl; cudaStream_t st; int cls; cudaEvent_t a = nullptr, b = nullptr;
     static cudaEvent_t get(qd_plan *p) {
@@ -207,8 +222,12 @@ int launch_freeze(int nc, const qd::SpecArgsT<T> &a, T *out, int64_t batch, cuda
 }
 
 template <class T>
-int launch_spec_prec(qd_plan *pl, qd::SpecArgsT<T> a, const float *src, float *dst, float *tap, int quant,
+int launch_spec_prec(qd_plan *pl, qd::SpecArgsT<T> a, const Packing &pk, const float *src, float *dst, float *tap, int quant,
                      int epilogue, int64_t batch, cudaStream_t st, int fx_pass, int clip_offset, float *clip_peak) {
+    a.starts = pk.starts;
+    a.lengths = pk.lengths;
+    a.clip0 = 0;
+    a.n = pk.max_n;
     a.x = src;
     a.y = dst;
     a.tap = tap;
@@ -226,15 +245,17 @@ int launch_spec_prec(qd_plan *pl, qd::SpecArgsT<T> a, const float *src, float *d
     const int ng = (nw == 16) ? 2 : 1;   // clips per CTA
     // three-pass plans without FX: the team kernel (qd_spec_team.cuh; several warps per frame at n_fft >= 4096)
     const bool team = !fx && pl->team_nf > 0;
-    // tiling: whole clips when the batch alone fills the GPU, else cut clips along time
-    const int total_blocks = (a.n + pl->hop - 1) / pl->hop;
+    // tiling: whole clips when the batch alone fills the GPU, else cut clips along time.  The grid covers the longest
+    // clip (CTAs past a shorter clip's end exit at once); the tile is cut from the mean clip
+    const int total_blocks = (pk.max_n + pl->hop - 1) / pl->hop;
+    const int mean_blocks = (int)((pk.span / batch + pl->hop - 1) / pl->hop);
     const int ctas_per_sm = std::max<int>(1, (int)((227 * 1024) / ((team ? pl->team_smem : pl->spec_smem) + 1024)));
     const int64_t want = (int64_t)pl->sm_count * ctas_per_sm * 2 * ng;
     const int wpg = team ? pl->team_nf : nw / ng;  // frames per batch of one clip group
     int tile = total_blocks;
     if (batch < want) {
         const int64_t per_clip = (want + batch - 1) / batch;
-        tile = (int)((total_blocks + per_clip - 1) / per_clip);
+        tile = (int)((mean_blocks + per_clip - 1) / per_clip);
         const int min_tile = 4 * wpg - 3;  // keeps the 3-frame halo recompute below 10 %
         if (tile < min_tile) tile = min_tile;
         tile = ((tile + 3 + wpg - 1) / wpg) * wpg - 3;  // whole batches of frames
@@ -258,11 +279,11 @@ int launch_spec_prec(qd_plan *pl, qd::SpecArgsT<T> a, const float *src, float *d
 }
 
 // One spectral pass over [batch, n]: src -> dst (+ optional tap of the pre-epilogue signal).
-int launch_spec(qd_plan *pl, const float *src, float *dst, float *tap, int quant, int epilogue,
+int launch_spec(qd_plan *pl, const Packing &pk, const float *src, float *dst, float *tap, int quant, int epilogue,
                 int64_t batch, cudaStream_t st, int fx_pass = 0, int clip_offset = 0, float *clip_peak = nullptr) {
     TimeScope ts(pl, st, QD_KERNEL_SPECTRAL);
-    if (pl->f64) return launch_spec_prec<double>(pl, pl->spec64, src, dst, tap, quant, epilogue, batch, st, fx_pass, clip_offset, clip_peak);
-    return launch_spec_prec<float>(pl, pl->spec, src, dst, tap, quant, epilogue, batch, st, fx_pass, clip_offset, clip_peak);
+    if (pl->f64) return launch_spec_prec<double>(pl, pl->spec64, pk, src, dst, tap, quant, epilogue, batch, st, fx_pass, clip_offset, clip_peak);
+    return launch_spec_prec<float>(pl, pl->spec, pk, src, dst, tap, quant, epilogue, batch, st, fx_pass, clip_offset, clip_peak);
 }
 
 int launch_limiter(const qd::LimiterArgs &a, int64_t batch, cudaStream_t st) {
@@ -273,11 +294,15 @@ int launch_limiter(const qd::LimiterArgs &a, int64_t batch, cudaStream_t st) {
     for (int64_t b0 = 0; b0 < batch; b0 += (1 << 30)) {
         const int64_t nb = std::min<int64_t>(1 << 30, batch - b0);
         qd::LimiterArgs c = a;
-        const size_t off = (size_t)b0 * (size_t)a.n;
-        c.x = a.x + off; c.y = a.y + off;
-        if (a.dry) c.dry = a.dry + off;
-        if (a.low) c.low = a.low + off;
-        if (a.orig) c.orig = a.orig + off;
+        if (a.starts) {
+            c.clip0 = a.clip0 + (int)b0;   // ragged: offsets stay relative to starts[0]
+        } else {
+            const size_t off = (size_t)b0 * (size_t)a.n;
+            c.x = a.x + off; c.y = a.y + off;
+            if (a.dry) c.dry = a.dry + off;
+            if (a.low) c.low = a.low + off;
+            if (a.orig) c.orig = a.orig + off;
+        }
         if (a.clip_peak) c.clip_peak = a.clip_peak + b0;
         qd::limiter_mix_kernel<<<(unsigned)nb, qd::QD_TT, smem, st>>>(c);
     }
@@ -297,8 +322,12 @@ void launch_crossover(const qd::CrossoverArgs &c, int64_t batch, cudaStream_t st
     for (int64_t b0 = 0; b0 < batch; b0 += 65535) {   // gridDim.y limit
         const int64_t nb = std::min<int64_t>(65535, batch - b0);
         qd::CrossoverArgs k = c;
-        const size_t off = (size_t)b0 * (size_t)c.n;
-        k.x = c.x + off; k.low = c.low + off; k.high = c.high + off;
+        if (c.starts) {
+            k.clip0 = c.clip0 + (int)b0;   // ragged: offsets stay relative to starts[0]
+        } else {
+            const size_t off = (size_t)b0 * (size_t)c.n;
+            k.x = c.x + off; k.low = c.low + off; k.high = c.high + off;
+        }
         qd::crossover_kernel<<<dim3(gx, (unsigned)nb, 1), 32 * qd::QD_XO_WARPS, 0, st>>>(k);
     }
 }
@@ -604,18 +633,24 @@ void qd_plan_destroy(qd_plan *pl) {
         if (hp.ev_ring_out[i]) cudaEventDestroy(hp.ev_ring_out[i]);
     }
     if (hp.ws) cudaFree(hp.ws);
+    if (hp.d_starts) cudaFree(hp.d_starts);
+    if (hp.d_lengths) cudaFree(hp.d_lengths);
     if (hp.s_in) cudaStreamDestroy(hp.s_in);
     if (hp.s_run) cudaStreamDestroy(hp.s_run);
     if (hp.s_out) cudaStreamDestroy(hp.s_out);
     delete pl;
 }
 
+size_t qd_plan_workspace_bytes_varlen(const qd_plan *pl, int64_t batch, int64_t span_samples) {
+    if (!pl || batch <= 0 || span_samples < 0) return 0;
+    const size_t bufs = pl->p.multiband ? 3 : 1;  // [x_dist] (+ [low][high]), packed like x
+    const size_t frozen = pl->p.spectral_freeze ? (size_t)batch * (size_t)(pl->nc + pl->nc / 32) * sizeof(double) + 256 : 0;
+    return bufs * padded_span(span_samples) * sizeof(float) + 256 + frozen + (size_t)batch * sizeof(float) + 256;   // + per-clip peaks
+}
+
 size_t qd_plan_workspace_bytes(const qd_plan *pl, int64_t batch) {
     if (!pl || batch <= 0) return 0;
-    const size_t clip = (size_t)pl->p.n_samples * sizeof(float);
-    const size_t bufs = pl->p.multiband ? 3 : 1;  // [x_dist] (+ [low][high])
-    const size_t frozen = pl->p.spectral_freeze ? (size_t)batch * (size_t)(pl->nc + pl->nc / 32) * sizeof(double) + 256 : 0;
-    return bufs * clip * (size_t)batch + 256 + frozen + (size_t)batch * sizeof(float) + 256;   // + per-clip peaks
+    return qd_plan_workspace_bytes_varlen(pl, batch, (int64_t)pl->p.n_samples * batch);
 }
 
 int qd_plan_launches_per_render(const qd_plan *pl) {
@@ -665,11 +700,13 @@ int qd_plan_set_fx_table(qd_plan *pl, const void *device_table, int64_t n_tables
     return QD_OK;
 }
 
-int qd_render_device(qd_plan *pl, const float *x, float *y, int64_t batch, const qd_taps *taps,
-                     void *workspace, size_t workspace_bytes, void *stream) {
-    if (!pl || !x || !y || batch < 0) return fail(QD_ERR_INVALID_ARG, "null argument");
-    if (batch == 0 || pl->p.n_samples == 0) return QD_OK;
-    if (workspace_bytes < qd_plan_workspace_bytes(pl, batch) || !workspace)
+}  // extern "C"
+
+namespace {
+// qd_render_device and qd_render_device_varlen: one render of `batch` clips packed as `pk` says (batch, span > 0)
+int render_impl(qd_plan *pl, const float *x, float *y, const Packing &pk, int64_t batch, const qd_taps *taps,
+                void *workspace, size_t workspace_bytes, void *stream) {
+    if (workspace_bytes < qd_plan_workspace_bytes_varlen(pl, batch, pk.span) || !workspace)
         return fail(QD_ERR_WORKSPACE, "workspace too small (see qd_plan_workspace_bytes)");
     const qd_params &p = pl->p;
     if (p.fx_mode != QD_FX_NONE && (p.pre_quant || p.post_quant) && !p.passthrough) {
@@ -680,14 +717,14 @@ int qd_render_device(qd_plan *pl, const float *x, float *y, int64_t batch, const
             return fail(QD_ERR_INVALID_ARG, "per-clip FX table shorter than the batch");
     }
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t n = (size_t)p.n_samples;
-    const size_t count = n * (size_t)batch;
+    const size_t count = (size_t)pk.span;   // elementwise kernels and tap copies run over the packed span
+    const size_t stride = padded_span(pk.span);
     float *tap_pre = taps ? taps->pre_quant : nullptr;
     float *tap_dist = taps ? taps->post_dist : nullptr;
     float *w_a = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
-    float *w_low = w_a + count;
-    float *w_high = w_low + count;
-    pl->frozen_ws = reinterpret_cast<void *>((reinterpret_cast<uintptr_t>(w_a + (p.multiband ? 3 : 1) * count) + 255) & ~(uintptr_t)255);
+    float *w_low = w_a + stride;
+    float *w_high = w_low + stride;
+    pl->frozen_ws = reinterpret_cast<void *>((reinterpret_cast<uintptr_t>(w_a + (p.multiband ? 3 : 1) * stride) + 255) & ~(uintptr_t)255);
     // per-clip peak of the limiter input, written by the spectral pass that produces it (behind the freeze scratch)
     const size_t frozen_bytes = p.spectral_freeze ? (size_t)batch * (size_t)(pl->nc + pl->nc / 32) * sizeof(double) + 256 : 0;
     float *clip_peak = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(pl->frozen_ws) + frozen_bytes + 255) & ~(uintptr_t)255);
@@ -698,7 +735,8 @@ int qd_render_device(qd_plan *pl, const float *x, float *y, int64_t batch, const
     const float *low = nullptr;
     if (p.multiband) {
         qd::CrossoverArgs c{};
-        c.x = x; c.low = w_low; c.high = w_high; c.n = (long long)n;
+        c.x = x; c.low = w_low; c.high = w_high; c.n = (long long)pk.max_n;
+        c.starts = pk.starts; c.lengths = pk.lengths;
         qd_host::fill_crossover(c, &p.sos_low[0][0], &p.sos_high[0][0]);
         c.low_delay = p.low_delay;
         c.process_low = 1;
@@ -716,7 +754,7 @@ int qd_render_device(qd_plan *pl, const float *x, float *y, int64_t batch, const
 
     if (p.passthrough) {  // dsp/pipeline.py:477-535: no distortion, limiter or mix
         float *dst = p.multiband ? w_a : y;
-        if ((rc = launch_spec(pl, src, dst, nullptr, 0, 0, batch, st)) != QD_OK) return rc;
+        if ((rc = launch_spec(pl, pk, src, dst, nullptr, 0, 0, batch, st)) != QD_OK) return rc;
         if (tap_pre) QD_CUDA(cudaMemcpyAsync(tap_pre, src, count * sizeof(float), cudaMemcpyDeviceToDevice, st));
         if (p.multiband) {
             qd::add_kernel<<<ew_grid((int64_t)count, pl->sm_count), 256, 0, st>>>(low, w_a, y, (long long)count);
@@ -728,7 +766,8 @@ int qd_render_device(qd_plan *pl, const float *x, float *y, int64_t batch, const
         if (p.delta_listen) {
             // output = input - processed (dsp/pipeline.py:1371-1375)
             qd::LimiterArgs d{};
-            d.x = y; d.y = y; d.dry = y; d.orig = x; d.n = (long long)n; d.limiter_on = 0; d.lookahead = 1;
+            d.x = y; d.y = y; d.dry = y; d.orig = x; d.n = (long long)pk.max_n; d.limiter_on = 0; d.lookahead = 1;
+            d.starts = pk.starts; d.lengths = pk.lengths;
             d.wet = 1.0f; d.dry_gain = 0.0f; d.apply_mix = 1;
             if ((rc = launch_limiter(d, batch, st)) != QD_OK) return rc;
         }
@@ -748,10 +787,10 @@ int qd_render_device(qd_plan *pl, const float *x, float *y, int64_t batch, const
         clip_peak = nullptr;   // no spectral pass measured the limiter input
     } else if (p.pre_quant) {
         // pass A: STFT -> quantize -> iSTFT (= pre_quant tap) -> distortion        (:635-721)
-        if ((rc = launch_spec(pl, src, w_a, tap_pre, 1, epi, batch, st, 0, pl->clip_offset,
+        if ((rc = launch_spec(pl, pk, src, w_a, tap_pre, 1, epi, batch, st, 0, pl->clip_offset,
                               p.post_quant ? nullptr : clip_peak)) != QD_OK) return rc;
         if (p.post_quant) {  // pass B on the distorted signal                         (:729-801)
-            if ((rc = launch_spec(pl, w_a, y, nullptr, 1, 0, batch, st, 1, pl->clip_offset, clip_peak)) != QD_OK) return rc;
+            if ((rc = launch_spec(pl, pk, w_a, y, nullptr, 1, 0, batch, st, 1, pl->clip_offset, clip_peak)) != QD_OK) return rc;
             x_pq = y;
         } else {
             x_pq = w_a;       // :851-853
@@ -764,7 +803,7 @@ int qd_render_device(qd_plan *pl, const float *x, float *y, int64_t batch, const
                 src, w_a, (long long)count, p.distortion_mode, p.fold_amount, p.bias, p.tube_gain, p.tube_norm);
             QD_CUDA(cudaGetLastError());
         }
-        if ((rc = launch_spec(pl, src, y, nullptr, p.post_quant ? 1 : 0, 0, batch, st, 0, pl->clip_offset, clip_peak)) != QD_OK) return rc;
+        if ((rc = launch_spec(pl, pk, src, y, nullptr, p.post_quant ? 1 : 0, 0, batch, st, 0, pl->clip_offset, clip_peak)) != QD_OK) return rc;
         x_pq = y;
     }
     if (tap_dist) {  // dsp/pipeline.py:916 / :1107 (low band added in multiband mode)
@@ -776,13 +815,43 @@ int qd_render_device(qd_plan *pl, const float *x, float *y, int64_t batch, const
         }
     }
     qd::LimiterArgs l{};
-    l.x = x_pq; l.dry = src; l.low = low; l.orig = p.delta_listen ? x : nullptr; l.y = y; l.n = (long long)n;
+    l.x = x_pq; l.dry = src; l.low = low; l.orig = p.delta_listen ? x : nullptr; l.y = y; l.n = (long long)pk.max_n;
+    l.starts = pk.starts; l.lengths = pk.lengths;
     l.limiter_on = p.limiter_on; l.lookahead = p.lookahead > 0 ? p.lookahead : 1;
     l.ceiling = p.ceiling_lin; l.c = p.release_coeff;
     l.wet = p.wet; l.dry_gain = p.dry; l.trim = p.trim_gain; l.apply_trim = p.apply_trim; l.apply_mix = 1;
     l.clip_peak = clip_peak;   // written by the spectral pass that produced x_pq
     TimeScope ts(pl, st, QD_KERNEL_LIMITER);
     return launch_limiter(l, batch, st);
+}
+}  // namespace
+
+extern "C" {
+
+int qd_render_device(qd_plan *pl, const float *x, float *y, int64_t batch, const qd_taps *taps,
+                     void *workspace, size_t workspace_bytes, void *stream) {
+    if (!pl || !x || !y || batch < 0) return fail(QD_ERR_INVALID_ARG, "null argument");
+    if (batch == 0 || pl->p.n_samples == 0) return QD_OK;
+    Packing pk;
+    pk.span = (int64_t)pl->p.n_samples * batch;
+    pk.max_n = pl->p.n_samples;
+    return render_impl(pl, x, y, pk, batch, taps, workspace, workspace_bytes, stream);
+}
+
+int qd_render_device_varlen(qd_plan *pl, const float *x, float *y, const int64_t *starts, const int32_t *lengths,
+                            int64_t batch, int64_t span_samples, int32_t max_samples, const qd_taps *taps,
+                            void *workspace, size_t workspace_bytes, void *stream) {
+    if (!pl || !x || !y || !starts || !lengths || batch < 0 || span_samples < 0 || max_samples < 0)
+        return fail(QD_ERR_INVALID_ARG, "null / negative argument");
+    if (max_samples > pl->p.n_samples) return fail(QD_ERR_INVALID_ARG, "max_samples exceeds the plan's n_samples");
+    if (batch > INT32_MAX) return fail(QD_ERR_INVALID_ARG, "ragged batch of more than 2^31 - 1 clips");
+    if (batch == 0 || span_samples == 0 || max_samples == 0) return QD_OK;
+    Packing pk;
+    pk.starts = starts;
+    pk.lengths = lengths;
+    pk.span = span_samples;
+    pk.max_n = max_samples;
+    return render_impl(pl, x, y, pk, batch, taps, workspace, workspace_bytes, stream);
 }
 
 int qd_limiter_device(const float *x, float *y, int64_t batch, int64_t n, int32_t lookahead, double ceiling_lin,

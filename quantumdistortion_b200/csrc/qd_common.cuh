@@ -221,4 +221,16 @@ QD_DEV void dft_reg(V2<T> (&v)[R]) {
     }
 }
 
+// clip c of a launch inside its packed buffers: sample offset and length.  Uniform batches (starts == null) sit at
+// c * n; a ragged batch reads its per-clip arrays (see SpecArgsT::starts), offsets relative to starts[0].
+struct ClipSpan { long long base; int n; };
+template <class A>
+QD_DEV ClipSpan clip_span(const A &a, int c) {
+    if (a.starts) {
+        const int i = a.clip0 + c;
+        return {(long long)(a.starts[i] - a.starts[0]), (int)a.lengths[i]};
+    }
+    return {(long long)c * (long long)a.n, (int)a.n};
+}
+
 }  // namespace qd

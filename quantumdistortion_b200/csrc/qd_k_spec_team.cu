@@ -19,9 +19,13 @@ static int launch_spec_team_t(const qd::SpecArgsT<T> &a, const qd::TeamGather &t
         const int64_t nb = std::min<int64_t>(65535, batch - b0);
         qd::SpecArgsT<T> c = a;
         c.batch = (int)nb;
-        c.x = a.x + (size_t)b0 * a.n;
-        c.y = a.y + (size_t)b0 * a.n;
-        if (a.tap) c.tap = a.tap + (size_t)b0 * a.n;
+        if (a.starts) {
+            c.clip0 = a.clip0 + (int)b0;   // ragged: offsets stay relative to starts[0]
+        } else {
+            c.x = a.x + (size_t)b0 * a.n;
+            c.y = a.y + (size_t)b0 * a.n;
+            if (a.tap) c.tap = a.tap + (size_t)b0 * a.n;
+        }
         if (a.clip_peak) c.clip_peak = a.clip_peak + b0;
         kern<<<dim3((unsigned)tiles, (unsigned)nb, 1), 32 * NF * CW, smem, st>>>(c, tg);
     }

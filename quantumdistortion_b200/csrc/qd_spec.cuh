@@ -112,9 +112,14 @@ struct SpecArgsT {
     float *tap;            // optional [batch, n]: iSTFT output before the epilogue
     float *clip_peak;      // optional [batch]: max |y| per clip (atomicMax on the bit pattern; caller zeroes it).
                            // The limiter skips a clip whose peak never exceeds the ceiling: its gain is exactly 1.
-    int n;                 // samples per clip
+    int n;                 // samples per clip; ragged batch: the longest clip
     int batch;             // clips in this launch (a CTA may hold several clip groups)
-    int n_frames;          // T = 1 + n / hop
+    int n_frames;          // T = 1 + n / hop of a uniform batch (the kernels derive each clip's own from its length)
+    // ragged batch (null = uniform clips at clip * n): clip c of the launch is starts[clip0 + c] - starts[0] samples
+    // into x / y / tap and has lengths[clip0 + c] samples.  Launch splits advance clip0, not the pointers.
+    const int64_t *starts;
+    const int32_t *lengths;
+    int clip0;
     int tile_blocks;       // output hops per CTA tile
     int quant;             // run the quantizer (else pure STFT -> iSTFT)
     int epilogue;          // 0 none, 1 wavefold, 2 tube
@@ -1041,21 +1046,32 @@ spec_pass_kernel(const SpecArgsT<T> a) {
     V2<T> *slotP = reinterpret_cast<V2<T> *>(slotG + slot_cap);
 
     const int clip = (int)blockIdx.y * NG + grp;
-    const bool group_live = clip < a.batch;   // the last CTA may carry an empty group
-    const float *x = a.x + (size_t)(group_live ? clip : 0) * a.n;
-    float *y = a.y + (size_t)(group_live ? clip : 0) * a.n;
-    float *tap = a.tap ? a.tap + (size_t)(group_live ? clip : 0) * a.n : nullptr;
-    // 8-byte vector stores need an even clip length (every row then starts 8-byte aligned)
-    const bool vec2 = ((a.n & 1) == 0) && ((reinterpret_cast<uintptr_t>(a.y) & 7) == 0) &&
-                      (!a.tap || (reinterpret_cast<uintptr_t>(a.tap) & 7) == 0);
-    const bool vec4 = ((a.n & 3) == 0) && ((reinterpret_cast<uintptr_t>(a.x) & 15) == 0);
+    bool group_live = clip < a.batch;   // the last CTA may carry an empty group
+    const ClipSpan cs = clip_span(a, group_live ? clip : 0);
+    const int n = cs.n;
+    const float *x = a.x + cs.base;
+    float *y = a.y + cs.base;
+    float *tap = a.tap ? a.tap + cs.base : nullptr;
+    // 8-byte vector stores need an even clip length and 8-byte aligned rows; 16-byte staging loads an aligned clip start
+    const bool vec2 = ((n & 1) == 0) && ((reinterpret_cast<uintptr_t>(y) & 7) == 0) &&
+                      (!tap || (reinterpret_cast<uintptr_t>(tap) & 7) == 0);
+    const bool vec4 = (reinterpret_cast<uintptr_t>(x) & 15) == 0;
 
     // output hop-blocks (of the zero-padded timeline) this CTA owns: [j0, j1); block 2 <-> sample 0
-    const int j_end = 2 + (a.n + HOP - 1) / HOP;
+    const int j_end = 2 + (n + HOP - 1) / HOP;
     const int j0 = 2 + blockIdx.x * a.tile_blocks;
     const int j1 = min(j0 + a.tile_blocks, j_end);
-    if (j0 >= j1) return;
+    // a group past its clip's end has nothing to do.  With NG = 2 the groups of a CTA may belong to clips of different
+    // lengths, and the table fill below needs the whole CTA: such a group leaves with the empty group, after the last
+    // CTA-wide barrier; the CTA returns here only when neither group has work.
+    if constexpr (NG == 1) {
+        if (j0 >= j1) return;
+    } else {
+        group_live = group_live && j0 < j1;
+        if (!__syncthreads_or(group_live)) return;
+    }
     const int t_first = j0 - 3;  // first frame that touches block j0 (may be < 0: skipped)
+    const int n_frames = 1 + n / HOP;
 
     for (int i = tid; i < 3 * HP; i += nthreads) tail[i] = mk2<T>(0.0f, 0.0f);
 
@@ -1112,12 +1128,12 @@ spec_pass_kernel(const SpecArgsT<T> a) {
         // ---- stage the samples of frames tb .. tb+NW-1 (zero outside the clip)
         const long long s0 = (long long)tb * HOP - NC;  // clip index of staging[0]
         const long long s0n = s0 + (long long)NW * HOP;  // the same for the next batch
-        const bool next_by_tma = !SA && vec4 && (tb + NW < j1) && s0n >= 0 && s0n + L::STAGE <= a.n;
+        const bool next_by_tma = !SA && vec4 && (tb + NW < j1) && s0n >= 0 && s0n + L::STAGE <= n;
         if (tma_pending) {
             mbar_wait(full, full_parity);  // bulk copy issued during the previous batch
             full_parity ^= 1u;
         } else {
-            if (vec4 && s0 >= 0 && s0 + L::STAGE <= a.n) {
+            if (vec4 && s0 >= 0 && s0 + L::STAGE <= n) {
                 const float4 *src = reinterpret_cast<const float4 *>(x + s0);
                 float4 *dst = reinterpret_cast<float4 *>(stage);
 #pragma unroll 4
@@ -1125,7 +1141,7 @@ spec_pass_kernel(const SpecArgsT<T> a) {
             } else {
                 for (int i = tid; i < L::STAGE; i += nthreads) {
                     const long long s = s0 + i;
-                    stage[i] = (s >= 0 && s < a.n) ? x[s] : 0.0f;
+                    stage[i] = (s >= 0 && s < n) ? x[s] : 0.0f;
                 }
             }
             group_sync<NG, 32 * NW>(grp);
@@ -1133,7 +1149,7 @@ spec_pass_kernel(const SpecArgsT<T> a) {
         tma_pending = next_by_tma;
         // ---- one frame per warp (a frame outside the clip contributes zeros)
         const int t = tb + warp;
-        const bool live = t >= 0 && t < a.n_frames;
+        const bool live = t >= 0 && t < n_frames;
         if (live) {
             const float2 *frame = reinterpret_cast<const float2 *>(stage + warp * HOP);
             fwd_first<T, NC, FftCfg<T, NC>::R1>(buf, frame, wtab, tw1, lane);
@@ -1198,9 +1214,9 @@ spec_pass_kernel(const SpecArgsT<T> a) {
                 const int j = tb + h;
                 if (j < j0 || j >= j1) return;
                 const long long nidx = (long long)(j - 2) * HOP + 2 * c;
-                if (nidx >= a.n) return;
+                if (nidx >= n) return;
                 // frames covering block j: slices sl = j - t with t in [max(0,j-3), min(j,T-1)]
-                const int sl_a = j - a.n_frames + 1 > 0 ? j - a.n_frames + 1 : 0;
+                const int sl_a = j - n_frames + 1 > 0 ? j - n_frames + 1 : 0;
                 const int sl_b = j < 3 ? j : 3;
                 V2<T> inv = mk2<T>(0.0f, 0.0f);
                 if (sl_a <= sl_b) inv = __ldg(reinterpret_cast<const V2<T> *>(a.invw + (sl_a * 4 + sl_b) * HOP) + c);
@@ -1216,7 +1232,7 @@ spec_pass_kernel(const SpecArgsT<T> a) {
                     if (tap) tap[nidx] = o.x;
                     y[nidx] = r.x;
                     out_peak = fmaxf(out_peak, fabsf(r.x));
-                    if (nidx + 1 < a.n) {
+                    if (nidx + 1 < n) {
                         if (tap) tap[nidx + 1] = o.y;
                         y[nidx + 1] = r.y;
                         out_peak = fmaxf(out_peak, fabsf(r.y));
@@ -1254,10 +1270,11 @@ freeze_mag_kernel(const SpecArgsT<T> a, T *out) {
     float *stage = reinterpret_cast<float *>(smem + (size_t)BUF * sizeof(V2<T>));
     const int lane = threadIdx.x;
     const int clip = blockIdx.x;
-    const float *x = a.x + (size_t)clip * a.n;
+    const ClipSpan cs = clip_span(a, clip);
+    const float *x = a.x + cs.base;
     for (int i = lane; i < 2 * NC; i += 32) {
         const long long s = (long long)i - NC;
-        stage[i] = (s >= 0 && s < a.n) ? x[s] : 0.0f;
+        stage[i] = (s >= 0 && s < cs.n) ? x[s] : 0.0f;
     }
     __syncwarp();
     fwd_first<T, NC, FftCfg<T, NC>::R1>(buf, reinterpret_cast<const float2 *>(stage), a.wtab, a.tw1, lane);

@@ -418,18 +418,21 @@ spec_pass_team_kernel(const SpecArgsT<T> a, const TeamGather tg) {
     V2<T> *slotP = reinterpret_cast<V2<T> *>(slotG + slot_cap);
 
     const int clip = (int)blockIdx.y;
-    const float *x = a.x + (size_t)clip * a.n;
-    float *y = a.y + (size_t)clip * a.n;
-    float *tap = a.tap ? a.tap + (size_t)clip * a.n : nullptr;
-    const bool vec2 = ((a.n & 1) == 0) && ((reinterpret_cast<uintptr_t>(a.y) & 7) == 0) &&
-                      (!a.tap || (reinterpret_cast<uintptr_t>(a.tap) & 7) == 0);
-    const bool vec4 = ((a.n & 3) == 0) && ((reinterpret_cast<uintptr_t>(a.x) & 15) == 0);
+    const ClipSpan cs = clip_span(a, clip);   // one clip per CTA: the early return below is uniform
+    const int n = cs.n;
+    const float *x = a.x + cs.base;
+    float *y = a.y + cs.base;
+    float *tap = a.tap ? a.tap + cs.base : nullptr;
+    const bool vec2 = ((n & 1) == 0) && ((reinterpret_cast<uintptr_t>(y) & 7) == 0) &&
+                      (!tap || (reinterpret_cast<uintptr_t>(tap) & 7) == 0);
+    const bool vec4 = (reinterpret_cast<uintptr_t>(x) & 15) == 0;
 
-    const int j_end = 2 + (a.n + HOP - 1) / HOP;
+    const int j_end = 2 + (n + HOP - 1) / HOP;
     const int j0 = 2 + blockIdx.x * a.tile_blocks;
     const int j1 = min(j0 + a.tile_blocks, j_end);
     if (j0 >= j1) return;
     const int t_first = j0 - 3;
+    const int n_frames = 1 + n / HOP;
 
     for (int i = tid; i < 3 * HP; i += nthreads) tail[i] = mk2<T>(0.0f, 0.0f);
     uint64_t *full = reinterpret_cast<uint64_t *>(smem + L::off_flags);
@@ -448,12 +451,12 @@ spec_pass_team_kernel(const SpecArgsT<T> a, const TeamGather tg) {
         // ---- stage the samples of frames tb .. tb+NF-1 (see spec_pass_kernel)
         const long long s0 = (long long)tb * HOP - NC;
         const long long s0n = s0 + (long long)NF * HOP;
-        const bool next_by_tma = vec4 && (tb + NF < j1) && s0n >= 0 && s0n + L::STAGE <= a.n;
+        const bool next_by_tma = vec4 && (tb + NF < j1) && s0n >= 0 && s0n + L::STAGE <= n;
         if (tma_pending) {
             mbar_wait(full, full_parity);
             full_parity ^= 1u;
         } else {
-            if (vec4 && s0 >= 0 && s0 + L::STAGE <= a.n) {
+            if (vec4 && s0 >= 0 && s0 + L::STAGE <= n) {
                 const float4 *src = reinterpret_cast<const float4 *>(x + s0);
                 float4 *dst = reinterpret_cast<float4 *>(stage);
 #pragma unroll 4
@@ -461,14 +464,14 @@ spec_pass_team_kernel(const SpecArgsT<T> a, const TeamGather tg) {
             } else {
                 for (int i = tid; i < L::STAGE; i += nthreads) {
                     const long long s = s0 + i;
-                    stage[i] = (s >= 0 && s < a.n) ? x[s] : 0.0f;
+                    stage[i] = (s >= 0 && s < n) ? x[s] : 0.0f;
                 }
             }
             __syncthreads();
         }
         tma_pending = next_by_tma;
         const int t = tb + team;
-        const bool live = t >= 0 && t < a.n_frames;   // uniform over the team
+        const bool live = t >= 0 && t < n_frames;   // uniform over the team
         if (live) {
             const float2 *frame = reinterpret_cast<const float2 *>(stage + team * HOP);
             t_fwd_first<T, NC, C::R1, CW>(buf, frame, a.wtab, a.tw1, lane, wsub, team);
@@ -517,8 +520,8 @@ spec_pass_team_kernel(const SpecArgsT<T> a, const TeamGather tg) {
                 const int j = tb + h;
                 if (j < j0 || j >= j1) continue;
                 const long long nidx = (long long)(j - 2) * HOP + 2 * c;
-                if (nidx >= a.n) continue;
-                const int sl_a = j - a.n_frames + 1 > 0 ? j - a.n_frames + 1 : 0;
+                if (nidx >= n) continue;
+                const int sl_a = j - n_frames + 1 > 0 ? j - n_frames + 1 : 0;
                 const int sl_b = j < 3 ? j : 3;
                 V2<T> inv = mk2<T>(0.0f, 0.0f);
                 if (sl_a <= sl_b) inv = __ldg(reinterpret_cast<const V2<T> *>(a.invw + (sl_a * 4 + sl_b) * HOP) + c);
@@ -534,7 +537,7 @@ spec_pass_team_kernel(const SpecArgsT<T> a, const TeamGather tg) {
                     if (tap) tap[nidx] = o.x;
                     y[nidx] = r.x;
                     out_peak = fmaxf(out_peak, fabsf(r.x));
-                    if (nidx + 1 < a.n) {
+                    if (nidx + 1 < n) {
                         if (tap) tap[nidx + 1] = o.y;
                         y[nidx + 1] = r.y;
                         out_peak = fmaxf(out_peak, fabsf(r.y));

@@ -38,6 +38,9 @@ struct LimiterArgs {
     const float *clip_peak;   // optional [batch]: max |x| per clip from the producing spectral pass.  A clip that never
                               // exceeds the ceiling has gain exactly 1 (dsp/limiter.py:68-76): its limiter is skipped,
                               // and with an identity mix in place (x == y) the CTA has nothing to do at all.
+    const int64_t *starts;    // optional ragged batch, as SpecArgsT::starts (null: clip * n, n samples each)
+    const int32_t *lengths;
+    int clip0;
 };
 
 // 8 consecutive samples of one clip starting at s (zero past the end); 2 x 16-byte loads when aligned
@@ -90,10 +93,12 @@ __global__ void __launch_bounds__(QD_TT, 3) limiter_mix_kernel(const LimiterArgs
     double *s_warp0 = reinterpret_cast<double *>((reinterpret_cast<uintptr_t>(s_gmax0 + 2 * gmax_stride) + 7) & ~(uintptr_t)7);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr int NWARP = QD_TT / 32;
-    const size_t base = (size_t)blockIdx.x * (size_t)a.n;
+    const ClipSpan cs = clip_span(a, (int)blockIdx.x);
+    const size_t base = (size_t)cs.base;
+    const long long n = cs.n;
     const float *x = a.x + base;
-    const bool vec = ((a.n & 3) == 0) && ((reinterpret_cast<uintptr_t>(a.x) & 15) == 0);
-    const bool vec_out = ((a.n & 3) == 0) && ((reinterpret_cast<uintptr_t>(a.y) & 15) == 0);
+    const bool vec = (reinterpret_cast<uintptr_t>(x) & 15) == 0;
+    const bool vec_out = (reinterpret_cast<uintptr_t>(a.y + base) & 15) == 0;
     const bool need_dry = a.apply_mix && a.dry_gain != 0.0f;
     const bool clip_quiet = a.clip_peak != nullptr && !((double)a.clip_peak[blockIdx.x] > a.ceiling);
     const bool limiter_on = a.limiter_on && !clip_quiet;
@@ -117,11 +122,11 @@ __global__ void __launch_bounds__(QD_TT, 3) limiter_mix_kernel(const LimiterArgs
     const bool fast = limiter_on && L >= QD_KS && L + 8 <= QD_CHUNK;
 
     float cur[QD_KS], nxt[QD_KS], nn[QD_KS];
-    load8(x, (long long)tid * QD_KS, a.n, vec, cur);
-    load8(x, (long long)QD_CHUNK + (long long)tid * QD_KS, a.n, vec, nxt);
+    load8(x, (long long)tid * QD_KS, n, vec, cur);
+    load8(x, (long long)QD_CHUNK + (long long)tid * QD_KS, n, vec, nxt);
     int par = 0;
-    for (long long n0 = 0; n0 < a.n; n0 += QD_CHUNK, par ^= 1) {
-        load8(x, n0 + 2LL * QD_CHUNK + (long long)tid * QD_KS, a.n, vec, nn);  // lands during this chunk
+    for (long long n0 = 0; n0 < n; n0 += QD_CHUNK, par ^= 1) {
+        load8(x, n0 + 2LL * QD_CHUNK + (long long)tid * QD_KS, n, vec, nn);  // lands during this chunk
         float *s_abs = s_abs0 + par * abs_stride;
         float *s_gmax = s_gmax0 + par * gmax_stride;
         double *s_warp = s_warp0 + par * (NWARP + 2);
@@ -153,7 +158,7 @@ __global__ void __launch_bounds__(QD_TT, 3) limiter_mix_kernel(const LimiterArgs
             } else {  // very short or very long lookahead: generic staging from global memory
                 for (int i = tid; i < span; i += QD_TT) {
                     const long long s = n0 + i;
-                    s_abs[padi(i)] = s < a.n ? fabsf(x[s]) : 0.0f;
+                    s_abs[padi(i)] = s < n ? fabsf(x[s]) : 0.0f;
                 }
                 __syncthreads();
                 for (int g = tid; g < ngroups; g += QD_TT) {
@@ -249,7 +254,7 @@ __global__ void __launch_bounds__(QD_TT, 3) limiter_mix_kernel(const LimiterArgs
         if (a.apply_mix) {
             float t[QD_KS];
             if (need_dry) {
-                load8(a.dry + base, s0, a.n, vec && ((reinterpret_cast<uintptr_t>(a.dry) & 15) == 0), t);
+                load8(a.dry + base, s0, n, vec && ((reinterpret_cast<uintptr_t>(a.dry + base) & 15) == 0), t);
 #pragma unroll
                 for (int k = 0; k < QD_KS; ++k) out[k] = __fadd_rn(__fmul_rn(a.wet, out[k]), __fmul_rn(a.dry_gain, t[k]));
             } else {
@@ -261,24 +266,24 @@ __global__ void __launch_bounds__(QD_TT, 3) limiter_mix_kernel(const LimiterArgs
                 for (int k = 0; k < QD_KS; ++k) out[k] = __fmul_rn(out[k], a.trim);
             }
             if (a.low) {
-                load8(a.low + base, s0, a.n, vec && ((reinterpret_cast<uintptr_t>(a.low) & 15) == 0), t);
+                load8(a.low + base, s0, n, vec && ((reinterpret_cast<uintptr_t>(a.low + base) & 15) == 0), t);
 #pragma unroll
                 for (int k = 0; k < QD_KS; ++k) out[k] = __fadd_rn(t[k], out[k]);
             }
             if (a.orig) {
-                load8(a.orig + base, s0, a.n, vec && ((reinterpret_cast<uintptr_t>(a.orig) & 15) == 0), t);
+                load8(a.orig + base, s0, n, vec && ((reinterpret_cast<uintptr_t>(a.orig + base) & 15) == 0), t);
 #pragma unroll
                 for (int k = 0; k < QD_KS; ++k) out[k] = __fsub_rn(t[k], out[k]);
             }
         }
         float *yo = a.y + base;
-        if (vec_out && s0 + QD_KS <= a.n) {
+        if (vec_out && s0 + QD_KS <= n) {
             *reinterpret_cast<float4 *>(yo + s0) = make_float4(out[0], out[1], out[2], out[3]);
             *reinterpret_cast<float4 *>(yo + s0 + 4) = make_float4(out[4], out[5], out[6], out[7]);
         } else {
 #pragma unroll
             for (int k = 0; k < QD_KS; ++k)
-                if (s0 + k < a.n) yo[s0 + k] = out[k];
+                if (s0 + k < n) yo[s0 + k] = out[k];
         }
 #pragma unroll
         for (int k = 0; k < QD_KS; ++k) { cur[k] = nxt[k]; nxt[k] = nn[k]; }
@@ -302,6 +307,9 @@ struct CrossoverArgs {
     int apply_mono;
     float low_trim;
     int apply_low_trim;
+    const int64_t *starts;    // optional ragged batch, as SpecArgsT::starts; n is then the longest clip (grid size)
+    const int32_t *lengths;
+    int clip0;
 };
 
 QD_DEV float low_process(float v, const CrossoverArgs &a) {
@@ -334,14 +342,16 @@ __global__ void __launch_bounds__(32 * QD_XO_WARPS) crossover_kernel(const Cross
     __shared__ float s_lo[QD_XO_WARPS][32][33];   // input row, overwritten by the low band
     __shared__ float s_hi[QD_XO_WARPS][32][33];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const size_t base = (size_t)blockIdx.y * (size_t)a.n;
+    const ClipSpan cs = clip_span(a, (int)blockIdx.y);
+    const size_t base = (size_t)cs.base;
+    const long long n = cs.n;
     const float *x = a.x + base;
     float *low = a.low + base, *high = a.high + base;
-    const long long n_tiles = (a.n + a.tile - 1) / a.tile;
+    const long long n_tiles = (n + a.tile - 1) / a.tile;
     const long long tile0 = ((long long)blockIdx.x * QD_XO_WARPS + warp) * 32;   // the warp's first tile; lane l owns tile0 + l
     if (blockIdx.x == 0 && a.low_delay > 0) {   // head of the delayed low band: the processed zero input
         const float z = a.process_low ? low_process(0.0f, a) : 0.0f;
-        for (long long i = threadIdx.x; i < a.low_delay && i < a.n; i += 32 * QD_XO_WARPS) low[i] = z;
+        for (long long i = threadIdx.x; i < a.low_delay && i < n; i += 32 * QD_XO_WARPS) low[i] = z;
     }
     if (tile0 >= n_tiles) return;
     float (*rl)[33] = s_lo[warp];
@@ -356,7 +366,7 @@ __global__ void __launch_bounds__(32 * QD_XO_WARPS) crossover_kernel(const Cross
     float nxt[32];
     auto fetch = [&](int j) {
         const long long s0 = s_first + 32LL * j;                  // row 0, column 0 of this step
-        if (rows == 32 && s0 >= 0 && s0 + 31LL * a.tile + 32 <= a.n) {
+        if (rows == 32 && s0 >= 0 && s0 + 31LL * a.tile + 32 <= n) {
             const float *p = x + s0 + lane;
 #pragma unroll
             for (int r = 0; r < 32; ++r) nxt[r] = __ldg(p + (size_t)r * a.tile);
@@ -364,7 +374,7 @@ __global__ void __launch_bounds__(32 * QD_XO_WARPS) crossover_kernel(const Cross
 #pragma unroll
             for (int r = 0; r < 32; ++r) {
                 const long long sidx = s0 + (long long)r * a.tile + lane;
-                nxt[r] = (r < rows && sidx >= 0 && sidx < a.n) ? x[sidx] : 0.0f;
+                nxt[r] = (r < rows && sidx >= 0 && sidx < n) ? x[sidx] : 0.0f;
             }
         }
     };
@@ -406,7 +416,7 @@ __global__ void __launch_bounds__(32 * QD_XO_WARPS) crossover_kernel(const Cross
         // ---- store
         if (emit) {
             const long long s0 = s_first + 32LL * j;
-            if (rows == 32 && s0 + 31LL * a.tile + 32 + a.low_delay <= a.n) {
+            if (rows == 32 && s0 + 31LL * a.tile + 32 + a.low_delay <= n) {
                 float *ph = high + s0 + lane, *pl = low + s0 + lane + a.low_delay;
 #pragma unroll 8
                 for (int r = 0; r < 32; ++r) {
@@ -416,9 +426,9 @@ __global__ void __launch_bounds__(32 * QD_XO_WARPS) crossover_kernel(const Cross
             } else {
                 for (int r = 0; r < rows; ++r) {
                     const long long sidx = s0 + (long long)r * a.tile + lane;
-                    if (sidx < a.n) {
+                    if (sidx < n) {
                         high[sidx] = rh[r][lane];
-                        if (sidx + a.low_delay < a.n) low[sidx + a.low_delay] = rl[r][lane];
+                        if (sidx + a.low_delay < n) low[sidx + a.low_delay] = rl[r][lane];
                     }
                 }
             }

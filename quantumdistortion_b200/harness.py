@@ -1,5 +1,5 @@
 """File-to-file front end (reference: quantum_distortion/dsp/harness.py:24-63), plus a batched variant that
-renders many files of equal length in one GPU call."""
+renders many files, of any lengths, in one GPU call."""
 from __future__ import annotations
 
 from dataclasses import asdict
@@ -39,8 +39,8 @@ def process_file_to_file(infile: Path, outfile: Path, preset: Optional[str] = No
 def process_files(pairs: Iterable[Tuple[Path, Path]], preset: Optional[str] = None,
                   extra_params: Optional[Dict[str, Any]] = None, seeds=None) -> int:
     """Render many (infile, outfile) pairs with one parameter set -- the same files ``process_file_to_file`` would
-    write one by one.  Files sharing (length, sample rate) are stacked and rendered as one batch (`process_batch`).
-    ``seeds`` (random spectral FX): None, one int for every file, or one seed per file in the order of ``pairs``.
+    write one by one.  Files sharing (sample rate, 16-bit PCM mono or not) are rendered as one ragged batch
+    (`process_batch` on a list of clips), whatever their lengths.  ``seeds`` (random spectral FX): None, one int for every file, or one seed per file in the order of ``pairs``.
     Returns the number of files written."""
     from .pipeline import preview_truncate, process_batch
     cfg = _config(preset, extra_params)
@@ -48,8 +48,8 @@ def process_files(pairs: Iterable[Tuple[Path, Path]], preset: Optional[str] = No
     per_file = seeds is not None and not isinstance(seeds, (int, np.integer))
     if per_file and len(seeds) != len(pairs):
         raise ValueError("need one seed per file")
-    # (length, sample rate, is 16-bit PCM mono) -> [(outfile, samples, seed)]
-    groups: Dict[Tuple[int, int, bool], List[Tuple[Path, np.ndarray, Any]]] = {}
+    # (sample rate, is 16-bit PCM mono) -> [(outfile, samples, seed)]
+    groups: Dict[Tuple[int, bool], List[Tuple[Path, np.ndarray, Any]]] = {}
     for i, (infile, outfile) in enumerate(pairs):
         infile = Path(infile)
         if not infile.exists():
@@ -61,20 +61,20 @@ def process_files(pairs: Iterable[Tuple[Path, Path]], preset: Optional[str] = No
         else:
             audio, sr = load_audio(infile)
             x = ensure_mono_float32(preview_truncate(audio, sr, None, cfg))   # process_audio truncates before the mono mix
-        groups.setdefault((x.shape[0], sr, x.dtype == np.int16), []).append((Path(outfile), x, seeds[i] if per_file else None))
+        groups.setdefault((sr, x.dtype == np.int16), []).append((Path(outfile), x, seeds[i] if per_file else None))
     written = 0
-    for (n, sr, is_pcm), items in groups.items():
-        if n == 0:
-            for out, x, _ in items:
+    for (sr, is_pcm), items in groups.items():
+        live = [it for it in items if it[1].shape[0] > 0]
+        ys, _ = process_batch([x for _, x, _ in live], sr, pipeline_config=cfg,
+                              seeds=[s for _, _, s in live] if per_file else seeds) if live else ([], None)
+        rendered = {id(it): y for it, y in zip(live, ys)}
+        for it in items:
+            out, x, _ = it
+            if x.shape[0] == 0:
                 save_audio(out, x.astype(np.float32), sr)
-                written += 1
-            continue
-        batch = np.stack([x for _, x, _ in items])
-        y, _ = process_batch(batch, sr, pipeline_config=cfg, seeds=[s for _, _, s in items] if per_file else seeds)
-        for (out, _, _), row in zip(items, y):
-            if is_pcm:
-                save_pcm16(out, row, sr)    # the device already applied save_audio's float -> PCM16 rule
+            elif is_pcm:
+                save_pcm16(out, rendered[id(it)], sr)    # the device already applied save_audio's float -> PCM16 rule
             else:
-                save_audio(out, row, sr)
+                save_audio(out, rendered[id(it)], sr)
             written += 1
     return written

@@ -12,7 +12,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 from dataclasses import dataclass
-from typing import Any, Dict, Optional, Tuple, Union
+from typing import Any, Dict, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 
@@ -58,8 +58,12 @@ def _torch():
     return torch
 
 
-def fx_tables(r: "tables.Resolved", batch: int, seeds=None, shard=None):
+def fx_tables(r: "tables.Resolved", batch: int, seeds=None, shard=None, frames: Optional[Sequence[int]] = None):
     """np.random replay tables (tables.replay_fx_table) of the random spectral FX for `batch` clips.
+
+    ``frames`` (a ragged batch): the frame count 1 + n_c // hop of every clip.  Each clip's table is then replayed
+    with its own count -- the draws a reference call on that clip makes -- and padded to the plan's r.n_frames; the
+    tables are always per clip, also for an int seed (reseeded before every clip).
 
     seeds=None : draw from the current global np.random state, clip after clip -- what a loop of reference
                  ``process_audio`` calls would consume;
@@ -69,6 +73,27 @@ def fx_tables(r: "tables.Resolved", batch: int, seeds=None, shard=None):
     (multi-GPU sharding): a seed list may then cover the whole batch (it is sliced), and with seeds=None the draws of
     the clips before the shard are consumed first and those of the clips after it afterwards, so every clip gets
     the draws it would get in an unsharded render and the global state ends where that render would leave it."""
+    if frames is not None:
+        if shard is not None:
+            raise ValueError("a ragged batch cannot be sharded")
+        frames = [int(t) for t in frames]
+        if len(frames) != batch or any(t < 1 or t > r.n_frames for t in frames):
+            raise ValueError("need one frame count in 1..n_frames per clip")
+        if isinstance(seeds, (int, np.integer)):
+            seeds = [int(seeds)] * batch
+        elif seeds is not None:
+            seeds = list(seeds)
+            if len(seeds) != batch:
+                raise ValueError("need one seed per clip")
+        tabs = []
+        for c, t in enumerate(frames):
+            if seeds is not None:
+                np.random.seed(int(seeds[c]))
+            tab = tables.replay_fx_table(r.fx_rng, r.fx_passes, t, r.n_bins)
+            full = tables.replay_fx_table(r.fx_rng, 0, r.n_frames, r.n_bins)   # identity / zero: frames past T_c
+            full[:, :t] = tab
+            tabs.append(full)
+        return tabs
     one = lambda: tables.replay_fx_table(r.fx_rng, r.fx_passes, r.n_frames, r.n_bins)  # noqa: E731
     lo, total = (int(shard[0]), int(shard[2])) if shard is not None else (0, batch)
     if seeds is None:
@@ -91,6 +116,36 @@ def fx_tables(r: "tables.Resolved", batch: int, seeds=None, shard=None):
         np.random.seed(int(sd))
         tabs.append(one())
     return tabs
+
+
+def pack_layout(lengths: Sequence[int], itemsize: int = 4) -> Tuple[np.ndarray, int]:
+    """Packed layout of a ragged batch: clip c starts at starts[c] (int64, samples), every start aligned to 16 bytes
+    of ``itemsize``-byte samples; returns (starts, span) with span = starts[-1] + lengths[-1] (0 for no clips)."""
+    n = np.asarray(lengths, dtype=np.int64).reshape(-1)
+    if n.size == 0:
+        return np.zeros(0, dtype=np.int64), 0
+    if (n < 0).any():
+        raise ValueError("clip lengths must be >= 0")
+    align = max(1, 16 // int(itemsize))
+    padded = (n + align - 1) // align * align
+    starts = np.zeros(n.size, dtype=np.int64)
+    np.cumsum(padded[:-1], out=starts[1:])
+    return starts, int(starts[-1] + n[-1])
+
+
+def check_layout(starts, lengths, max_samples: int) -> None:
+    """The rules of qd_render_*_varlen (include/qd_b200.h) on host arrays: starts non-decreasing, clips not
+    overlapping, 0 <= length <= max_samples.  Raises ValueError; the device entry point does not check them."""
+    st = np.asarray(starts)
+    ln = np.asarray(lengths)
+    if st.ndim != 1 or st.shape != ln.shape:
+        raise ValueError("starts and lengths must be 1-D and of one length")
+    if (ln < 0).any():
+        raise ValueError("clip lengths must be >= 0")
+    if (ln > int(max_samples)).any():
+        raise ValueError(f"a clip is longer than the renderer's {int(max_samples)} samples")
+    if st.size > 1 and (st[1:].astype(np.int64) < st[:-1].astype(np.int64) + ln[:-1].astype(np.int64)).any():
+        raise ValueError("clip starts must be non-decreasing and clips must not overlap")
 
 
 class Renderer:
@@ -145,14 +200,15 @@ class Renderer:
             self._ws = torch.empty(need, dtype=torch.uint8, device="cuda")
         return self._ws, need
 
-    def set_fx_seeds(self, batch: int, seeds=None, shard=None) -> None:
-        """Replay the reference's np.random draws for the spectral FX (fx_tables) and upload them."""
+    def set_fx_seeds(self, batch: int, seeds=None, shard=None, frames: Optional[Sequence[int]] = None) -> None:
+        """Replay the reference's np.random draws for the spectral FX (fx_tables) and upload them.  ``frames``: per-clip
+        frame counts of a ragged batch (per-clip tables; the renderer must come from make_renderer(..., ragged=True))."""
         r = self.resolved
         if not r.fx_rng:
             return
         torch = _torch()
-        tabs = fx_tables(r, batch, seeds, shard)
-        shared = isinstance(seeds, (int, np.integer))
+        tabs = fx_tables(r, batch, seeds, shard, frames)
+        shared = isinstance(seeds, (int, np.integer)) and frames is None
         if bool(r.params.fx_table_per_clip) == shared:
             raise ValueError("renderer built for %s FX tables; use make_renderer(..., seeds=...) with the same kind of seeds"
                              % ("per-clip" if r.params.fx_table_per_clip else "shared"))
@@ -179,6 +235,58 @@ class Renderer:
                                                   C.byref(ctaps) if ctaps is not None else None,
                                                   ws.data_ptr(), need, stream))
         return y, taps
+
+    def render_device_varlen(self, x, starts, lengths, span: int, max_samples: int, want_taps: bool = False):
+        """Ragged batch on the device: x is a flat CUDA float32 tensor holding clip c at
+        x[starts[c] - starts[0] : ... + lengths[c]]; starts (int64) and lengths (int32) are CUDA tensors, already
+        validated (pack_clips) -- the library does not read them on the host.  Returns (y, taps) packed like x (gap
+        samples unspecified).  Asynchronous on the current stream."""
+        torch = _torch()
+        if x.dtype != torch.float32 or x.dim() != 1 or not x.is_cuda or not x.is_contiguous():
+            raise ValueError("expected a contiguous flat CUDA float32 tensor")
+        if (starts.dtype != torch.int64 or lengths.dtype != torch.int32 or not starts.is_cuda or not lengths.is_cuda
+                or starts.shape != lengths.shape or starts.dim() != 1):
+            raise ValueError("starts / lengths: CUDA int64 / int32 tensors of one length")
+        if max_samples > self.n:
+            raise ValueError(f"a clip of {max_samples} samples is longer than this renderer's {self.n}")
+        batch = int(starts.shape[0])
+        y = torch.empty_like(x)
+        taps = None
+        ctaps = None
+        if want_taps:
+            taps = {"pre_quant": torch.empty_like(x), "post_dist": torch.empty_like(x)}
+            ctaps = _lib.QdTaps(taps["pre_quant"].data_ptr(), taps["post_dist"].data_ptr())
+        if batch and span and max_samples:
+            need = int(self._lib.qd_plan_workspace_bytes_varlen(self._plan, batch, int(span)))
+            if self._ws is None or self._ws.numel() < need:
+                self._ws = torch.empty(need, dtype=torch.uint8, device="cuda")
+            stream = torch.cuda.current_stream().cuda_stream
+            _lib.check(self._lib.qd_render_device_varlen(
+                self._plan, x.data_ptr(), y.data_ptr(), starts.data_ptr(), lengths.data_ptr(), batch, int(span),
+                int(max_samples), C.byref(ctaps) if ctaps is not None else None, self._ws.data_ptr(), need, stream))
+        return y, taps
+
+    def render_host_varlen(self, x_host, y_host, starts: np.ndarray, lengths: np.ndarray, chunk_samples: int = 0) -> None:
+        """Ragged batch in host memory: flat contiguous CPU tensors x_host / y_host (float32 or int16 PCM16, like
+        render_host) with clip c at [starts[c] - starts[0], + lengths[c]); starts / lengths: NumPy int64 / int32.
+        Chunks are clip ranges whose packed span fits ``chunk_samples`` (0: 128 clips of this renderer's length).
+        The library validates starts / lengths.  Synchronous."""
+        torch = _torch()
+        fmt = {torch.float32: 0, torch.int16: 1}
+        if x_host.dtype not in fmt or y_host.dtype not in fmt:
+            raise ValueError("host buffers must be float32 or int16 (PCM16)")
+        if (x_host.dim() != 1 or x_host.shape != y_host.shape or not x_host.is_contiguous()
+                or not y_host.is_contiguous()):
+            raise ValueError("x_host and y_host must be flat, contiguous and of the same length")
+        starts = np.ascontiguousarray(starts, dtype=np.int64)
+        lengths = np.ascontiguousarray(lengths, dtype=np.int32)
+        if starts.shape != lengths.shape or starts.ndim != 1:
+            raise ValueError("starts and lengths must be 1-D and of one length")
+        if len(starts) and int(starts[-1] - starts[0]) + int(lengths[-1]) > int(x_host.shape[0]):
+            raise ValueError("the clips reach past the end of the host buffers")
+        _lib.check(self._lib.qd_render_host_varlen(self._plan, x_host.data_ptr(), y_host.data_ptr(),
+                                                   starts.ctypes.data, lengths.ctypes.data, len(starts),
+                                                   int(chunk_samples), fmt[x_host.dtype], fmt[y_host.dtype]))
 
     def render_host(self, x_host, y_host, chunk_clips: int = 128) -> None:
         """x_host / y_host: contiguous CPU tensors [B, n], float32 or int16 (16-bit PCM, converted on the device with
@@ -377,9 +485,10 @@ def _resolve_kwargs(n_samples: int, sr: int, n_fft: int, kw: Dict[str, Any]) -> 
 
 
 def make_renderer(n_samples: int, sr: int = DEFAULT_SAMPLE_RATE, n_fft: int = N_FFT_DEFAULT, seeds=None,
-                  **kwargs) -> Renderer:
+                  ragged: bool = False, **kwargs) -> Renderer:
     """Resolve the reference keyword arguments once and return the cached CUDA renderer.  ``seeds`` only
-    matters for the random spectral FX (see Renderer.set_fx_seeds): an int selects one shared table."""
+    matters for the random spectral FX (see Renderer.set_fx_seeds): an int selects one shared table, unless
+    ``ragged`` (a renderer for clips of up to ``n_samples``, Renderer.render_*_varlen): per-clip tables always."""
     res, _ = _resolve_kwargs(int(n_samples), int(sr), int(n_fft), dict(kwargs))
     if isinstance(res, autotune.QdAutotuneParams):
         torch = _torch()
@@ -391,13 +500,125 @@ def make_renderer(n_samples: int, sr: int = DEFAULT_SAMPLE_RATE, n_fft: int = N_
             r = _RENDERERS[key] = AutotuneRenderer(res)
         return r
     if res.fx_rng:
-        res.params.fx_table_per_clip = 0 if isinstance(seeds, (int, np.integer)) else 1
+        res.params.fx_table_per_clip = 0 if isinstance(seeds, (int, np.integer)) and not ragged else 1
     return _renderer_for(res)
+
+
+def _ragged_batch(clips: List[Any], sr: int, n_fft: int, return_taps: bool, chunk_clips: int, seeds, kwargs):
+    """process_batch on a list of 1-D clips of any lengths (see there)."""
+    torch = _torch()
+    if all(isinstance(c, np.ndarray) for c in clips):
+        is_np, cuda = True, False
+    elif all(isinstance(c, torch.Tensor) for c in clips):
+        is_np, cuda = False, bool(clips and clips[0].is_cuda)
+        if any(bool(c.is_cuda) != cuda for c in clips):
+            raise ValueError("a list of clips must be all CUDA or all CPU tensors")
+    else:
+        raise ValueError("a list of clips must be all NumPy arrays or all tensors")
+    if any(c.ndim != 1 for c in clips):
+        raise ValueError("a list of clips holds 1-D (mono) clips")
+    pcm_of = (lambda c: c.dtype == np.int16) if is_np else (lambda c: c.dtype == torch.int16)  # noqa: E731
+    pcm = bool(clips) and pcm_of(clips[0])
+    if any(pcm_of(c) != pcm for c in clips):
+        raise ValueError("a list of clips is all int16 (PCM16) or all floating point")
+    if pcm and (cuda or return_taps):
+        raise ValueError("int16 (PCM16) input is the host transport format: CPU arrays only, no taps")
+    lengths = np.array([int(c.shape[0]) for c in clips], dtype=np.int64)
+    if seeds is not None and not isinstance(seeds, (int, np.integer)):
+        seeds = list(seeds)
+        if len(seeds) != len(clips):
+            raise ValueError("need one seed per clip")
+    out_dtype = (np.int16 if pcm else np.float32) if is_np else (torch.int16 if pcm else torch.float32)
+
+    def empty():
+        if is_np:
+            return np.zeros(0, dtype=out_dtype)
+        return torch.zeros(0, dtype=out_dtype, device="cuda" if cuda else "cpu")
+
+    r = make_renderer(int(lengths.max()) if len(clips) else 0, sr, n_fft, seeds=seeds, ragged=True, **kwargs)
+    ys: List[Any] = [None] * len(clips)
+    taps: Optional[Dict[str, List[Any]]] = {"pre_quant": [None] * len(clips), "post_dist": [None] * len(clips)} \
+        if return_taps else None
+    if isinstance(r, AutotuneRenderer):
+        # no ragged autotune_v1 kernels: clips of one length are rendered as one uniform batch
+        groups: Dict[int, List[int]] = {}
+        for i, n in enumerate(lengths.tolist()):
+            groups.setdefault(n, []).append(i)
+        for n, idx in groups.items():
+            if n == 0:
+                continue
+            xb = np.stack([clips[i] for i in idx]) if is_np else torch.stack([clips[i] for i in idx])
+            yb, tb = process_batch(xb, sr, n_fft=n_fft, return_taps=return_taps, chunk_clips=chunk_clips, **kwargs)
+            for k, i in enumerate(idx):
+                ys[i] = yb[k]
+                if taps is not None:
+                    for name in taps:
+                        taps[name][i] = tb[name][k]
+    else:
+        live = [i for i in range(len(clips)) if lengths[i] > 0]
+        if live:
+            n_live = lengths[live]
+            hop = int(n_fft) // 4
+            r.set_fx_seeds(len(live), [seeds[i] for i in live] if isinstance(seeds, list) else seeds,
+                           frames=[1 + int(n) // hop for n in n_live])
+            starts, span = pack_layout(n_live, 2 if pcm else 4)
+            max_n = int(n_live.max())
+            ends = starts + n_live
+            if cuda:   # one concatenation on the device: clips and the zero gaps that align the next start
+                zero = torch.zeros(4, dtype=torch.float32, device="cuda")
+                pieces = []
+                for k, i in enumerate(live):
+                    pieces.append(clips[i].float())
+                    if k + 1 < len(live) and starts[k + 1] > ends[k]:
+                        pieces.append(zero[:int(starts[k + 1] - ends[k])])
+                xf = torch.cat(pieces)
+            else:      # packed once into page-locked memory: this copy is the H2D staging
+                xf = torch.empty(span, dtype=torch.int16 if pcm else torch.float32, pin_memory=True)
+                xn = xf.numpy()
+                for k, i in enumerate(live):
+                    xn[starts[k]:ends[k]] = clips[i] if is_np else clips[i].numpy()
+                    if k + 1 < len(live):
+                        xn[ends[k]:starts[k + 1]] = 0
+            if cuda or return_taps:
+                d_starts = torch.from_numpy(starts).cuda()
+                d_lengths = torch.from_numpy(n_live.astype(np.int32)).cuda()
+                yf, tf = r.render_device_varlen(xf if cuda else xf.cuda().float(), d_starts, d_lengths, span, max_n,
+                                                want_taps=return_taps)
+                if not cuda:
+                    yf, tf = yf.cpu(), {k: v.cpu() for k, v in tf.items()}
+            else:
+                yf, tf = torch.empty_like(xf, pin_memory=True), None
+                r.render_host_varlen(xf, yf, starts, n_live, chunk_samples=int(chunk_clips) * max(1, span // len(live)))
+            if is_np:
+                yf, tf = yf.numpy(), (None if tf is None else {k: v.numpy() for k, v in tf.items()})
+            for k, i in enumerate(live):
+                ys[i] = yf[starts[k]:ends[k]]
+                if taps is not None:
+                    for name in taps:
+                        taps[name][i] = tf[name][starts[k]:ends[k]]
+    for i in range(len(clips)):
+        if ys[i] is None:   # zero-length clip: not rendered, consumes no FX draws
+            ys[i] = empty()
+            if taps is not None:
+                for name in taps:
+                    taps[name][i] = empty()
+    return ys, taps
 
 
 def process_batch(x, sr: int = DEFAULT_SAMPLE_RATE, *, n_fft: int = N_FFT_DEFAULT, return_taps: bool = False,
                   chunk_clips: int = 128, out=None, seeds=None, shard=None, **kwargs):
     """Render a batch of mono clips ``x[B, n]`` with one parameter set.
+
+    ``x`` may also be a list or tuple of 1-D clips of any lengths (a ragged batch): all NumPy arrays, all CPU tensors
+    or all CUDA tensors, floating point or all int16 (PCM16, host only).  The result is a list of the same kind, and
+    the taps (``return_taps``) a dict of lists; a zero-length clip comes back empty.  Each clip renders exactly as it
+    would alone: the STFT path packs the clips into one flat buffer and renders them in one call
+    (qd_render_*_varlen), with a plan sized for the longest clip and ``chunk_clips`` clips of mean length per host
+    chunk.  Random spectral FX always get one table per clip, replayed over that clip's own frames: seeds=None
+    draws clip after clip in list order (a loop of process_audio calls), an int reseeds before every clip, a list
+    gives one seed per clip.  ``shard`` and ``out`` are not supported with a list.  ``quantize_mode="autotune_v1"``
+    has no ragged kernels: the clips are grouped by length and each group is rendered as a uniform batch -- the
+    results are the same, but nothing gets faster than one call per distinct length.
 
     ``seeds`` controls the np.random replay of the random spectral FX (None: consume the global state clip by
     clip like a loop of reference calls; int: reseed before every clip; list: one seed per clip); ``shard=(lo, hi,
@@ -409,6 +630,12 @@ def process_batch(x, sr: int = DEFAULT_SAMPLE_RATE, *, n_fft: int = N_FFT_DEFAUL
     result comes back as int16, converted on the device with the WAV layer's rules (audio_io).  ``out`` (CPU
     tensor, ideally pinned like ``x``) receives the result of the host path without a fresh allocation.  Keyword arguments are the reference's ``process_audio`` arguments.
     """
+    if isinstance(x, (list, tuple)):
+        if shard is not None:
+            raise ValueError("shard= is not supported for a list of clips")
+        if out is not None:
+            raise ValueError("out= is not supported for a list of clips")
+        return _ragged_batch(list(x), sr, n_fft, return_taps, chunk_clips, seeds, kwargs)
     torch = _torch()
     is_np = isinstance(x, np.ndarray)
     if is_np:
