@@ -321,6 +321,21 @@ int    qd_autotune_render_device(const qd_autotune_params *params, const float *
                                  size_t workspace_bytes, void *stream);
 
 /*
+ * Ragged batch of the autotune_v1 mode: clips of different lengths in one call, packed as in qd_render_device_varlen
+ * (clip c at x[starts[c] - starts[0] ... + lengths[c]), y and the taps packed the same way, gap samples unspecified;
+ * starts / lengths are device arrays that are not read on the host).  params->n_samples is the longest clip the call
+ * accepts; max_samples is the longest clip of the batch.  Every clip renders exactly as it does alone.  With the
+ * pitch stage on (params->apply), a clip of 1..15 samples is not rendered (the caller rejects it, as
+ * qd_autotune_render_device rejects such a batch); a zero-length clip is skipped.  No debug outputs: those are for
+ * uniform batches.  qd_autotune_render_device is the special case starts[c] = c * n_samples.
+ */
+size_t qd_autotune_workspace_bytes_varlen(const qd_autotune_params *p, int64_t batch, int64_t span_samples);
+int    qd_autotune_render_device_varlen(const qd_autotune_params *p, const float *x, float *y,
+                                        const int64_t *starts /* device */, const int32_t *lengths /* device */,
+                                        int64_t batch, int64_t span_samples, int32_t max_samples,
+                                        const qd_taps *taps, void *workspace, size_t workspace_bytes, void *stream);
+
+/*
  * Measurement helper for the roofline report: FP32 throughput of the CUDA cores in TFLOP/s, measured with the packed
  * fma.rn.f32x2 (FFMA2) instruction the spectral pass is built from (best of a few launches on `stream`; synchronous).
  */

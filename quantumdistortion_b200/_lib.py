@@ -97,6 +97,10 @@ def load() -> C.CDLL:
     lib.qd_autotune_workspace_bytes.argtypes = [vp, i64]
     lib.qd_autotune_workspace_bytes.restype = C.c_size_t
     lib.qd_autotune_render_device.argtypes = [vp, vp, vp, i64, vp, vp, vp, C.c_size_t, vp]
+    lib.qd_autotune_workspace_bytes_varlen.argtypes = [vp, i64, i64]
+    lib.qd_autotune_workspace_bytes_varlen.restype = C.c_size_t
+    lib.qd_autotune_render_device_varlen.argtypes = [vp, vp, vp, vp, vp, i64, i64, i32, C.POINTER(QdTaps), vp,
+                                                     C.c_size_t, vp]
     lib.qd_measure_fp32_peak.argtypes = [C.POINTER(C.c_double), vp]
     lib.qd_host_alloc.argtypes = [C.c_size_t]
     lib.qd_host_alloc.restype = vp

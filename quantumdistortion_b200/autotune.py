@@ -141,9 +141,16 @@ def resolve(*, sr: int, n_samples: int, key: str, scale: str, snap_strength: flo
     p.apply_trim = int(output_trim_db != 0.0)
     p.trim_gain = float(np.float32(10.0 ** (output_trim_db / 20.0)))
     p.delta_listen = int(bool(delta_listen))
-    if p.apply and n_samples and n_samples <= 15:
-        raise ValueError("The length of the input vector x must be greater than padlen, which is 15.")  # scipy sosfiltfilt
+    check_lengths(p, [n_samples])
     return p
+
+
+def check_lengths(p: QdAutotuneParams, lengths) -> None:
+    """The reference's error for a clip the zero-phase filters cannot pad (scipy sosfiltfilt), per clip: with the pitch
+    stage on, a clip of 1..15 samples raises ValueError; a zero-length clip is not rendered."""
+    n = np.asarray(lengths, dtype=np.int64)
+    if p.apply and ((n > 0) & (n <= 15)).any():
+        raise ValueError("The length of the input vector x must be greater than padlen, which is 15.")
 
 
 def render_device(p: QdAutotuneParams, x, want_taps: bool = False, debug: bool = False, chunk_clips: int = 2048,
@@ -183,3 +190,35 @@ def render_device(p: QdAutotuneParams, x, want_taps: bool = False, debug: bool =
                                                  C.byref(cd) if cd is not None else None,
                                                  ws.data_ptr(), ws.numel(), stream))
     return y, taps, dbg, ws
+
+
+def render_device_varlen(p: QdAutotuneParams, x, starts, lengths, span: int, max_samples: int, want_taps: bool = False,
+                         workspace=None):
+    """Ragged batch on the device: x is a flat CUDA float32 tensor holding clip c at x[starts[c] - starts[0] : ... +
+    lengths[c]]; starts (int64) and lengths (int32) are CUDA tensors, already validated (pipeline.check_layout and
+    check_lengths) -- the library does not read them on the host.  Returns (y, taps or None, workspace) with y and
+    the taps packed like x (gap samples unspecified).  One call: the workspace holds about 40 bytes per packed sample
+    plus the YIN difference functions (qd_autotune_workspace_bytes_varlen)."""
+    import torch
+    lib = _lib.load()
+    if x.dtype != torch.float32 or x.dim() != 1 or not x.is_cuda or not x.is_contiguous():
+        raise ValueError("expected a contiguous flat CUDA float32 tensor")
+    if (starts.dtype != torch.int64 or lengths.dtype != torch.int32 or not starts.is_cuda or not lengths.is_cuda
+            or starts.shape != lengths.shape or starts.dim() != 1):
+        raise ValueError("starts / lengths: CUDA int64 / int32 tensors of one length")
+    if max_samples > p.n_samples:
+        raise ValueError(f"a clip of {max_samples} samples is longer than this renderer's {p.n_samples}")
+    batch = int(starts.shape[0])
+    y = torch.empty_like(x)
+    taps = {"pre_quant": torch.empty_like(x), "post_dist": torch.empty_like(x)} if want_taps else None
+    if batch and span and max_samples:
+        need = int(lib.qd_autotune_workspace_bytes_varlen(C.byref(p), batch, int(span)))
+        ws = workspace if workspace is not None and workspace.numel() >= need and workspace.device == x.device else \
+            torch.empty(need, dtype=torch.uint8, device=x.device)
+        ct = _lib.QdTaps(taps["pre_quant"].data_ptr(), taps["post_dist"].data_ptr()) if taps else None
+        _lib.check(lib.qd_autotune_render_device_varlen(
+            C.byref(p), x.data_ptr(), y.data_ptr(), starts.data_ptr(), lengths.data_ptr(), batch, int(span),
+            int(max_samples), C.byref(ct) if ct is not None else None, ws.data_ptr(), ws.numel(),
+            torch.cuda.current_stream().cuda_stream))
+        workspace = ws
+    return y, taps, workspace

@@ -33,13 +33,16 @@ constexpr int AT_EDGE = 15;   // sosfiltfilt default padlen = 3 * ntaps, ntaps =
 // from the state zi * ext[0], backward sweep from zi * y[-1], float64 in between (oracle/qd_autotune.py
 // sosfiltfilt_restated).  `scratch` holds the forward result: [jobs][batch][n + 30] doubles.
 struct AtFiltArgs {
-    const float *x[2];    // input per job, [batch, n]
+    const float *x[2];    // input per job, packed like the batch
     float *y[2];          // output per job
     AtFilter f[2];
     int jobs;
-    double *scratch;
+    double *scratch;      // clip i of job j at j * scratch_job + base_i + 2 AT_EDGE i (uniform: [job][batch][n + 30])
+    long long scratch_job;
     long long n;
-    int batch;
+    const int64_t *starts;
+    const int32_t *lengths;
+    int clip0;
 };
 
 // tile / CTA shape of the warp-staged sequential kernels below (delay taps, envelope follower): all lanes move a tile of
@@ -57,29 +60,39 @@ constexpr int AT_FW = 4;      // warps per CTA
 // shared memory (coalesced rows both ways); no scan, no block barrier.  41 -> ~10 ms per 1024 clips for the four filters.
 struct AtFiltSegArgs {
     AtFiltArgs base;
-    int tile[2], halo[2];   // per job, multiples of 32, tile >= 2 * halo
+    int tile[2], halo[2];   // per job, multiples of 32, tile >= 2 * halo; the tile before at_filt_tile
 };
 
 constexpr int AT_SW = 4;    // warps per CTA
+
+// A low cutoff has a long warm-up and few tiles per clip: while a clip of m extended samples does not fill one warp,
+// halve the tile (down to the warm-up length): twice the threads and a shorter dependent chain per thread.  Chosen per
+// clip, because the warm-up start points depend on the tile: a clip gets the tile (and the rounding) it gets alone.
+__host__ __device__ inline int at_filt_tile(int tile, int halo, long long m) {
+    while (tile / 2 >= (halo > 4096 ? halo : 4096) && (m + tile - 1) / tile < 32) tile /= 2;
+    return tile;
+}
 
 template <bool BWD>
 __global__ void __launch_bounds__(32 * AT_SW) at_filt_seg_kernel(const AtFiltSegArgs q) {
     const AtFiltArgs &a = q.base;
     __shared__ double s_row[AT_SW][32][33];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int job = blockIdx.z, clip = blockIdx.y;
-    const float *__restrict__ x = a.x[job] + (size_t)clip * a.n;
-    float *__restrict__ y = a.y[job] + (size_t)clip * a.n;
+    const int job = blockIdx.z;
+    const AtClip c = at_clip(a, blockIdx.y);
+    const long long n = c.n;
+    if (n <= AT_EDGE) return;   // not rendered: the odd extension needs more than AT_EDGE samples
+    const float *__restrict__ x = a.x[job] + c.base;
+    float *__restrict__ y = a.y[job] + c.base;
     const AtFilter &f = a.f[job];
-    const long long n = a.n;
     if (!f.on) {   // identity (astype float32): copied once, by the forward launch
         if (!BWD)
             for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) y[i] = x[i];
         return;
     }
     const long long m = n + 2 * AT_EDGE;
-    double *__restrict__ s = a.scratch + ((size_t)job * a.batch + clip) * (size_t)m;
-    const int tile = q.tile[job], halo = q.halo[job];
+    double *__restrict__ s = a.scratch + job * a.scratch_job + c.base + 2LL * AT_EDGE * c.idx;
+    const int halo = q.halo[job], tile = at_filt_tile(q.tile[job], halo, m);
     const long long n_tiles = (m + tile - 1) / tile;
     const long long tile0 = ((long long)blockIdx.x * AT_SW + warp) * 32;
     if (tile0 >= n_tiles) return;
@@ -226,10 +239,13 @@ __global__ void at_body_kernel(const float *__restrict__ x, const float *__restr
 // ---------------------------------------------------------------- detector (dsp/autotune.py:217-236)
 // rms and spectral flatness (symmetric Hann, float32 warp FFT) per frame here, YIN (float64) by the sliding kernels below.
 struct AtDetArgs {
-    const float *det;        // [batch, n] detector side chain
-    double *feat;            // [batch, frames, 4]: rms, flatness, pitch, confidence
+    const float *det;        // detector side chain, packed like the batch
+    double *feat;            // [frame rows, 4] (at_row0): rms, flatness, pitch, confidence
     long long n;
-    int frames, frame_size, hop;
+    const int64_t *starts;
+    const int32_t *lengths;
+    int clip0, batch;
+    int frame_size, hop;
     int min_tau, max_tau;
     double sr, min_freq, max_freq, threshold;
     const float *hann;       // [frame_size] np.hanning (symmetric), float32
@@ -249,14 +265,28 @@ __global__ void __launch_bounds__(32 * AT_SW_STATS) at_frame_stats_kernel(const 
     const long long fr = (long long)blockIdx.x * AT_SW_STATS + warp;
     if (fr >= total_frames) return;
     float2 *buf = reinterpret_cast<float2 *>(smem) + (size_t)warp * BUF;
-    const long long clip = fr / a.frames;
-    const int frame = (int)(fr % a.frames);
-    const float *x = a.det + (size_t)clip * a.n;
-    const long long start = (long long)frame * a.hop;
+    // the clip that owns frame row fr: uniform rows are clip-major; a ragged batch searches its row starts (at_row0)
+    int ci;
+    if (a.starts) {
+        int lo = 0, hi = a.batch - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if ((long long)(a.starts[mid] - a.starts[0]) / a.hop + mid <= fr) lo = mid; else hi = mid - 1;
+        }
+        ci = lo;
+    } else {
+        ci = (int)(fr / at_rows(a.n, a.hop));
+    }
+    const AtClip c = at_clip(a, ci);
+    const long long frame = fr - at_row0(a.starts != nullptr, c, a.n, a.hop);
+    if (frame >= at_rows(c.n, a.hop)) return;            // a row between two clips
+    const long long n = c.n;
+    const float *x = a.det + c.base;
+    const long long start = frame * a.hop;
     float sq = 0.0f, mx = 0.0f;
     for (int j = lane; j < NC; j += 32) {
         const long long s0 = start + 2 * j;
-        const float v0 = s0 < a.n ? x[s0] : 0.0f, v1 = s0 + 1 < a.n ? x[s0 + 1] : 0.0f;
+        const float v0 = s0 < n ? x[s0] : 0.0f, v1 = s0 + 1 < n ? x[s0 + 1] : 0.0f;
         sq += v0 * v0 + v1 * v1;
         mx = fmaxf(mx, fmaxf(fabsf(v0), fabsf(v1)));
         buf[tpos<float, NC>(j)] = make_float2(v0 * a.hann[2 * j], v1 * a.hann[2 * j + 1]);
@@ -375,9 +405,12 @@ __global__ void __launch_bounds__(256) at_yin_pick_kernel(const AtYinArgs a) {
 
 // ---------------------------------------------------------------- note-hold state machine, one thread per clip
 struct AtHoldArgs {
-    const double *feat;      // [batch, frames, 4]
-    double *ratio;           // [batch, frames]
-    int batch, frames;
+    const double *feat;      // [frame rows, 4]
+    double *ratio;           // [frame rows]
+    long long n, total_frames;   // total_frames: frame rows of the batch
+    const int64_t *starts;
+    const int32_t *lengths;
+    int clip0, batch, hop;
     int root_pc, n_intervals;
     int intervals[8];
     double strength, rms_thr, flat_thr, conf_thr, change_cents;
@@ -409,7 +442,7 @@ QD_DEV double at_nearest_scale_freq(double freq, const AtHoldArgs &a) {   // dsp
 // so the sequential kernel below only runs the state machine.
 __global__ void at_target_kernel(const AtHoldArgs a) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (long long)a.batch * a.frames) return;
+    if (i >= a.total_frames) return;                     // (rows between the clips of a ragged batch are never read)
     const double *f = a.feat + (size_t)i * 4;
     const double rms = f[0], flat = f[1], p = f[2], conf = f[3];
     const bool voiced = p > 0.0 && rms >= a.rms_thr && flat <= a.flat_thr && conf >= a.conf_thr;
@@ -420,14 +453,18 @@ __global__ void at_target_kernel(const AtHoldArgs a) {
 __global__ void at_hold_kernel(const AtHoldArgs a) {
     const int clip = blockIdx.x * blockDim.x + threadIdx.x;
     if (clip >= a.batch) return;
-    const double *f = a.feat + (size_t)clip * a.frames * 4;
-    double *out = a.ratio + (size_t)clip * a.frames;
+    const AtClip c = at_clip(a, clip);
+    const int frames = (int)at_rows(c.n, a.hop);
+    if (frames == 0) return;
+    const long long r0 = at_row0(a.starts != nullptr, c, a.n, a.hop);
+    const double *f = a.feat + r0 * 4;
+    double *out = a.ratio + r0;
     double held = 0.0, cand = 0.0, last = 1.0;
     int cand_n = 0, rel = a.release_frames + 1;
     double tgt_n = out[0], p_n = f[2];                   // the next frame's inputs are loaded one step ahead
-    for (int i = 0; i < a.frames; ++i) {
+    for (int i = 0; i < frames; ++i) {
         const double tgt = tgt_n, p = p_n;
-        if (i + 1 < a.frames) { tgt_n = out[i + 1]; p_n = f[4 * (i + 1) + 2]; }
+        if (i + 1 < frames) { tgt_n = out[i + 1]; p_n = f[4 * (i + 1) + 2]; }
         const bool voiced = tgt > 0.0;                   // the target of a voiced frame is a positive frequency
         double r;
         if (voiced) {
@@ -483,14 +520,16 @@ QD_DEV float at_ratio_at(const double *ratio, int frames, long long n, int hop, 
 // Pass 1 (one thread per clip): the two delay taps, exactly the reference's sequential float64 accumulation with wraps
 // (dsp/autotune.py:327-337), plus the np.allclose(ratio, 1, atol=1e-3) early-out flag.  Pass 2 (wide): read-out.
 struct AtShiftArgs {
-    const float *body;       // [batch, n]
-    const double *ratio;     // [batch, frames]
-    long long *tile_sum;     // [batch, tiles] slope sums per 512-sample tile, then the tap at every tile start
-    float *ratio_track;      // optional [batch, n]
+    const float *body;       // packed like the batch
+    const double *ratio;     // [frame rows]
+    long long *tile_sum;     // [tile rows] (at_row0, unit AT_TS) slope sums per tile, then the tap at every tile start
+    float *ratio_track;      // optional, packed like the batch
     int *flat_flag;          // [batch] 1: ratio track allclose to 1 -> output = body
-    float *out;              // [batch, n] corrected body
-    long long n, tiles;      // tiles = ceil(n / 512)
-    int batch, frames, hop, half;
+    float *out;              // corrected body, packed like the batch
+    long long n;
+    const int64_t *starts;
+    const int32_t *lengths;
+    int clip0, hop, half;
     int max_delay, buf_size;
 };
 
@@ -526,38 +565,42 @@ struct AtTileCtx {
     AtSeg sg;                // the np.interp segment of the whole tile (aligned tiles only)
     bool aligned;
     double r_last;
+    long long n;             // the clip's samples and frames
+    int frames;
 };
 QD_DEV long long at_slope(const AtShiftArgs &a, const double *__restrict__ ratio, const AtTileCtx &c, long long i, float *r_out) {
     float r;
-    if (!c.aligned) r = at_ratio_at(ratio, a.frames, a.n, a.hop, a.half, i);
-    else if (i == a.n - 1) r = (float)c.r_last;                 // the last sample sits on the (repeated) last centre
+    if (!c.aligned) r = at_ratio_at(ratio, c.frames, c.n, a.hop, a.half, i);
+    else if (i == c.n - 1) r = (float)c.r_last;                 // the last sample sits on the (repeated) last centre
     else if ((double)i == c.sg.x0) r = (float)c.sg.y0;
     else r = (float)__dadd_rn(__dmul_rn(c.sg.slope, (double)i - c.sg.x0), c.sg.y0);
     *r_out = r;
     return (long long)((1.0 - (double)fminf(fmaxf(r, 0.5f), 2.0f)) * (double)(1ll << 24));   // exact: a multiple of 2^-24
 }
-QD_DEV AtTileCtx at_tile_ctx(const AtShiftArgs &a, const double *__restrict__ ratio, long long i0) {
-    AtTileCtx c{AtSeg{0.0, 1.0, 0.0}, false, ratio[a.frames - 1]};
+QD_DEV AtTileCtx at_tile_ctx(const AtShiftArgs &a, const double *__restrict__ ratio, long long n, long long i0) {
+    const int frames = (int)at_rows(n, a.hop);
+    AtTileCtx c{AtSeg{0.0, 1.0, 0.0}, false, ratio[frames - 1], n, frames};
     c.aligned = (a.hop % AT_TS) == 0 && (a.half % AT_TS) == 0 && (a.max_delay % 4) == 0;
-    if (c.aligned) c.sg = at_segment_at(ratio, a.frames, a.n, a.hop, a.half, i0);
+    if (c.aligned) c.sg = at_segment_at(ratio, frames, n, a.hop, a.half, i0);
     return c;
 }
 
 // (a tile holds no frame centre strictly inside when hop and frame_size / 2 are multiples of the tile: 512 | 512, 2048)
 __global__ void __launch_bounds__(32 * AT_TW) at_tap_sums_kernel(const AtShiftArgs a) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int clip = blockIdx.y;
+    const AtClip c = at_clip(a, blockIdx.y);
     const long long tile = (long long)blockIdx.x * AT_TW + warp;
-    if (tile >= a.tiles) return;
-    const double *__restrict__ ratio = a.ratio + (size_t)clip * a.frames;
-    float *__restrict__ rt = a.ratio_track ? a.ratio_track + (size_t)clip * a.n : nullptr;
-    const AtTileCtx cx = at_tile_ctx(a, ratio, tile * AT_TS);
+    if (tile >= at_rows(c.n, AT_TS)) return;
+    const bool rg = a.starts != nullptr;
+    const double *__restrict__ ratio = a.ratio + at_row0(rg, c, a.n, a.hop);
+    float *__restrict__ rt = a.ratio_track ? a.ratio_track + c.base : nullptr;
+    const AtTileCtx cx = at_tile_ctx(a, ratio, c.n, tile * AT_TS);
     bool flat = true;
     long long run = 0;
 #pragma unroll 4
     for (int k = 0; k < AT_SPL; ++k) {
         const long long i = tile * AT_TS + (long long)lane * AT_SPL + k;
-        if (i < a.n) {
+        if (i < c.n) {
             float r;
             run += at_slope(a, ratio, cx, i, &r);
             if (rt) rt[i] = r;
@@ -568,21 +611,22 @@ __global__ void __launch_bounds__(32 * AT_TW) at_tap_sums_kernel(const AtShiftAr
     for (int d = 16; d > 0; d >>= 1) run += __shfl_xor_sync(QD_FULL, run, d);
     flat = __all_sync(QD_FULL, flat);
     if (lane == 0) {
-        a.tile_sum[(size_t)clip * a.tiles + tile] = run;
-        if (!flat) a.flat_flag[clip] = 1;                // zeroed before the launch: "some tile is not flat" until the scan
+        a.tile_sum[at_row0(rg, c, a.n, AT_TS) + tile] = run;
+        if (!flat) a.flat_flag[c.idx] = 1;               // zeroed before the launch: "some tile is not flat" until the scan
     }
 }
 
 // tile_sum -> tap 0 at the start of every tile (in [0, M)); flat_flag -> 1 when no tile of the clip raised it
 __global__ void __launch_bounds__(32) at_tap_scan_kernel(const AtShiftArgs a) {
     const int lane = threadIdx.x;
-    const int clip = blockIdx.x;
-    long long *ts = a.tile_sum + (size_t)clip * a.tiles;
+    const AtClip c = at_clip(a, blockIdx.x);
+    const long long tiles = at_rows(c.n, AT_TS);
+    long long *ts = a.tile_sum + at_row0(a.starts != nullptr, c, a.n, AT_TS);
     const long long M = (long long)a.max_delay << 24;
     long long carry = M / 4;                             // tap 0 starts at 0.25 * max_delay
-    for (long long t0 = 0; t0 < a.tiles; t0 += 32) {
+    for (long long t0 = 0; t0 < tiles; t0 += 32) {
         const long long t = t0 + lane;
-        const long long v = t < a.tiles ? ts[t] : 0;
+        const long long v = t < tiles ? ts[t] : 0;
         long long inc = v;
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) {
@@ -592,12 +636,12 @@ __global__ void __launch_bounds__(32) at_tap_scan_kernel(const AtShiftArgs a) {
         long long start = carry + (inc - v);             // 32 tiles move a tap by at most 2^38 units: a few wraps
         while (start < 0) start += M;
         while (start >= M) start -= M;
-        if (t < a.tiles) ts[t] = start;
+        if (t < tiles) ts[t] = start;
         carry += __shfl_sync(QD_FULL, inc, 31);
         while (carry < 0) carry += M;
         while (carry >= M) carry -= M;
     }
-    if (lane == 0) a.flat_flag[clip] = a.flat_flag[clip] ? 0 : 1;   // from "some tile is not flat" to "the clip is flat"
+    if (lane == 0) a.flat_flag[c.idx] = a.flat_flag[c.idx] ? 0 : 1;   // from "some tile is not flat" to "the clip is flat"
 }
 
 // read-out with the latency trim folded in: out = raw[lat:] ++ zeros(lat) unless the early-out copied the body
@@ -606,27 +650,29 @@ __global__ void __launch_bounds__(32) at_tap_scan_kernel(const AtShiftArgs a) {
 __global__ void __launch_bounds__(32 * AT_TW) at_shift_kernel(const AtShiftArgs a) {
     __shared__ float s_out[AT_TW][AT_TS + AT_TS / 16];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int clip = blockIdx.y;
+    const AtClip c = at_clip(a, blockIdx.y);
+    const long long n = c.n;
     const long long tile = (long long)blockIdx.x * AT_TW + warp;
-    if (tile >= a.tiles) return;
+    if (tile >= at_rows(n, AT_TS)) return;
     const long long i0 = tile * AT_TS;
-    const float *__restrict__ x = a.body + (size_t)clip * a.n;
-    float *__restrict__ out = a.out + (size_t)clip * a.n;
-    if (a.flat_flag[clip] != 0) {
-        for (long long i = i0 + lane; i < i0 + AT_TS && i < a.n; i += 32) out[i] = x[i];
+    const float *__restrict__ x = a.body + c.base;
+    float *__restrict__ out = a.out + c.base;
+    if (a.flat_flag[c.idx] != 0) {
+        for (long long i = i0 + lane; i < i0 + AT_TS && i < n; i += 32) out[i] = x[i];
         return;
     }
-    const long long lat = a.n > a.max_delay / 2 ? a.max_delay / 2 : 0;
-    const double *__restrict__ ratio = a.ratio + (size_t)clip * a.frames;
+    const long long lat = n > a.max_delay / 2 ? a.max_delay / 2 : 0;
+    const bool rg = a.starts != nullptr;
+    const double *__restrict__ ratio = a.ratio + at_row0(rg, c, a.n, a.hop);
     const long long unit = 1ll << 24;
     const long long M = (long long)a.max_delay * unit, half_m = M / 2;   // the second tap runs half a grain behind
-    const AtTileCtx cx = at_tile_ctx(a, ratio, i0);
+    const AtTileCtx cx = at_tile_ctx(a, ratio, n, i0);
     long long run = 0;                                   // the lane's 16 slopes: summed here, walked again below
 #pragma unroll 4
     for (int k = 0; k < AT_SPL; ++k) {
         const long long i = i0 + (long long)lane * AT_SPL + k;
         float r;
-        if (i < a.n) run += at_slope(a, ratio, cx, i, &r);
+        if (i < n) run += at_slope(a, ratio, cx, i, &r);
     }
     long long incl = run;
 #pragma unroll
@@ -634,7 +680,7 @@ __global__ void __launch_bounds__(32 * AT_TW) at_shift_kernel(const AtShiftArgs 
         const long long o = __shfl_up_sync(QD_FULL, incl, d);
         if (lane >= d) incl += o;
     }
-    long long tap = a.tile_sum[(size_t)clip * a.tiles + tile] + (incl - run);   // tap 0 before the lane's first sample, unwrapped
+    long long tap = a.tile_sum[at_row0(rg, c, a.n, AT_TS) + tile] + (incl - run);   // tap 0 before the lane's first sample, unwrapped
     const double md = (double)a.max_delay, size = (double)a.buf_size;
     const int mask = a.buf_size - 1;
     float *so = s_out[warp];
@@ -642,11 +688,11 @@ __global__ void __launch_bounds__(32 * AT_TW) at_shift_kernel(const AtShiftArgs 
     for (int k = 0; k < AT_SPL; ++k) {
         const long long i = i0 + (long long)lane * AT_SPL + k;
         float val = 0.0f;
-        if (i < a.n) {
+        if (i < n) {
             float r;
             tap += at_slope(a, ratio, cx, i, &r);        // |tap| stays below M + 2^34: a few wraps at most
         }
-        if (i < a.n && i >= lat) {
+        if (i < n && i >= lat) {
             long long t0 = tap;
             while (t0 < 0) t0 += M;
             while (t0 >= M) t0 -= M;
@@ -678,21 +724,24 @@ __global__ void __launch_bounds__(32 * AT_TW) at_shift_kernel(const AtShiftArgs 
     __syncwarp();
     for (int j = lane; j < AT_TS; j += 32) {
         const long long i = i0 + j;
-        if (i >= a.n) break;
-        if (i >= a.n - lat) out[i] = 0.0f;               // the tail that no shifted sample reaches
+        if (i >= n) break;
+        if (i >= n - lat) out[i] = 0.0f;               // the tail that no shifted sample reaches
         if (i >= lat) out[i - lat] = so[j + j / AT_SPL];
     }
 }
 
 // ---------------------------------------------------------------- sub layer and final mix
 struct AtMixArgs {
-    const float *x, *sub, *air, *corrected;
-    float *env;              // [batch, n] scratch
+    const float *x, *sub, *air, *corrected;   // packed like the batch, as are env, sub_layer and y
+    float *env;              // scratch
     float *env_max;          // [batch]
-    float *sub_layer;        // optional [batch, n]
-    float *y;                // [batch, n] autotune output
+    float *sub_layer;        // optional
+    float *y;                // autotune output
     long long n;
-    int batch;
+    long long seg_min;       // clips of at least seg_min samples take at_env_seg_kernel, shorter ones at_env_kernel
+    const int64_t *starts;
+    const int32_t *lengths;
+    int clip0, batch;
     int sub_enabled;         // cfg.sub_enabled
     int layer_on;            // sub_enabled and sub_level > 0 and freq > 0
     float att, rel;          // float32(exp(-1/(ms*sr/1000)))
@@ -706,22 +755,25 @@ __global__ void __launch_bounds__(32 * AT_FW) at_env_kernel(const AtMixArgs a) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int clip = blockIdx.x * AT_FW + warp;
     if (clip >= a.batch) return;
-    const float *__restrict__ x = a.x + (size_t)clip * a.n;
-    float *__restrict__ env = a.env + (size_t)clip * a.n;
+    const AtClip c = at_clip(a, clip);
+    if (c.n >= a.seg_min) return;
+    const long long n = c.n;
+    const float *__restrict__ x = a.x + c.base;
+    float *__restrict__ env = a.env + c.base;
     float *io = s_io[warp];
     constexpr int PER = AT_TS / 32;
     float nxt[PER];
     float cur = 0.0f, top = 0.0f;
 #pragma unroll
-    for (int k = 0; k < PER; ++k) io[lane + 32 * k] = lane + 32 * k < a.n ? x[lane + 32 * k] : 0.0f;
+    for (int k = 0; k < PER; ++k) io[lane + 32 * k] = lane + 32 * k < n ? x[lane + 32 * k] : 0.0f;
     __syncwarp();
-    for (long long i0 = 0; i0 < a.n; i0 += AT_TS) {
-        const bool more = i0 + AT_TS < a.n;
+    for (long long i0 = 0; i0 < n; i0 += AT_TS) {
+        const bool more = i0 + AT_TS < n;
         if (more) {
 #pragma unroll
-            for (int k = 0; k < PER; ++k) { const long long i = i0 + AT_TS + lane + 32 * k; nxt[k] = i < a.n ? x[i] : 0.0f; }
+            for (int k = 0; k < PER; ++k) { const long long i = i0 + AT_TS + lane + 32 * k; nxt[k] = i < n ? x[i] : 0.0f; }
         }
-        const int cnt = (int)(a.n - i0 < AT_TS ? a.n - i0 : AT_TS);
+        const int cnt = (int)(n - i0 < AT_TS ? n - i0 : AT_TS);
         if (lane == 0) {
             for (int k = 0; k < cnt; ++k) {
                 const float s = fabsf(io[k]);
@@ -740,7 +792,7 @@ __global__ void __launch_bounds__(32 * AT_FW) at_env_kernel(const AtMixArgs a) {
         }
         __syncwarp();
     }
-    if (lane == 0) a.env_max[clip] = top;
+    if (lane == 0) a.env_max[c.idx] = top;
 }
 
 // The same follower, segment-parallel: both branches of the recurrence pull `cur` towards |x| by a factor of at least
@@ -752,10 +804,11 @@ __global__ void __launch_bounds__(32 * AT_FW) at_env_kernel(const AtMixArgs a) {
 __global__ void __launch_bounds__(32 * AT_SW) at_env_seg_kernel(const AtMixArgs a, int tile, int halo) {
     __shared__ float s_row[AT_SW][32][33];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int clip = blockIdx.y;
-    const long long n = a.n;
-    const float *__restrict__ x = a.x + (size_t)clip * n;
-    float *__restrict__ env = a.env + (size_t)clip * n;
+    const AtClip c = at_clip(a, blockIdx.y);
+    const long long n = c.n;
+    if (n < a.seg_min) return;
+    const float *__restrict__ x = a.x + c.base;
+    float *__restrict__ env = a.env + c.base;
     const long long n_tiles = (n + tile - 1) / tile;
     const long long tile0 = ((long long)blockIdx.x * AT_SW + warp) * 32;
     if (tile0 >= n_tiles) return;
@@ -820,14 +873,14 @@ __global__ void __launch_bounds__(32 * AT_SW) at_env_seg_kernel(const AtMixArgs 
         __syncwarp();
     }
     top = warp_max(top);
-    if (lane == 0) atomicMax(reinterpret_cast<int *>(a.env_max + clip), __float_as_int(top));
+    if (lane == 0) atomicMax(reinterpret_cast<int *>(a.env_max + c.idx), __float_as_int(top));
 }
 
 __global__ void at_mix_kernel(const AtMixArgs a) {
-    const int clip = blockIdx.y;
-    const size_t base = (size_t)clip * a.n;
-    const float top = a.layer_on ? a.env_max[clip] : 0.0f;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < a.n; i += (long long)gridDim.x * blockDim.x) {
+    const AtClip c = at_clip(a, blockIdx.y);
+    const long long base = c.base;
+    const float top = a.layer_on ? a.env_max[c.idx] : 0.0f;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < c.n; i += (long long)gridDim.x * blockDim.x) {
         float layer = 0.0f;
         if (a.layer_on) {
             float e = a.env[base + i];

@@ -233,4 +233,27 @@ QD_DEV ClipSpan clip_span(const A &a, int c) {
     return {(long long)c * (long long)a.n, (int)a.n};
 }
 
+// The autotune_v1 kernels (qd_autotune.cuh, qd_yin.cuh) take optional per-clip arrays `starts` / `lengths` (a ragged
+// batch, as SpecArgsT::starts; null: uniform clips of n samples at i * n).  n is the longest clip, which sizes the
+// grids.  Unlike clip_span's callers they advance clip0 at launch splits in uniform batches too, so per-clip arrays
+// are indexed by clip0 + c and no pointer moves.
+struct AtClip { int idx; long long base, n; };
+template <class A>
+QD_DEV AtClip at_clip(const A &a, int c) {
+    if (a.starts) {
+        const ClipSpan s = clip_span(a, c);
+        return {a.clip0 + c, s.base, (long long)s.n};
+    }
+    const int i = a.clip0 + c;
+    return {i, (long long)i * a.n, a.n};
+}
+// Per-clip tables with one row per `unit` samples (detector frames: unit = hop, ceil(n / hop) frames per clip;
+// delay-tap tiles: unit = AT_TS).  Uniform batches keep clip i at row i * rows(n).  Ragged batches put it at
+// floor(base / unit) + i: no scan, valid for any sub-range of clips, and rows of consecutive clips cannot overlap
+// because starts[i + 1] >= starts[i] + n_i.  So a ragged batch has at most span / unit + batch rows.
+__host__ __device__ inline long long at_rows(long long n, int unit) { return (n + unit - 1) / unit; }
+QD_DEV long long at_row0(bool ragged, const AtClip &c, long long n_uniform, int unit) {
+    return ragged ? c.base / unit + c.idx : (long long)c.idx * at_rows(n_uniform, unit);
+}
+
 }  // namespace qd

@@ -38,12 +38,16 @@
 namespace qd {
 
 struct AtYinArgs {
-    const float *det;        // [batch, n]
-    double *diff;            // [batch, frames, stride] difference function, entry tau
-    double *feat;            // [batch, frames, 4]; feat[2] holds 1 / 0 (frame not silent) on entry of the pick kernel
+    const float *det;        // packed like the batch (qd_autotune.cuh: at_clip)
+    double *diff;            // [frame rows, stride] difference function, entry tau (frame rows: at_row0)
+    double *feat;            // [frame rows, 4]; feat[2] holds 1 / 0 (frame not silent) on entry of the pick kernel
     long long n;
-    long long total_frames;  // batch * frames
-    int frames, frame_size, hop, stride;
+    long long total_frames;  // frame rows of the batch
+    const int64_t *starts;   // optional ragged batch
+    const int32_t *lengths;
+    int clip0;
+    int frames;              // ceil(n / hop), the longest clip's; the kernels derive every clip's own
+    int frame_size, hop, stride;
     int min_tau, max_tau;
     int lag_threads;         // columns (of AT_YL lags) per CTA, <= AT_YC
     double sr, min_freq, max_freq, threshold;
@@ -135,9 +139,12 @@ __global__ void __launch_bounds__(AT_YT, 1) at_yin_diff_kernel(const AtYinArgs a
     double *ebq = be + 16;                              // [16] ebq[q] = energy of the q blocks before the one being assembled
     uint64_t *mbar = reinterpret_cast<uint64_t *>(ebq + 16);   // full[3] (helpers -> walkers), done[3] (walkers -> helpers)
     int *lagc = reinterpret_cast<int *>(mbar + 2 * AT_YNS);      // [L * cols] per lag: off | q << 12 | group << 16 | live << 20
-    const float *x = a.det + (size_t)blockIdx.y * a.n;
-    double *out = a.diff + (size_t)blockIdx.y * a.frames * a.stride;
-    const int blocks = a.frames + W / hop;
+    const AtClip clip = at_clip(a, blockIdx.y);
+    const long long n = clip.n;
+    const int frames = (int)at_rows(n, hop);
+    const float *x = a.det + clip.base;
+    double *out = a.diff + at_row0(a.starts != nullptr, clip, a.n, hop) * a.stride;
+    const int blocks = frames + W / hop;
     const int n_all = hop / L;                          // iterations per block, split over the G groups as evenly as possible
     auto group_begin = [&](int g) { return g * (n_all / G) + min(g, n_all % G); };
     uint64_t *full = mbar, *done = mbar + AT_YNS;
@@ -231,14 +238,14 @@ __global__ void __launch_bounds__(AT_YT, 1) at_yin_diff_kernel(const AtYinArgs a
             for (int r = 0; r < PF; ++r) {
                 const int i = h + r * AT_YH;
                 const long long sidx = j0 + B0 + i;
-                pf[r] = (i < span && sidx < a.n) ? x[sidx] : 0.0f;
+                pf[r] = (i < span && sidx < n) ? x[sidx] : 0.0f;
             }
             if (c0 > 0) {
 #pragma unroll
                 for (int r = 0; r < PFO; ++r) {
                     const int i = h + r * AT_YH;
                     const long long sidx = j0 + i;
-                    pfo[r] = (i < hop && sidx < a.n) ? x[sidx] : 0.0f;
+                    pfo[r] = (i < hop && sidx < n) ? x[sidx] : 0.0f;
                 }
             }
         };
@@ -295,7 +302,7 @@ __global__ void __launch_bounds__(AT_YT, 1) at_yin_diff_kernel(const AtYinArgs a
             }
             for (int i = h + PF * AT_YH; i < span; i += AT_YH) {
                 const long long sidx = (long long)b * hop + B0 + i;
-                tl[(i % L) * Q + i / L] = sidx < a.n ? (double)x[sidx] : 0.0;
+                tl[(i % L) * Q + i / L] = sidx < n ? (double)x[sidx] : 0.0;
             }
             if (c0 > 0) {
 #pragma unroll
@@ -305,7 +312,7 @@ __global__ void __launch_bounds__(AT_YT, 1) at_yin_diff_kernel(const AtYinArgs a
                 }
                 for (int i = h + PFO * AT_YH; i < hop; i += AT_YH) {
                     const long long sidx = (long long)b * hop + i;
-                    ow[i] = sidx < a.n ? (double)x[sidx] : 0.0;
+                    ow[i] = sidx < n ? (double)x[sidx] : 0.0;
                 }
             }
             helper_sync();
@@ -352,7 +359,7 @@ __global__ void __launch_bounds__(AT_YT, 1) at_yin_diff_kernel(const AtYinArgs a
                 const double v = ((rv[0] + rv[1]) + (rv[2] + rv[3])) + ((rv[4] + rv[5]) + (rv[6] + rv[7]));
                 const int tr = 1 + col;                                                  // tau relative to the lagged range
                 const double qtau = qv(tr);
-                if ((lc >> 20) && f >= 0 && f < a.frames) {
+                if ((lc >> 20) && f >= 0 && f < frames) {
                     const double e1 = ebq[qq] + (c0 == 0 ? qv(off) : qown[off]);         // E(s, p)
                     const double cur = (qv(off + tr) - qtau) - 2.0 * pu;                 // the partial block: E(. + tau) - 2 R
                     out[(size_t)f * a.stride + tau] = fmax(e1 + (v + cur), 0.0);

@@ -318,14 +318,74 @@ class AutotuneRenderer:
     def close(self) -> None:
         self._ws = None
 
-    def set_fx_seeds(self, batch: int, seeds=None, shard=None) -> None:   # no random stage in this mode
-        pass
+    def set_fx_seeds(self, batch: int, seeds=None, shard=None, frames: Optional[Sequence[int]] = None) -> None:
+        pass   # no random stage in this mode
 
     def render_device(self, x, want_taps: bool = False, debug: bool = False, chunk_clips: int = 2048):
         _torch()
         y, taps, dbg, self._ws = autotune.render_device(self.params, x, want_taps=want_taps, debug=debug,
                                                         chunk_clips=chunk_clips, workspace=self._ws)
         return (y, taps, dbg) if debug else (y, taps)
+
+    def render_device_varlen(self, x, starts, lengths, span: int, max_samples: int, want_taps: bool = False):
+        """Ragged batch on the device, as Renderer.render_device_varlen (autotune.render_device_varlen)."""
+        _torch()
+        y, taps, self._ws = autotune.render_device_varlen(self.params, x, starts, lengths, span, max_samples,
+                                                          want_taps=want_taps, workspace=self._ws)
+        return y, taps
+
+    def render_host_varlen(self, x_host, y_host, starts: np.ndarray, lengths: np.ndarray, chunk_samples: int = 0) -> None:
+        """Ragged batch in host memory, as Renderer.render_host_varlen: flat contiguous CPU tensors (float32 or int16
+        PCM16) with clip c at [starts[c] - starts[0], + lengths[c]).  Chunks are clip ranges whose packed span fits
+        ``chunk_samples`` (0: 128 clips of this renderer's length; a longer clip gets a chunk of its own), and the
+        copies overlap the kernels as in render_host.  Validates starts / lengths.  Synchronous."""
+        torch = _torch()
+        fmt = (torch.float32, torch.int16)
+        if x_host.dtype not in fmt or y_host.dtype not in fmt:
+            raise ValueError("host buffers must be float32 or int16 (PCM16)")
+        if (x_host.dim() != 1 or x_host.shape != y_host.shape or not x_host.is_contiguous()
+                or not y_host.is_contiguous()):
+            raise ValueError("x_host and y_host must be flat, contiguous and of the same length")
+        starts = np.ascontiguousarray(starts, dtype=np.int64)
+        lengths = np.ascontiguousarray(lengths, dtype=np.int32)
+        check_layout(starts, lengths, self.n)
+        autotune.check_lengths(self.params, lengths)
+        if not len(starts):
+            return
+        off = starts - starts[0]
+        ends = off + lengths
+        if int(ends[-1]) > int(x_host.shape[0]):
+            raise ValueError("the clips reach past the end of the host buffers")
+        budget = int(chunk_samples) if chunk_samples > 0 else 128 * max(1, self.n)
+        d_starts, d_lengths = torch.from_numpy(starts).cuda(), torch.from_numpy(lengths).cuda()
+        run = torch.cuda.current_stream()
+        if not hasattr(self, "_s_in"):
+            self._s_in, self._s_out = torch.cuda.Stream(), torch.cuda.Stream()
+        s_in, s_out = self._s_in, self._s_out
+        s_in.wait_stream(run)
+        c0 = 0
+        while c0 < len(starts):
+            c1 = c0 + 1
+            while c1 < len(starts) and ends[c1] - off[c0] <= budget:
+                c1 += 1
+            lo, hi = int(off[c0]), int(ends[c1 - 1])
+            with torch.cuda.stream(s_in):
+                xs = x_host[lo:hi].to("cuda", non_blocking=True)
+            run.wait_stream(s_in)
+            xs.record_stream(run)
+            if xs.dtype == torch.int16:
+                xs = xs.to(torch.float32) * (1.0 / 32768.0)
+            y, _ = self.render_device_varlen(xs.float(), d_starts[c0:c1], d_lengths[c0:c1], hi - lo,
+                                             int(lengths[c0:c1].max()))
+            if y_host.dtype == torch.int16:
+                y = torch.clamp(torch.round(y.double() * 32767.0), -32768.0, 32767.0).to(torch.int16)
+            s_out.wait_stream(run)
+            with torch.cuda.stream(s_out):
+                y_host[lo:hi].copy_(y, non_blocking=True)
+            y.record_stream(s_out)
+            c0 = c1
+        s_out.synchronize()
+        run.synchronize()
 
     def render_host(self, x_host, y_host, chunk_clips: int = 128) -> None:
         """Chunked H2D -> render -> D2H with the copies on their own streams, so that the transfers of chunk i+1 / i-1
@@ -539,63 +599,49 @@ def _ragged_batch(clips: List[Any], sr: int, n_fft: int, return_taps: bool, chun
     ys: List[Any] = [None] * len(clips)
     taps: Optional[Dict[str, List[Any]]] = {"pre_quant": [None] * len(clips), "post_dist": [None] * len(clips)} \
         if return_taps else None
+    live = [i for i in range(len(clips)) if lengths[i] > 0]
     if isinstance(r, AutotuneRenderer):
-        # no ragged autotune_v1 kernels: clips of one length are rendered as one uniform batch
-        groups: Dict[int, List[int]] = {}
-        for i, n in enumerate(lengths.tolist()):
-            groups.setdefault(n, []).append(i)
-        for n, idx in groups.items():
-            if n == 0:
-                continue
-            xb = np.stack([clips[i] for i in idx]) if is_np else torch.stack([clips[i] for i in idx])
-            yb, tb = process_batch(xb, sr, n_fft=n_fft, return_taps=return_taps, chunk_clips=chunk_clips, **kwargs)
-            for k, i in enumerate(idx):
-                ys[i] = yb[k]
-                if taps is not None:
-                    for name in taps:
-                        taps[name][i] = tb[name][k]
-    else:
-        live = [i for i in range(len(clips)) if lengths[i] > 0]
-        if live:
-            n_live = lengths[live]
-            hop = int(n_fft) // 4
-            r.set_fx_seeds(len(live), [seeds[i] for i in live] if isinstance(seeds, list) else seeds,
-                           frames=[1 + int(n) // hop for n in n_live])
-            starts, span = pack_layout(n_live, 2 if pcm else 4)
-            max_n = int(n_live.max())
-            ends = starts + n_live
-            if cuda:   # one concatenation on the device: clips and the zero gaps that align the next start
-                zero = torch.zeros(4, dtype=torch.float32, device="cuda")
-                pieces = []
-                for k, i in enumerate(live):
-                    pieces.append(clips[i].float())
-                    if k + 1 < len(live) and starts[k + 1] > ends[k]:
-                        pieces.append(zero[:int(starts[k + 1] - ends[k])])
-                xf = torch.cat(pieces)
-            else:      # packed once into page-locked memory: this copy is the H2D staging
-                xf = torch.empty(span, dtype=torch.int16 if pcm else torch.float32, pin_memory=True)
-                xn = xf.numpy()
-                for k, i in enumerate(live):
-                    xn[starts[k]:ends[k]] = clips[i] if is_np else clips[i].numpy()
-                    if k + 1 < len(live):
-                        xn[ends[k]:starts[k + 1]] = 0
-            if cuda or return_taps:
-                d_starts = torch.from_numpy(starts).cuda()
-                d_lengths = torch.from_numpy(n_live.astype(np.int32)).cuda()
-                yf, tf = r.render_device_varlen(xf if cuda else xf.cuda().float(), d_starts, d_lengths, span, max_n,
-                                                want_taps=return_taps)
-                if not cuda:
-                    yf, tf = yf.cpu(), {k: v.cpu() for k, v in tf.items()}
-            else:
-                yf, tf = torch.empty_like(xf, pin_memory=True), None
-                r.render_host_varlen(xf, yf, starts, n_live, chunk_samples=int(chunk_clips) * max(1, span // len(live)))
-            if is_np:
-                yf, tf = yf.numpy(), (None if tf is None else {k: v.numpy() for k, v in tf.items()})
+        autotune.check_lengths(r.params, lengths)
+    if live:
+        n_live = lengths[live]
+        hop = int(n_fft) // 4
+        r.set_fx_seeds(len(live), [seeds[i] for i in live] if isinstance(seeds, list) else seeds,
+                       frames=[1 + int(n) // hop for n in n_live])
+        starts, span = pack_layout(n_live, 2 if pcm else 4)
+        max_n = int(n_live.max())
+        ends = starts + n_live
+        if cuda:   # one concatenation on the device: clips and the zero gaps that align the next start
+            zero = torch.zeros(4, dtype=torch.float32, device="cuda")
+            pieces = []
             for k, i in enumerate(live):
-                ys[i] = yf[starts[k]:ends[k]]
-                if taps is not None:
-                    for name in taps:
-                        taps[name][i] = tf[name][starts[k]:ends[k]]
+                pieces.append(clips[i].float())
+                if k + 1 < len(live) and starts[k + 1] > ends[k]:
+                    pieces.append(zero[:int(starts[k + 1] - ends[k])])
+            xf = torch.cat(pieces)
+        else:      # packed once into page-locked memory: this copy is the H2D staging
+            xf = torch.empty(span, dtype=torch.int16 if pcm else torch.float32, pin_memory=True)
+            xn = xf.numpy()
+            for k, i in enumerate(live):
+                xn[starts[k]:ends[k]] = clips[i] if is_np else clips[i].numpy()
+                if k + 1 < len(live):
+                    xn[ends[k]:starts[k + 1]] = 0
+        if cuda or return_taps:
+            d_starts = torch.from_numpy(starts).cuda()
+            d_lengths = torch.from_numpy(n_live.astype(np.int32)).cuda()
+            yf, tf = r.render_device_varlen(xf if cuda else xf.cuda().float(), d_starts, d_lengths, span, max_n,
+                                            want_taps=return_taps)
+            if not cuda:
+                yf, tf = yf.cpu(), {k: v.cpu() for k, v in tf.items()}
+        else:
+            yf, tf = torch.empty_like(xf, pin_memory=True), None
+            r.render_host_varlen(xf, yf, starts, n_live, chunk_samples=int(chunk_clips) * max(1, span // len(live)))
+        if is_np:
+            yf, tf = yf.numpy(), (None if tf is None else {k: v.numpy() for k, v in tf.items()})
+        for k, i in enumerate(live):
+            ys[i] = yf[starts[k]:ends[k]]
+            if taps is not None:
+                for name in taps:
+                    taps[name][i] = tf[name][starts[k]:ends[k]]
     for i in range(len(clips)):
         if ys[i] is None:   # zero-length clip: not rendered, consumes no FX draws
             ys[i] = empty()
@@ -613,12 +659,12 @@ def process_batch(x, sr: int = DEFAULT_SAMPLE_RATE, *, n_fft: int = N_FFT_DEFAUL
     or all CUDA tensors, floating point or all int16 (PCM16, host only).  The result is a list of the same kind, and
     the taps (``return_taps``) a dict of lists; a zero-length clip comes back empty.  Each clip renders exactly as it
     would alone: the STFT path packs the clips into one flat buffer and renders them in one call
-    (qd_render_*_varlen), with a plan sized for the longest clip and ``chunk_clips`` clips of mean length per host
-    chunk.  Random spectral FX always get one table per clip, replayed over that clip's own frames: seeds=None
-    draws clip after clip in list order (a loop of process_audio calls), an int reseeds before every clip, a list
-    gives one seed per clip.  ``shard`` and ``out`` are not supported with a list.  ``quantize_mode="autotune_v1"``
-    has no ragged kernels: the clips are grouped by length and each group is rendered as a uniform batch -- the
-    results are the same, but nothing gets faster than one call per distinct length.
+    (qd_render_*_varlen, and qd_autotune_render_device_varlen in ``quantize_mode="autotune_v1"``), sized for the
+    longest clip, with ``chunk_clips`` clips of mean length per host chunk.  Random spectral FX always get one table
+    per clip, replayed over that clip's own frames: seeds=None draws clip after clip in list order (a loop of
+    process_audio calls), an int reseeds before every clip, a list gives one seed per clip.  ``shard`` and ``out``
+    are not supported with a list.  In ``autotune_v1`` with the pitch stage on, a clip of 1..15 samples raises the
+    ValueError it raises alone.
 
     ``seeds`` controls the np.random replay of the random spectral FX (None: consume the global state clip by
     clip like a loop of reference calls; int: reseed before every clip; list: one seed per clip); ``shard=(lo, hi,
