@@ -1,5 +1,7 @@
 // tests/emu/cuda_emu_at.h -- TEST INFRASTRUCTURE: the few CUDA intrinsics the autotune_v1 kernels use beyond
-// cuda_emu.h (warp votes, find-first-set, float division rounded to nearest, the float bits of the envelope maximum).
+// cuda_emu.h (warp votes, find-first-set, float division rounded to nearest, the float bits of the envelope maximum,
+// the fast float32 logarithm of the flatness).  The shuffles of cuda_emu.h already move any 8-byte type (long long taps,
+// double scans); sinf, exp, log2, exp2, fmod and rint are the C library's.
 // Included after cuda_emu.h and before the kernel headers by tests/emu/emu_at_ragged.cpp.
 #pragma once
 #include "cuda_emu.h"
@@ -19,3 +21,7 @@ static inline int atomicMax(int *p, int v) {
     return old;
 }
 static inline int __float_as_int(float f) { int u; std::memcpy(&u, &f, 4); return u; }
+// lg2.approx.f32 on the device (~2^-22 relative); the frame-stats test bounds the flatness at 1e-4 relative
+// (glibc declares its own __log2f, hence the rename)
+static inline float qd_emu_log2f(float x) { return std::log2(x); }
+#define __log2f qd_emu_log2f

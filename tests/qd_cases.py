@@ -561,3 +561,22 @@ def harness_extra_params(name):
         from quantumdistortion_b200.presets import spectral_fx_preset_kwargs
         return dict(_MB, **spectral_fx_preset_kwargs(ep[1]))
     return dict(ep)
+
+
+def flatness_interval(frame, rtol: float = 1e-4):
+    """Where a float32 FFT may put the spectral flatness of one detector frame (dsp/autotune.py:130-137, symmetric
+    Hann): every bin of a float32 FFT of length N may move by up to delta = eps32 log2(N) ||frame * window||_2, so the
+    flatness lies between that of max(|X| - delta, 0) and that of |X| + delta (float64 |X|), widened by rtol for the
+    float32 logarithm and sums.  On a frame whose spectrum sits well above delta everywhere this is rtol itself; on a
+    band-limited, tonal frame (the detector band above 3 kHz) the stopband bins hold only the FFT's rounding noise and
+    the flatness is that noise's: a float32 FFT moves it by up to 160 % (4.6e-6 -> 1.1e-5 measured on the B200)."""
+    frame = np.asarray(frame, dtype=np.float64)
+    xw = frame * np.hanning(len(frame))
+    mag = np.abs(np.fft.rfft(xw))
+    delta = float(np.finfo(np.float32).eps) * np.log2(len(frame)) * float(np.linalg.norm(xw))
+
+    def flat(m):
+        spec = m + 1e-8
+        ari = float(np.mean(spec))
+        return 1.0 if ari <= 1e-8 else float(np.exp(np.mean(np.log(spec)))) / ari
+    return flat(np.maximum(mag - delta, 0.0)) * (1.0 - rtol), flat(mag + delta) * (1.0 + rtol)
