@@ -17,7 +17,8 @@
  *
  * All functions return 0 on success or a negative qd_status; qd_last_error() gives a
  * thread-local message.  All "device" pointers are CUDA device pointers on the
- * current device; `stream` is a cudaStream_t passed as void*.
+ * current device; `stream` is a cudaStream_t passed as void*.  The device entry
+ * points take at most 2^31 - 1 clips per call (more: QD_ERR_INVALID_ARG).
  */
 #ifndef QD_B200_H
 #define QD_B200_H

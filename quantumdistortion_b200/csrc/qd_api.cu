@@ -77,8 +77,6 @@ struct qd_plan {
     int64_t fx_tables = 0;
     HostPipe pipe;
     int sm_count = 148;
-    int clip_offset = 0;       // first clip of the current render inside a per-clip FX table
-    void *frozen_ws = nullptr; // slice of the render workspace: frame-0 magnitudes (spectral freeze)
     qd::TeamGather team_tg{};  // gather lists of the team kernel (long frames, plain passes); team_nf = 0: not used
     int team_nf = 0, team_cw = 0;
     size_t team_smem = 0;
@@ -99,6 +97,7 @@ struct Packing {
     const int32_t *lengths = nullptr;
     int64_t span = 0;
     int max_n = 0;
+    int64_t clip_offset = 0;   // row of clip 0 in a per-clip FX table (qd_render_host: the chunk's first clip)
 };
 // intermediates of a render ([x_dist], [low], [high]) use the packing of x, each padded to 256 bytes
 size_t padded_span(int64_t span) { return ((size_t)span + 63) & ~(size_t)63; }
@@ -223,7 +222,7 @@ int launch_freeze(int nc, const qd::SpecArgsT<T> &a, T *out, int64_t batch, cuda
 
 template <class T>
 int launch_spec_prec(qd_plan *pl, qd::SpecArgsT<T> a, const Packing &pk, const float *src, float *dst, float *tap, int quant,
-                     int epilogue, int64_t batch, cudaStream_t st, int fx_pass, int clip_offset, float *clip_peak) {
+                     int epilogue, int64_t batch, cudaStream_t st, int fx_pass, float *clip_peak, void *frozen_ws) {
     a.starts = pk.starts;
     a.lengths = pk.lengths;
     a.clip0 = 0;
@@ -237,7 +236,7 @@ int launch_spec_prec(qd_plan *pl, qd::SpecArgsT<T> a, const Packing &pk, const f
     a.epilogue = epilogue;
     const bool fx = quant && (pl->p.fx_mode != QD_FX_NONE || pl->p.spectral_freeze || pl->p.formant_ratio > 0.0);
     a.fx.pass = fx_pass;
-    a.fx.clip_offset = clip_offset;
+    a.fx.clip_offset = (int)pk.clip_offset;
     a.fx.table = pl->fx_table;
     // a pass that does not run the FX uses the plain kernel of the same warp count
     int nw = fx ? pl->nw : pick_nw<T>(pl->nc, false) == 16 && !pl->ts ? 8 : pick_nw<T>(pl->nc, false);
@@ -267,7 +266,7 @@ int launch_spec_prec(qd_plan *pl, qd::SpecArgsT<T> a, const Packing &pk, const f
     a.frozen = nullptr;
     if (fx && pl->p.spectral_freeze) {
         // frame-0 magnitudes of THIS pass's input (each quantised pass freezes its own first frame)
-        T *frozen = reinterpret_cast<T *>(pl->frozen_ws);
+        T *frozen = reinterpret_cast<T *>(frozen_ws);
         int rc = launch_freeze<T>(pl->nc, a, frozen, batch, st);
         if (rc != QD_OK) return rc;
         a.frozen = frozen;
@@ -278,12 +277,13 @@ int launch_spec_prec(qd_plan *pl, qd::SpecArgsT<T> a, const Packing &pk, const f
     (void)nw;
 }
 
-// One spectral pass over [batch, n]: src -> dst (+ optional tap of the pre-epilogue signal).
+// One spectral pass over [batch, n]: src -> dst (+ optional tap of the pre-epilogue signal).  frozen_ws: the render
+// workspace's scratch for the frame-0 magnitudes of the spectral freeze.
 int launch_spec(qd_plan *pl, const Packing &pk, const float *src, float *dst, float *tap, int quant, int epilogue,
-                int64_t batch, cudaStream_t st, int fx_pass = 0, int clip_offset = 0, float *clip_peak = nullptr) {
+                int64_t batch, cudaStream_t st, int fx_pass = 0, float *clip_peak = nullptr, void *frozen_ws = nullptr) {
     TimeScope ts(pl, st, QD_KERNEL_SPECTRAL);
-    if (pl->f64) return launch_spec_prec<double>(pl, pl->spec64, pk, src, dst, tap, quant, epilogue, batch, st, fx_pass, clip_offset, clip_peak);
-    return launch_spec_prec<float>(pl, pl->spec, pk, src, dst, tap, quant, epilogue, batch, st, fx_pass, clip_offset, clip_peak);
+    if (pl->f64) return launch_spec_prec<double>(pl, pl->spec64, pk, src, dst, tap, quant, epilogue, batch, st, fx_pass, clip_peak, frozen_ws);
+    return launch_spec_prec<float>(pl, pl->spec, pk, src, dst, tap, quant, epilogue, batch, st, fx_pass, clip_peak, frozen_ws);
 }
 
 int launch_limiter(const qd::LimiterArgs &a, int64_t batch, cudaStream_t st) {
@@ -291,21 +291,11 @@ int launch_limiter(const qd::LimiterArgs &a, int64_t batch, cudaStream_t st) {
     const size_t smem = qd_host::limiter_smem_bytes(a.lookahead);
     if (smem > 200 * 1024) return fail(QD_ERR_UNSUPPORTED, "limiter lookahead too long");
     if (int rc_ = ensure_dyn_smem(qd::limiter_mix_kernel, attr_mask, 200 * 1024)) return rc_;
-    for (int64_t b0 = 0; b0 < batch; b0 += (1 << 30)) {
-        const int64_t nb = std::min<int64_t>(1 << 30, batch - b0);
+    qd::for_each_launch(batch, 1 << 30, [&](int clip0, int nb) {   // one clip per CTA on gridDim.x
         qd::LimiterArgs c = a;
-        if (a.starts) {
-            c.clip0 = a.clip0 + (int)b0;   // ragged: offsets stay relative to starts[0]
-        } else {
-            const size_t off = (size_t)b0 * (size_t)a.n;
-            c.x = a.x + off; c.y = a.y + off;
-            if (a.dry) c.dry = a.dry + off;
-            if (a.low) c.low = a.low + off;
-            if (a.orig) c.orig = a.orig + off;
-        }
-        if (a.clip_peak) c.clip_peak = a.clip_peak + b0;
+        c.clip0 = clip0;
         qd::limiter_mix_kernel<<<(unsigned)nb, qd::QD_TT, smem, st>>>(c);
-    }
+    });
     QD_CUDA(cudaGetLastError());
     return QD_OK;
 }
@@ -319,17 +309,11 @@ int fold_exact_in_f32(double fold, double bias) {
 void launch_crossover(const qd::CrossoverArgs &c, int64_t batch, cudaStream_t st) {
     const long long n_tiles = (c.n + c.tile - 1) / c.tile;
     const unsigned gx = (unsigned)((n_tiles + 32 * qd::QD_XO_WARPS - 1) / (32 * qd::QD_XO_WARPS));
-    for (int64_t b0 = 0; b0 < batch; b0 += 65535) {   // gridDim.y limit
-        const int64_t nb = std::min<int64_t>(65535, batch - b0);
+    qd::for_each_launch(batch, qd::QD_GRID_Y_MAX, [&](int clip0, int nb) {
         qd::CrossoverArgs k = c;
-        if (c.starts) {
-            k.clip0 = c.clip0 + (int)b0;   // ragged: offsets stay relative to starts[0]
-        } else {
-            const size_t off = (size_t)b0 * (size_t)c.n;
-            k.x = c.x + off; k.low = c.low + off; k.high = c.high + off;
-        }
+        k.clip0 = clip0;
         qd::crossover_kernel<<<dim3(gx, (unsigned)nb, 1), 32 * qd::QD_XO_WARPS, 0, st>>>(k);
-    }
+    });
 }
 
 int ew_grid(int64_t count, int sm_count) {
@@ -374,13 +358,11 @@ int launch_peaks_t(qd::PeaksArgsT<T> a, int64_t batch, cudaStream_t st) {
     const size_t per_warp = (size_t)qd::buf_slots<NC>() * sizeof(qd::V2<T>) + (size_t)2 * NC * sizeof(float);
     const int nw = (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / per_warp));
     const unsigned gx = (unsigned)((a.n_frames + nw - 1) / nw);
-    for (int64_t b0 = 0; b0 < batch; b0 += 65535) {
-        const int64_t nb = std::min<int64_t>(65535, batch - b0);
+    qd::for_each_launch(batch, qd::QD_GRID_Y_MAX, [&](int clip0, int nb) {
         qd::PeaksArgsT<T> c = a;
-        c.x = a.x + (size_t)b0 * a.n;
-        c.bins = a.bins + (size_t)b0 * a.n_frames * a.topn;
+        c.clip0 = clip0;
         kern<<<dim3(gx, (unsigned)nb, 1), 32 * nw, per_warp * nw, st>>>(c);
-    }
+    });
     QD_CUDA(cudaGetLastError());
     return QD_OK;
 }
@@ -431,6 +413,7 @@ int qd_device_count(void) {
 int qd_spectral_peaks_device(const float *x, int64_t batch, int32_t n_samples, int32_t n_fft, int32_t topn,
                              double min_mag, int32_t precision, int16_t *bins, void *stream) {
     if (!x || !bins || batch < 0 || n_samples < 0) return fail(QD_ERR_INVALID_ARG, "null / negative argument");
+    if (batch > INT32_MAX) return fail(QD_ERR_INVALID_ARG, "batch of more than 2^31 - 1 clips");
     if (topn < 1 || topn > qd::QD_PEAKS_MAX) return fail(QD_ERR_INVALID_ARG, "topn must be 1..8");
     if (batch == 0) return QD_OK;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -713,7 +696,7 @@ int render_impl(qd_plan *pl, const float *x, float *y, const Packing &pk, int64_
         const bool needs_table = p.fx_mode == QD_FX_SCRAMBLE_PICK || p.fx_mode == QD_FX_SCRAMBLE_SWAP ||
                                  (p.fx_mode == QD_FX_PHASE_DISPERSAL && p.fx_b != 0.0);
         if (needs_table && !pl->fx_table) return fail(QD_ERR_INVALID_ARG, "FX table missing (qd_plan_set_fx_table)");
-        if (needs_table && p.fx_table_per_clip && pl->clip_offset + batch > pl->fx_tables)
+        if (needs_table && p.fx_table_per_clip && pk.clip_offset + batch > pl->fx_tables)
             return fail(QD_ERR_INVALID_ARG, "per-clip FX table shorter than the batch");
     }
     cudaStream_t st = (cudaStream_t)stream;
@@ -724,10 +707,10 @@ int render_impl(qd_plan *pl, const float *x, float *y, const Packing &pk, int64_
     float *w_a = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
     float *w_low = w_a + stride;
     float *w_high = w_low + stride;
-    pl->frozen_ws = reinterpret_cast<void *>((reinterpret_cast<uintptr_t>(w_a + (p.multiband ? 3 : 1) * stride) + 255) & ~(uintptr_t)255);
+    void *frozen_ws = reinterpret_cast<void *>((reinterpret_cast<uintptr_t>(w_a + (p.multiband ? 3 : 1) * stride) + 255) & ~(uintptr_t)255);
     // per-clip peak of the limiter input, written by the spectral pass that produces it (behind the freeze scratch)
     const size_t frozen_bytes = p.spectral_freeze ? (size_t)batch * (size_t)(pl->nc + pl->nc / 32) * sizeof(double) + 256 : 0;
-    float *clip_peak = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(pl->frozen_ws) + frozen_bytes + 255) & ~(uintptr_t)255);
+    float *clip_peak = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(frozen_ws) + frozen_bytes + 255) & ~(uintptr_t)255);
     if (!p.limiter_on) clip_peak = nullptr;
     int rc;
 
@@ -787,10 +770,10 @@ int render_impl(qd_plan *pl, const float *x, float *y, const Packing &pk, int64_
         clip_peak = nullptr;   // no spectral pass measured the limiter input
     } else if (p.pre_quant) {
         // pass A: STFT -> quantize -> iSTFT (= pre_quant tap) -> distortion        (:635-721)
-        if ((rc = launch_spec(pl, pk, src, w_a, tap_pre, 1, epi, batch, st, 0, pl->clip_offset,
-                              p.post_quant ? nullptr : clip_peak)) != QD_OK) return rc;
+        if ((rc = launch_spec(pl, pk, src, w_a, tap_pre, 1, epi, batch, st, 0, p.post_quant ? nullptr : clip_peak,
+                              frozen_ws)) != QD_OK) return rc;
         if (p.post_quant) {  // pass B on the distorted signal                         (:729-801)
-            if ((rc = launch_spec(pl, pk, w_a, y, nullptr, 1, 0, batch, st, 1, pl->clip_offset, clip_peak)) != QD_OK) return rc;
+            if ((rc = launch_spec(pl, pk, w_a, y, nullptr, 1, 0, batch, st, 1, clip_peak, frozen_ws)) != QD_OK) return rc;
             x_pq = y;
         } else {
             x_pq = w_a;       // :851-853
@@ -803,7 +786,7 @@ int render_impl(qd_plan *pl, const float *x, float *y, const Packing &pk, int64_
                 src, w_a, (long long)count, p.distortion_mode, p.fold_amount, p.bias, p.tube_gain, p.tube_norm);
             QD_CUDA(cudaGetLastError());
         }
-        if ((rc = launch_spec(pl, pk, src, y, nullptr, p.post_quant ? 1 : 0, 0, batch, st, 0, pl->clip_offset, clip_peak)) != QD_OK) return rc;
+        if ((rc = launch_spec(pl, pk, src, y, nullptr, p.post_quant ? 1 : 0, 0, batch, st, 0, clip_peak, frozen_ws)) != QD_OK) return rc;
         x_pq = y;
     }
     if (tap_dist) {  // dsp/pipeline.py:916 / :1107 (low band added in multiband mode)
@@ -831,6 +814,7 @@ extern "C" {
 int qd_render_device(qd_plan *pl, const float *x, float *y, int64_t batch, const qd_taps *taps,
                      void *workspace, size_t workspace_bytes, void *stream) {
     if (!pl || !x || !y || batch < 0) return fail(QD_ERR_INVALID_ARG, "null argument");
+    if (batch > INT32_MAX) return fail(QD_ERR_INVALID_ARG, "batch of more than 2^31 - 1 clips");
     if (batch == 0 || pl->p.n_samples == 0) return QD_OK;
     Packing pk;
     pk.span = (int64_t)pl->p.n_samples * batch;
@@ -857,6 +841,7 @@ int qd_render_device_varlen(qd_plan *pl, const float *x, float *y, const int64_t
 int qd_limiter_device(const float *x, float *y, int64_t batch, int64_t n, int32_t lookahead, double ceiling_lin,
                       double release_coeff, void *stream) {
     if (!x || !y || batch < 0 || n < 0 || lookahead < 1) return fail(QD_ERR_INVALID_ARG, "bad limiter argument");
+    if (batch > INT32_MAX) return fail(QD_ERR_INVALID_ARG, "batch of more than 2^31 - 1 clips");
     if (batch == 0 || n == 0) return QD_OK;
     qd::LimiterArgs a{};
     a.x = x; a.y = y; a.n = (long long)n; a.limiter_on = 1; a.lookahead = lookahead;
@@ -867,6 +852,7 @@ int qd_limiter_device(const float *x, float *y, int64_t batch, int64_t n, int32_
 int qd_crossover_device(const float *x, float *low, float *high, int64_t batch, int64_t n,
                         const double sos_low[2][6], const double sos_high[2][6], void *stream) {
     if (!x || !low || !high || !sos_low || !sos_high || batch < 0 || n < 0) return fail(QD_ERR_INVALID_ARG, "bad crossover argument");
+    if (batch > INT32_MAX) return fail(QD_ERR_INVALID_ARG, "batch of more than 2^31 - 1 clips");
     if (batch == 0 || n == 0) return QD_OK;
     qd::CrossoverArgs c{};
     c.x = x; c.low = low; c.high = high; c.n = (long long)n;

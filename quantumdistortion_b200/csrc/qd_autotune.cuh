@@ -79,7 +79,7 @@ __global__ void __launch_bounds__(32 * AT_SW) at_filt_seg_kernel(const AtFiltSeg
     __shared__ double s_row[AT_SW][32][33];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int job = blockIdx.z;
-    const AtClip c = at_clip(a, blockIdx.y);
+    const ClipLoc c = clip_loc(a, blockIdx.y);
     const long long n = c.n;
     if (n <= AT_EDGE) return;   // not rendered: the odd extension needs more than AT_EDGE samples
     const float *__restrict__ x = a.x[job] + c.base;
@@ -277,7 +277,7 @@ __global__ void __launch_bounds__(32 * AT_SW_STATS) at_frame_stats_kernel(const 
     } else {
         ci = (int)(fr / at_rows(a.n, a.hop));
     }
-    const AtClip c = at_clip(a, ci);
+    const ClipLoc c = clip_loc(a, ci);
     const long long frame = fr - at_row0(a.starts != nullptr, c, a.n, a.hop);
     if (frame >= at_rows(c.n, a.hop)) return;            // a row between two clips
     const long long n = c.n;
@@ -453,7 +453,7 @@ __global__ void at_target_kernel(const AtHoldArgs a) {
 __global__ void at_hold_kernel(const AtHoldArgs a) {
     const int clip = blockIdx.x * blockDim.x + threadIdx.x;
     if (clip >= a.batch) return;
-    const AtClip c = at_clip(a, clip);
+    const ClipLoc c = clip_loc(a, clip);
     const int frames = (int)at_rows(c.n, a.hop);
     if (frames == 0) return;
     const long long r0 = at_row0(a.starts != nullptr, c, a.n, a.hop);
@@ -588,7 +588,7 @@ QD_DEV AtTileCtx at_tile_ctx(const AtShiftArgs &a, const double *__restrict__ ra
 // (a tile holds no frame centre strictly inside when hop and frame_size / 2 are multiples of the tile: 512 | 512, 2048)
 __global__ void __launch_bounds__(32 * AT_TW) at_tap_sums_kernel(const AtShiftArgs a) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const AtClip c = at_clip(a, blockIdx.y);
+    const ClipLoc c = clip_loc(a, blockIdx.y);
     const long long tile = (long long)blockIdx.x * AT_TW + warp;
     if (tile >= at_rows(c.n, AT_TS)) return;
     const bool rg = a.starts != nullptr;
@@ -619,7 +619,7 @@ __global__ void __launch_bounds__(32 * AT_TW) at_tap_sums_kernel(const AtShiftAr
 // tile_sum -> tap 0 at the start of every tile (in [0, M)); flat_flag -> 1 when no tile of the clip raised it
 __global__ void __launch_bounds__(32) at_tap_scan_kernel(const AtShiftArgs a) {
     const int lane = threadIdx.x;
-    const AtClip c = at_clip(a, blockIdx.x);
+    const ClipLoc c = clip_loc(a, blockIdx.x);
     const long long tiles = at_rows(c.n, AT_TS);
     long long *ts = a.tile_sum + at_row0(a.starts != nullptr, c, a.n, AT_TS);
     const long long M = (long long)a.max_delay << 24;
@@ -650,7 +650,7 @@ __global__ void __launch_bounds__(32) at_tap_scan_kernel(const AtShiftArgs a) {
 __global__ void __launch_bounds__(32 * AT_TW) at_shift_kernel(const AtShiftArgs a) {
     __shared__ float s_out[AT_TW][AT_TS + AT_TS / 16];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const AtClip c = at_clip(a, blockIdx.y);
+    const ClipLoc c = clip_loc(a, blockIdx.y);
     const long long n = c.n;
     const long long tile = (long long)blockIdx.x * AT_TW + warp;
     if (tile >= at_rows(n, AT_TS)) return;
@@ -755,7 +755,7 @@ __global__ void __launch_bounds__(32 * AT_FW) at_env_kernel(const AtMixArgs a) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int clip = blockIdx.x * AT_FW + warp;
     if (clip >= a.batch) return;
-    const AtClip c = at_clip(a, clip);
+    const ClipLoc c = clip_loc(a, clip);
     if (c.n >= a.seg_min) return;
     const long long n = c.n;
     const float *__restrict__ x = a.x + c.base;
@@ -804,7 +804,7 @@ __global__ void __launch_bounds__(32 * AT_FW) at_env_kernel(const AtMixArgs a) {
 __global__ void __launch_bounds__(32 * AT_SW) at_env_seg_kernel(const AtMixArgs a, int tile, int halo) {
     __shared__ float s_row[AT_SW][32][33];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const AtClip c = at_clip(a, blockIdx.y);
+    const ClipLoc c = clip_loc(a, blockIdx.y);
     const long long n = c.n;
     if (n < a.seg_min) return;
     const float *__restrict__ x = a.x + c.base;
@@ -877,7 +877,7 @@ __global__ void __launch_bounds__(32 * AT_SW) at_env_seg_kernel(const AtMixArgs 
 }
 
 __global__ void at_mix_kernel(const AtMixArgs a) {
-    const AtClip c = at_clip(a, blockIdx.y);
+    const ClipLoc c = clip_loc(a, blockIdx.y);
     const long long base = c.base;
     const float top = a.layer_on ? a.env_max[c.idx] : 0.0f;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < c.n; i += (long long)gridDim.x * blockDim.x) {

@@ -221,38 +221,33 @@ QD_DEV void dft_reg(V2<T> (&v)[R]) {
     }
 }
 
-// clip c of a launch inside its packed buffers: sample offset and length.  Uniform batches (starts == null) sit at
-// c * n; a ragged batch reads its per-clip arrays (see SpecArgsT::starts), offsets relative to starts[0].
-struct ClipSpan { long long base; int n; };
+// Clip c of a launch: its index in the batch (idx = clip0 + c), its sample offset in the packed buffers and its length.
+// Uniform batches (starts == null) hold clip i at i * n, n samples each; a ragged batch reads its per-clip arrays
+// starts / lengths, offsets relative to starts[0] (n is then the longest clip, which sizes the grids).  Launch splits
+// (for_each_launch) advance clip0 for both kinds, so no pointer moves and per-clip arrays are indexed by idx.
+struct ClipLoc { int idx; long long base, n; };
 template <class A>
-QD_DEV ClipSpan clip_span(const A &a, int c) {
-    if (a.starts) {
-        const int i = a.clip0 + c;
-        return {(long long)(a.starts[i] - a.starts[0]), (int)a.lengths[i]};
-    }
-    return {(long long)c * (long long)a.n, (int)a.n};
+QD_DEV ClipLoc clip_loc(const A &a, int c) {
+    const int i = a.clip0 + c;
+    if (a.starts) return {i, (long long)(a.starts[i] - a.starts[0]), (long long)a.lengths[i]};
+    return {i, (long long)i * a.n, (long long)a.n};
 }
 
-// The autotune_v1 kernels (qd_autotune.cuh, qd_yin.cuh) take optional per-clip arrays `starts` / `lengths` (a ragged
-// batch, as SpecArgsT::starts; null: uniform clips of n samples at i * n).  n is the longest clip, which sizes the
-// grids.  Unlike clip_span's callers they advance clip0 at launch splits in uniform batches too, so per-clip arrays
-// are indexed by clip0 + c and no pointer moves.
-struct AtClip { int idx; long long base, n; };
-template <class A>
-QD_DEV AtClip at_clip(const A &a, int c) {
-    if (a.starts) {
-        const ClipSpan s = clip_span(a, c);
-        return {a.clip0 + c, s.base, (long long)s.n};
-    }
-    const int i = a.clip0 + c;
-    return {i, (long long)i * a.n, a.n};
+// Covers clips [0, batch) with launches of at most per_launch clips: fn(clip0, nb) for each.  Grids put clips on
+// gridDim.y, whose limit is QD_GRID_Y_MAX; a kernel with g clips per CTA passes g * QD_GRID_Y_MAX.  Clip indices
+// are int: the entry points reject batches past INT32_MAX.
+constexpr int64_t QD_GRID_Y_MAX = 65535;
+template <class Fn>
+inline void for_each_launch(int64_t batch, int64_t per_launch, Fn &&fn) {
+    for (int64_t b0 = 0; b0 < batch; b0 += per_launch) fn((int)b0, (int)(batch - b0 < per_launch ? batch - b0 : per_launch));
 }
+
 // Per-clip tables with one row per `unit` samples (detector frames: unit = hop, ceil(n / hop) frames per clip;
 // delay-tap tiles: unit = AT_TS).  Uniform batches keep clip i at row i * rows(n).  Ragged batches put it at
 // floor(base / unit) + i: no scan, valid for any sub-range of clips, and rows of consecutive clips cannot overlap
 // because starts[i + 1] >= starts[i] + n_i.  So a ragged batch has at most span / unit + batch rows.
 __host__ __device__ inline long long at_rows(long long n, int unit) { return (n + unit - 1) / unit; }
-QD_DEV long long at_row0(bool ragged, const AtClip &c, long long n_uniform, int unit) {
+QD_DEV long long at_row0(bool ragged, const ClipLoc &c, long long n_uniform, int unit) {
     return ragged ? c.base / unit + c.idx : (long long)c.idx * at_rows(n_uniform, unit);
 }
 

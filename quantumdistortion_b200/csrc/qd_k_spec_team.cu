@@ -1,6 +1,5 @@
 // spectral pass for the three-pass FFT plans: teams of warps per frame on swizzled buffers (qd_spec_team.cuh) -- float32
 // n_fft 512 / 1024 / 4096, float64 n_fft 2048 / 4096 / 8192
-#include <algorithm>
 #include <atomic>
 
 #include "qd_err.hpp"
@@ -15,20 +14,12 @@ static int launch_spec_team_t(const qd::SpecArgsT<T> &a, const qd::TeamGather &t
     if (int rc_ = qd_err::ensure_dyn_smem(kern, attr_mask, 227 * 1024)) return rc_;
     const size_t smem = qd::SpecSmem<T, NC, NF>::bytes(a.q.n_slots);
     if (smem > 227 * 1024) return qd_err::fail(QD_ERR_UNSUPPORTED, "shared memory need of the team kernel exceeds 227 KB");
-    for (int64_t b0 = 0; b0 < batch; b0 += 65535) {  // gridDim.y limit
-        const int64_t nb = std::min<int64_t>(65535, batch - b0);
+    qd::for_each_launch(batch, qd::QD_GRID_Y_MAX, [&](int clip0, int nb) {
         qd::SpecArgsT<T> c = a;
-        c.batch = (int)nb;
-        if (a.starts) {
-            c.clip0 = a.clip0 + (int)b0;   // ragged: offsets stay relative to starts[0]
-        } else {
-            c.x = a.x + (size_t)b0 * a.n;
-            c.y = a.y + (size_t)b0 * a.n;
-            if (a.tap) c.tap = a.tap + (size_t)b0 * a.n;
-        }
-        if (a.clip_peak) c.clip_peak = a.clip_peak + b0;
+        c.clip0 = clip0;
+        c.batch = nb;
         kern<<<dim3((unsigned)tiles, (unsigned)nb, 1), 32 * NF * CW, smem, st>>>(c, tg);
-    }
+    });
     QD_CUDA(cudaGetLastError());
     return QD_OK;
 }

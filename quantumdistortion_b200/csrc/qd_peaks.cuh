@@ -21,6 +21,7 @@ struct PeaksArgsT {
     const float *x;       // [batch, n]
     int16_t *bins;        // [batch, n_frames, topn]: bin index, -1 = no (further) bin above the threshold
     int n, n_frames, topn;
+    int clip0;            // clip of blockIdx.y == 0 (launch splits advance it, see for_each_launch)
     T min_mag2;           // (10^(min_db/20))^2
     const V2<T> *wtab, *tw1, *tw2, *wsplit;
 };
@@ -35,7 +36,7 @@ peaks_kernel(const PeaksArgsT<T> a) {
     const size_t per_warp = (size_t)BUF * sizeof(V2<T>) + (size_t)2 * NC * sizeof(float);
     V2<T> *buf = reinterpret_cast<V2<T> *>(smem + (size_t)warp * per_warp);
     float *stage = reinterpret_cast<float *>(smem + (size_t)warp * per_warp + (size_t)BUF * sizeof(V2<T>));
-    const int clip = blockIdx.y;
+    const int clip = a.clip0 + (int)blockIdx.y;
     const int t = blockIdx.x * nw + warp;
     if (t >= a.n_frames) return;
     const float *x = a.x + (size_t)clip * a.n;

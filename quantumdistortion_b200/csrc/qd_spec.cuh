@@ -102,7 +102,7 @@ struct FxDev {
     int table_frames;       // frames per pass in the table
     int table_per_clip;     // 0: shared by all clips
     int pass;               // 0 / 1: which quantised pass of the render this launch is
-    int clip_offset;        // index of the launch's first clip inside the per-clip table
+    int clip_offset;        // row of the batch's clip 0 in the per-clip table (a host-pipe chunk's first clip)
 };
 
 template <class T>
@@ -116,7 +116,7 @@ struct SpecArgsT {
     int batch;             // clips in this launch (a CTA may hold several clip groups)
     int n_frames;          // T = 1 + n / hop of a uniform batch (the kernels derive each clip's own from its length)
     // ragged batch (null = uniform clips at clip * n): clip c of the launch is starts[clip0 + c] - starts[0] samples
-    // into x / y / tap and has lengths[clip0 + c] samples.  Launch splits advance clip0, not the pointers.
+    // into x / y / tap and has lengths[clip0 + c] samples.  Launch splits advance clip0, not the pointers (clip_loc).
     const int64_t *starts;
     const int32_t *lengths;
     int clip0;
@@ -1047,8 +1047,11 @@ spec_pass_kernel(const SpecArgsT<T> a) {
 
     const int clip = (int)blockIdx.y * NG + grp;
     bool group_live = clip < a.batch;   // the last CTA may carry an empty group
-    const ClipSpan cs = clip_span(a, group_live ? clip : 0);
-    const int n = cs.n;
+    const ClipLoc cs = clip_loc(a, group_live ? clip : 0);
+    const int idx = a.clip0 + clip;     // = cs.idx once the empty group has left; per-clip arrays are indexed by it
+    const long long fx_row = a.fx.table_per_clip ? a.fx.clip_offset + idx : 0;
+    const T *frozen = a.frozen ? a.frozen + (size_t)idx * L::BUF : nullptr;
+    const int n = (int)cs.n;
     const float *x = a.x + cs.base;
     float *y = a.y + cs.base;
     float *tap = a.tap ? a.tap + cs.base : nullptr;
@@ -1175,11 +1178,11 @@ spec_pass_kernel(const SpecArgsT<T> a) {
                     T *mags = reinterpret_cast<T *>(planes) + (size_t)(grp * NW + warp) * L::BUF;
                     const int tf = t < a.fx.table_frames ? t : a.fx.table_frames - 1;
                     const long long tab_base =
-                        (((long long)(a.fx.table_per_clip ? a.fx.clip_offset + clip : 0) * 2 + a.fx.pass) * a.fx.table_frames + tf) * (NC + 1);
+                        ((fx_row * 2 + a.fx.pass) * a.fx.table_frames + tf) * (NC + 1);
                     V2<T> *scr = reinterpret_cast<V2<T> *>(planes + (size_t)NG * NW * L::BUF * sizeof(T)) +
                                  (size_t)(grp * NW + warp) * L::BUF;   // only there when the formant shift is on
                     fx_frame<T, NC>(buf, mags, a.fx, lane, tab_base,
-                                    a.frozen ? a.frozen + (size_t)clip * L::BUF : nullptr, scr, a, tw1, wsplit);
+                                    frozen, scr, a, tw1, wsplit);
                     quantize_frame_fused<T, NC, TS, true>(buf, mags, slotG, slotP, qq, wsplit, lane);
                 } else {
                     quantize_frame_fused<T, NC, TS, false>(buf, nullptr, slotG, slotP, qq, wsplit, lane);
@@ -1255,7 +1258,7 @@ spec_pass_kernel(const SpecArgsT<T> a) {
     }
     if (a.clip_peak) {   // non-negative floats order like their bit patterns
         out_peak = warp_max(out_peak);
-        if (lane == 0) atomicMax(reinterpret_cast<unsigned *>(a.clip_peak) + clip, __float_as_uint(out_peak));
+        if (lane == 0) atomicMax(reinterpret_cast<unsigned *>(a.clip_peak) + idx, __float_as_uint(out_peak));
     }
 }
 
@@ -1269,8 +1272,7 @@ freeze_mag_kernel(const SpecArgsT<T> a, T *out) {
     V2<T> *buf = reinterpret_cast<V2<T> *>(smem);
     float *stage = reinterpret_cast<float *>(smem + (size_t)BUF * sizeof(V2<T>));
     const int lane = threadIdx.x;
-    const int clip = blockIdx.x;
-    const ClipSpan cs = clip_span(a, clip);
+    const ClipLoc cs = clip_loc(a, (int)blockIdx.x);
     const float *x = a.x + cs.base;
     for (int i = lane; i < 2 * NC; i += 32) {
         const long long s = (long long)i - NC;
@@ -1280,7 +1282,7 @@ freeze_mag_kernel(const SpecArgsT<T> a, T *out) {
     fwd_first<T, NC, FftCfg<T, NC>::R1>(buf, reinterpret_cast<const float2 *>(stage), a.wtab, a.tw1, lane);
     fft_forward<T, NC>(buf, nullptr, a, a.wtab, a.tw1, a.tw2, lane);
     real_split<T, NC>(buf, a.wsplit, lane);
-    T *o = out + (size_t)clip * BUF;
+    T *o = out + (size_t)cs.idx * BUF;
     for (int p = lane; p < BUF; p += 32) {
         const V2<T> v = buf[p];
         const T m2 = v.x * v.x + v.y * v.y;

@@ -417,9 +417,8 @@ spec_pass_team_kernel(const SpecArgsT<T> a, const TeamGather tg) {
     T *slotG = reinterpret_cast<T *>(smem + L::off_slot) + (size_t)team * slot_cap * 3;
     V2<T> *slotP = reinterpret_cast<V2<T> *>(slotG + slot_cap);
 
-    const int clip = (int)blockIdx.y;
-    const ClipSpan cs = clip_span(a, clip);   // one clip per CTA: the early return below is uniform
-    const int n = cs.n;
+    const ClipLoc cs = clip_loc(a, (int)blockIdx.y);   // one clip per CTA: the early return below is uniform
+    const int n = (int)cs.n;
     const float *x = a.x + cs.base;
     float *y = a.y + cs.base;
     float *tap = a.tap ? a.tap + cs.base : nullptr;
@@ -549,7 +548,7 @@ spec_pass_team_kernel(const SpecArgsT<T> a, const TeamGather tg) {
     }
     if (a.clip_peak) {
         out_peak = warp_max(out_peak);
-        if (lane == 0) atomicMax(reinterpret_cast<unsigned *>(a.clip_peak) + clip, __float_as_uint(out_peak));
+        if (lane == 0) atomicMax(reinterpret_cast<unsigned *>(a.clip_peak) + cs.idx, __float_as_uint(out_peak));
     }
 }
 

@@ -93,14 +93,14 @@ __global__ void __launch_bounds__(QD_TT, 3) limiter_mix_kernel(const LimiterArgs
     double *s_warp0 = reinterpret_cast<double *>((reinterpret_cast<uintptr_t>(s_gmax0 + 2 * gmax_stride) + 7) & ~(uintptr_t)7);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr int NWARP = QD_TT / 32;
-    const ClipSpan cs = clip_span(a, (int)blockIdx.x);
+    const ClipLoc cs = clip_loc(a, (int)blockIdx.x);
     const size_t base = (size_t)cs.base;
     const long long n = cs.n;
     const float *x = a.x + base;
     const bool vec = (reinterpret_cast<uintptr_t>(x) & 15) == 0;
     const bool vec_out = (reinterpret_cast<uintptr_t>(a.y + base) & 15) == 0;
     const bool need_dry = a.apply_mix && a.dry_gain != 0.0f;
-    const bool clip_quiet = a.clip_peak != nullptr && !((double)a.clip_peak[blockIdx.x] > a.ceiling);
+    const bool clip_quiet = a.clip_peak != nullptr && !((double)a.clip_peak[cs.idx] > a.ceiling);
     const bool limiter_on = a.limiter_on && !clip_quiet;
     if (!limiter_on && a.x == a.y && !need_dry && !a.low && !a.orig && (!a.apply_mix || (a.wet == 1.0f && !a.apply_trim)))
         return;   // y = float32(x * 1) in place
@@ -342,7 +342,7 @@ __global__ void __launch_bounds__(32 * QD_XO_WARPS) crossover_kernel(const Cross
     __shared__ float s_lo[QD_XO_WARPS][32][33];   // input row, overwritten by the low band
     __shared__ float s_hi[QD_XO_WARPS][32][33];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const ClipSpan cs = clip_span(a, (int)blockIdx.y);
+    const ClipLoc cs = clip_loc(a, (int)blockIdx.y);
     const size_t base = (size_t)cs.base;
     const long long n = cs.n;
     const float *x = a.x + base;

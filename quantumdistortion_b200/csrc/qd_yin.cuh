@@ -38,7 +38,7 @@
 namespace qd {
 
 struct AtYinArgs {
-    const float *det;        // packed like the batch (qd_autotune.cuh: at_clip)
+    const float *det;        // packed like the batch (qd_common.cuh: clip_loc)
     double *diff;            // [frame rows, stride] difference function, entry tau (frame rows: at_row0)
     double *feat;            // [frame rows, 4]; feat[2] holds 1 / 0 (frame not silent) on entry of the pick kernel
     long long n;
@@ -139,7 +139,7 @@ __global__ void __launch_bounds__(AT_YT, 1) at_yin_diff_kernel(const AtYinArgs a
     double *ebq = be + 16;                              // [16] ebq[q] = energy of the q blocks before the one being assembled
     uint64_t *mbar = reinterpret_cast<uint64_t *>(ebq + 16);   // full[3] (helpers -> walkers), done[3] (walkers -> helpers)
     int *lagc = reinterpret_cast<int *>(mbar + 2 * AT_YNS);      // [L * cols] per lag: off | q << 12 | group << 16 | live << 20
-    const AtClip clip = at_clip(a, blockIdx.y);
+    const ClipLoc clip = clip_loc(a, blockIdx.y);
     const long long n = clip.n;
     const int frames = (int)at_rows(n, hop);
     const float *x = a.det + clip.base;

@@ -16,7 +16,10 @@
 //   emu_at_ragged mix <sub_enabled> <layer_on> <att> <rel> <tile> <halo> <seg_min> <level> <preserve> <air_mix>
 //                     <phase_k> <sr> <x.f32> <sub.f32> <air.f32> <corrected.f32> <starts|-> <lengths|-> <y.f32>
 //                     <sub_layer.f32>
-// With "-" for starts / lengths x is one clip (the uniform path); otherwise x is packed and the batch is len(starts).
+// With "-" for starts / lengths x is one clip (the uniform path), with "u<B>" B uniform clips of len(x) / B samples;
+// otherwise x is packed and the batch is len(starts).  A leading "-p <clips>" splits the kernels that the library
+// splits at the grid limit (filt, yin, shift, the segment follower of env, mix) into launches of that many clips with
+// qd::for_each_launch (default: one launch).
 // Frame rows (stats / pick / hold / shift) are laid out as the library lays them out (qd::at_row0); feat and ratio rows
 // no clip owns keep their initial value.  Every mode launches the production kernels with the production block shapes
 // (qd_autotune_api.inc: at_render); the filter bank takes its tiles from the poles like the library
@@ -58,6 +61,13 @@ static void write_all(const char *path, const std::vector<T> &v) {
     std::ofstream(path, std::ios::binary).write(reinterpret_cast<const char *>(v.data()), (std::streamsize)(v.size() * sizeof(T)));
 }
 
+static int64_t g_per_launch = INT32_MAX;
+// fn(clip0, nb) for each launch of the split, with a.clip0 set
+template <class A, class Fn>
+static void each_launch(A &a, int batch, Fn fn) {
+    qd::for_each_launch(batch, g_per_launch, [&](int clip0, int nb) { a.clip0 = clip0; fn((unsigned)nb); });
+}
+
 struct Batch {
     std::vector<float> x;
     std::vector<int64_t> starts;
@@ -69,7 +79,7 @@ struct Batch {
 static Batch load(const char *xp, const char *sp, const char *lp) {
     Batch b;
     b.x = read_all<float>(xp);
-    b.ragged = std::string(sp) != "-";
+    b.ragged = sp[0] != '-' && sp[0] != 'u';
     b.span = (long long)b.x.size();
     if (b.ragged) {
         b.starts = read_all<int64_t>(sp);
@@ -77,8 +87,8 @@ static Batch load(const char *xp, const char *sp, const char *lp) {
         b.batch = (int)b.starts.size();
         b.n_max = *std::max_element(b.lengths.begin(), b.lengths.end());
     } else {
-        b.batch = 1;
-        b.n_max = b.span;
+        b.batch = sp[0] == 'u' ? std::atoi(sp + 1) : 1;
+        b.n_max = b.span / b.batch;
     }
     return b;
 }
@@ -107,7 +117,7 @@ static void set_clips(A &a, const Batch &b) {
 }
 // rows of a per-clip table with one row per `unit` samples (at_layout)
 static long long table_rows(const Batch &b, int unit) {
-    return b.ragged ? b.span / unit + b.batch : qd::at_rows(b.n_max, unit);
+    return b.ragged ? b.span / unit + b.batch : b.batch * qd::at_rows(b.n_max, unit);
 }
 static double num(const char *s) { return std::strtod(s, nullptr); }
 
@@ -118,13 +128,21 @@ static void run_env(qd::AtMixArgs &m, const Batch &b, int tile, int halo) {
     if (b.n_max >= m.seg_min) {
         const long long n_tiles = (b.n_max + tile - 1) / tile;
         const unsigned gx = (unsigned)((n_tiles + 32 * qd::AT_SW - 1) / (32 * qd::AT_SW));
-        qd_emu::launch(dim3(gx, b.batch, 1), dim3(32 * qd::AT_SW), 0, [&] { qd::at_env_seg_kernel(m, tile, halo); });
+        each_launch(m, b.batch, [&](unsigned nb) {
+            qd_emu::launch(dim3(gx, nb, 1), dim3(32 * qd::AT_SW), 0, [&] { qd::at_env_seg_kernel(m, tile, halo); });
+        });
+        m.clip0 = 0;
     }
     if (b.ragged || b.n_max < m.seg_min)
         qd_emu::launch(dim3((b.batch + qd::AT_FW - 1) / qd::AT_FW), dim3(32 * qd::AT_FW), 0, [&] { qd::at_env_kernel(m); });
 }
 
 int main(int argc, char **argv) {
+    if (argc > 2 && std::string(argv[1]) == "-p") {
+        g_per_launch = std::atoll(argv[2]);
+        argv += 2;
+        argc -= 2;
+    }
     if (argc < 2) { std::cerr << "usage: see source\n"; return 2; }
     const std::string mode = argv[1];
     if (mode == "yin" && argc == 10) {
@@ -138,11 +156,13 @@ int main(int argc, char **argv) {
         const int tblocks = (total_cols + a.lag_threads - 1) / a.lag_threads;
         a.frames = (int)qd::at_rows(a.n, a.hop);
         a.stride = (a.max_tau + 2) & ~1;
-        const long long rows = b.ragged ? b.span / a.hop + b.batch : qd::at_rows(a.n, a.hop);
+        const long long rows = table_rows(b, a.hop);
         std::vector<double> diff((size_t)rows * a.stride, -1.0);
         a.det = b.x.data(); a.diff = diff.data();
         const size_t smem = qd::at_yin_smem_doubles(a.hop, (tblocks - 1) * a.lag_threads, a.lag_threads) * sizeof(double) + 128;
-        qd_emu::launch(dim3(tblocks, b.batch, 1), dim3(qd::AT_YT), smem, [&] { qd::at_yin_diff_kernel(a); });
+        each_launch(a, b.batch, [&](unsigned nb) {
+            qd_emu::launch(dim3(tblocks, nb, 1), dim3(qd::AT_YT), smem, [&] { qd::at_yin_diff_kernel(a); });
+        });
         write_all(argv[9], diff);
         return 0;
     }
@@ -170,8 +190,10 @@ int main(int argc, char **argv) {
             tiles = std::max(tiles, qd::at_rows(m, qd::at_filt_tile(q.tile[j], q.halo[j], m)));
         }
         const unsigned gx = (unsigned)((tiles + 32 * qd::AT_SW - 1) / (32 * qd::AT_SW));
-        qd_emu::launch(dim3(gx, b.batch, jobs), dim3(32 * qd::AT_SW), 0, [&] { qd::at_filt_seg_kernel<false>(q); });
-        qd_emu::launch(dim3(gx, b.batch, jobs), dim3(32 * qd::AT_SW), 0, [&] { qd::at_filt_seg_kernel<true>(q); });
+        each_launch(a, b.batch, [&](unsigned nb) {
+            qd_emu::launch(dim3(gx, nb, jobs), dim3(32 * qd::AT_SW), 0, [&] { qd::at_filt_seg_kernel<false>(q); });
+            qd_emu::launch(dim3(gx, nb, jobs), dim3(32 * qd::AT_SW), 0, [&] { qd::at_filt_seg_kernel<true>(q); });
+        });
         write_all(argv[7], y);
         return 0;
     }
@@ -245,9 +267,13 @@ int main(int argc, char **argv) {
         s.body = b.x.data(); s.ratio = ratio.data(); s.tile_sum = tile_sum.data();
         s.ratio_track = track.data(); s.flat_flag = flag.data(); s.out = out.data();
         const unsigned gx = (unsigned)((qd::at_rows(b.n_max, qd::AT_TS) + qd::AT_TW - 1) / qd::AT_TW);
-        qd_emu::launch(dim3(gx, b.batch, 1), dim3(32 * qd::AT_TW), 0, [&] { qd::at_tap_sums_kernel(s); });
-        qd_emu::launch(dim3(b.batch), dim3(32), 0, [&] { qd::at_tap_scan_kernel(s); });
-        qd_emu::launch(dim3(gx, b.batch, 1), dim3(32 * qd::AT_TW), 0, [&] { qd::at_shift_kernel(s); });
+        each_launch(s, b.batch, [&](unsigned nb) {
+            qd_emu::launch(dim3(gx, nb, 1), dim3(32 * qd::AT_TW), 0, [&] { qd::at_tap_sums_kernel(s); });
+        });
+        each_launch(s, b.batch, [&](unsigned nb) { qd_emu::launch(dim3(nb), dim3(32), 0, [&] { qd::at_tap_scan_kernel(s); }); });
+        each_launch(s, b.batch, [&](unsigned nb) {
+            qd_emu::launch(dim3(gx, nb, 1), dim3(32 * qd::AT_TW), 0, [&] { qd::at_shift_kernel(s); });
+        });
         write_all(argv[10], out);
         write_all(argv[11], track);
         write_all(argv[12], flag);
@@ -288,7 +314,9 @@ int main(int argc, char **argv) {
         m.env = env.data(); m.env_max = emax.data(); m.sub_layer = layer.data(); m.y = y.data();
         if (m.layer_on) run_env(m, b, std::atoi(argv[6]), std::atoi(argv[7]));
         const unsigned gx = (unsigned)std::min<long long>((b.n_max + 255) / 256, 1024);
-        qd_emu::launch(dim3(gx, b.batch, 1), dim3(256), 0, [&] { qd::at_mix_kernel(m); });
+        each_launch(m, b.batch, [&](unsigned nb) {
+            qd_emu::launch(dim3(gx, nb, 1), dim3(256), 0, [&] { qd::at_mix_kernel(m); });
+        });
         write_all(argv[20], y);
         write_all(argv[21], layer);
         return 0;

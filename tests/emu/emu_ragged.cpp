@@ -1,11 +1,17 @@
 // tests/emu/emu_ragged.cpp -- TEST INFRASTRUCTURE: runs the kernels of a ragged batch (per-clip starts / lengths) on the
 // CPU through cuda_emu.h, so that tests/test_emu_ragged.py can compare every clip with the same clip rendered alone.
 //
+//   emu_ragged [-p <clips per launch>] [-q] [-x] <mode> ...
 //   emu_ragged spec <f32|f64> <n_fft> <nw> <tile_blocks> <quant> <x.f32> <starts.i64|-> <lengths.i32|-> <tb.i32> <mask.u8> <y.f32>
-//       nw = 16: the two-group kernel of n_fft 2048 (NG = 2); nw >= 100: team kernel, 100 * frames + warps per frame
+//       nw = 16: the two-group kernel of n_fft 2048 (NG = 2); nw >= 100: team kernel, 100 * frames + warps per frame.
+//       Also writes <y>.peak: the per-clip peaks (clip_peak) and two rows no clip owns.
 //   emu_ragged limiter <lookahead> <x.f32> <starts|-> <lengths|-> <y.f32>
 //   emu_ragged crossover <low_delay> <sos_lp.f64> <sos_hp.f64> <tile> <halo> <x.f32> <starts|-> <lengths|-> <low.f32> <high.f32>
-// With "-" for starts / lengths x is one clip (the uniform path); otherwise x is packed and the batch is len(starts).
+// With "-" for starts / lengths x is one clip (the uniform path), with "u<B>" B uniform clips of len(x) / B samples;
+// otherwise x is packed and the batch is len(starts).  -p splits the batch into launches of that many clips with
+// qd::for_each_launch, as the library does at its grid limits (default: one launch).  -q: the limiter reads per-clip
+// peaks that mark every odd clip quiet.  -x (spec, n_fft 1024, nw 4): the FX kernel with a per-clip bin-scramble table
+// (clip 0 at row 1, as in a chunk of a host render) and the spectral freeze (freeze_mag_kernel in one launch).
 #include "cuda_emu.h"
 
 namespace qd_emu {
@@ -20,6 +26,7 @@ thread_local dim3 g_tid, g_bid;
 #include "../../quantumdistortion_b200/csrc/qd_host_time.hpp"
 
 #include <algorithm>
+#include <climits>
 #include <cstdlib>
 #include <fstream>
 #include <iostream>
@@ -40,7 +47,10 @@ static void write_all(const char *path, const std::vector<T> &v) {
     std::ofstream(path, std::ios::binary).write(reinterpret_cast<const char *>(v.data()), (std::streamsize)(v.size() * sizeof(T)));
 }
 
-// batch layout: uniform (one clip = all of x) or the ragged arrays
+static int64_t g_per_launch = INT32_MAX;
+static bool g_quiet_odd = false, g_fx = false;
+
+// batch layout: uniform (B clips of len(x) / B samples) or the ragged arrays
 struct Layout {
     std::vector<int64_t> starts;
     std::vector<int32_t> lengths;
@@ -49,8 +59,9 @@ struct Layout {
 };
 static Layout layout(const char *sp, const char *lp, size_t x_size) {
     Layout l;
-    if (std::string(sp) == "-") {
-        l.max_n = (int)x_size;
+    if (sp[0] == '-' || sp[0] == 'u') {
+        if (sp[0] == 'u') l.batch = std::atoi(sp + 1);
+        l.max_n = (int)(x_size / l.batch);
         return l;
     }
     l.ragged = true;
@@ -63,7 +74,7 @@ static Layout layout(const char *sp, const char *lp, size_t x_size) {
 template <class A>
 static void apply(A &a, const Layout &l) {
     a.n = l.max_n;
-    if (l.ragged) { a.starts = l.starts.data(); a.lengths = l.lengths.data(); a.clip0 = 0; }
+    if (l.ragged) { a.starts = l.starts.data(); a.lengths = l.lengths.data(); }
 }
 
 template <class T>
@@ -92,11 +103,12 @@ static int spec(int argc, char **argv) {
     std::string err;
     if (!qd_host::build_quant_tables(ht, &qt, &err, sizeof(T) == 8)) { std::cerr << err << "\n"; return 2; }
     std::vector<float> y(x.size(), -777.0f);
+    std::vector<float> peak((size_t)l.batch + 2, 0.0f);   // zeroed by the caller, as in launch_spec_prec
     qd::SpecArgsT<T> a{};
     a.x = x.data();
     a.y = y.data();
+    a.clip_peak = peak.data();
     apply(a, l);
-    a.batch = l.batch;
     a.n_frames = 1 + a.n / st.hop;
     a.tile_blocks = tile_blocks;
     a.quant = quant;
@@ -120,6 +132,16 @@ static int spec(int argc, char **argv) {
     a.fx.table_frames = 1;
     const int tiles = std::max(1, ((a.n + st.hop - 1) / st.hop + tile_blocks - 1) / tile_blocks);   // the longest clip
     const int nc = n_fft / 2;
+    // one launch per range of clips; clips_per_cta = NG
+    auto each = [&](int clips_per_cta, auto kern) {
+        qd::for_each_launch(l.batch, g_per_launch, [&](int clip0, int nb) {
+            a.clip0 = clip0;
+            a.batch = nb;
+            kern((nb + clips_per_cta - 1) / clips_per_cta);
+        });
+        write_all(argv[12], y);
+        write_all((std::string(argv[12]) + ".peak").c_str(), peak);
+    };
     if (nw >= 100) {
         const int nf = nw / 100, cw = nw % 100;
         std::vector<uint32_t> ttab;
@@ -128,9 +150,10 @@ static int spec(int argc, char **argv) {
         tg.src_tab = ttab.data();
 #define QD_TEAMCASE(NC_, NF_, CW_)                                                                                       \
         if (nc == NC_ && nf == NF_ && cw == CW_) {                                                                       \
-            qd_emu::launch(dim3(tiles, a.batch, 1), dim3(32 * NF_ * CW_, 1, 1), qd::SpecSmem<T, NC_, NF_>::bytes(qt.n_slots), \
-                           [&] { qd::spec_pass_team_kernel<T, NC_, NF_, CW_>(a, tg); });                                    \
-            write_all(argv[12], y);                                                                                       \
+            each(1, [&](int rows) {                                                                                       \
+                qd_emu::launch(dim3(tiles, rows, 1), dim3(32 * NF_ * CW_, 1, 1), qd::SpecSmem<T, NC_, NF_>::bytes(qt.n_slots), \
+                               [&] { qd::spec_pass_team_kernel<T, NC_, NF_, CW_>(a, tg); });                                \
+            });                                                                                                           \
             return 0;                                                                                                     \
         }
         QD_TEAMCASE(512, 8, 1) QD_TEAMCASE(2048, 2, 2)
@@ -138,21 +161,51 @@ static int spec(int argc, char **argv) {
         return 2;
     }
     if (nc == 1024 && nw == 16) {   // two clip groups per CTA, tables in shared memory (the headline kernel's shape)
-        qd_emu::launch(dim3(tiles, (a.batch + 1) / 2, 1), dim3(32 * 16, 1, 1),
-                       qd::SpecSmem<T, 1024, 8, 2>::bytes(qt.n_slots, true, a.q.n_src, 0),
-                       [&] { qd::spec_pass_kernel<T, 1024, 8, true, false, 2>(a); });
+        each(2, [&](int rows) {
+            qd_emu::launch(dim3(tiles, rows, 1), dim3(32 * 16, 1, 1), qd::SpecSmem<T, 1024, 8, 2>::bytes(qt.n_slots, true, a.q.n_src, 0),
+                           [&] { qd::spec_pass_kernel<T, 1024, 8, true, false, 2>(a); });
+        });
+    } else if (nc == 512 && nw == 4 && g_fx) {
+        constexpr int NC = 512, BUF = qd::buf_slots<NC>();
+        std::vector<int16_t> table((size_t)(l.batch + 1) * 2 * a.n_frames * (NC + 1));
+        uint32_t r = 12345;   // source bins of the scramble: any bin 0 .. NC
+        for (int16_t &v : table) { r = r * 1664525u + 1013904223u; v = (int16_t)((r >> 8) % (NC + 1)); }
+        a.fx.mode = 4;
+        a.fx.table = table.data();
+        a.fx.table_frames = a.n_frames;
+        a.fx.table_per_clip = 1;
+        a.fx.clip_offset = 1;
+        std::vector<T> frozen((size_t)l.batch * BUF);
+        qd_emu::launch(dim3(l.batch), dim3(32), (size_t)BUF * sizeof(T2) + (size_t)2 * NC * sizeof(float) + 16,
+                       [&] { qd::freeze_mag_kernel<T, NC>(a, frozen.data()); });
+        a.frozen = frozen.data();
+        each(1, [&](int rows) {
+            qd_emu::launch(dim3(tiles, rows, 1), dim3(32 * 4, 1, 1), qd::SpecSmem<T, NC, 4>::bytes(qt.n_slots, false, 0, 0, true, false),
+                           [&] { qd::spec_pass_kernel<T, NC, 4, false, true>(a); });
+        });
     } else if (nc == 512 && nw == 4) {
-        qd_emu::launch(dim3(tiles, a.batch, 1), dim3(32 * 4, 1, 1), qd::SpecSmem<T, 512, 4>::bytes(qt.n_slots),
-                       [&] { qd::spec_pass_kernel<T, 512, 4>(a); });
+        each(1, [&](int rows) {
+            qd_emu::launch(dim3(tiles, rows, 1), dim3(32 * 4, 1, 1), qd::SpecSmem<T, 512, 4>::bytes(qt.n_slots),
+                           [&] { qd::spec_pass_kernel<T, 512, 4>(a); });
+        });
     } else {
         std::cerr << "no instantiation\n";
         return 2;
     }
-    write_all(argv[12], y);
     return 0;
 }
 
 int main(int argc, char **argv) {
+    for (;;) {
+        const std::string opt = argc > 1 ? argv[1] : "";
+        const int used = opt == "-p" ? 2 : (opt == "-q" || opt == "-x") ? 1 : 0;
+        if (!used) break;
+        if (opt == "-p") g_per_launch = std::atoll(argv[2]);
+        g_quiet_odd |= opt == "-q";
+        g_fx |= opt == "-x";
+        argv += used;
+        argc -= used;
+    }
     const std::string mode = argc > 1 ? argv[1] : "";
     if (mode == "spec" && argc == 13) return std::string(argv[2]) == "f64" ? spec<double>(argc, argv) : spec<float>(argc, argv);
     if (mode == "limiter" && argc == 7) {
@@ -164,7 +217,15 @@ int main(int argc, char **argv) {
         apply(a, l);
         a.limiter_on = 1; a.lookahead = std::atoi(argv[2]); a.ceiling = 0.5; a.c = 0.999;
         a.apply_mix = 0;
-        qd_emu::launch(dim3(l.batch), dim3(qd::QD_TT), qd_host::limiter_smem_bytes(a.lookahead), [&] { qd::limiter_mix_kernel(a); });
+        std::vector<float> peak;   // -q: odd clips quiet (skipped, y = x), even clips loud
+        if (g_quiet_odd) {
+            for (int i = 0; i < l.batch; ++i) peak.push_back(i % 2 ? 0.0f : 1e9f);
+            a.clip_peak = peak.data();
+        }
+        qd::for_each_launch(l.batch, g_per_launch, [&](int clip0, int nb) {
+            a.clip0 = clip0;
+            qd_emu::launch(dim3(nb), dim3(qd::QD_TT), qd_host::limiter_smem_bytes(a.lookahead), [&] { qd::limiter_mix_kernel(a); });
+        });
         write_all(argv[6], y);
         return 0;
     }
@@ -182,7 +243,10 @@ int main(int argc, char **argv) {
         a.halo = std::atoi(argv[6]);
         const long long n_tiles = (a.n + a.tile - 1) / a.tile;
         const unsigned gx = (unsigned)std::max<long long>(1, (n_tiles + 32 * qd::QD_XO_WARPS - 1) / (32 * qd::QD_XO_WARPS));
-        qd_emu::launch(dim3(gx, l.batch, 1), dim3(32 * qd::QD_XO_WARPS), 0, [&] { qd::crossover_kernel(a); });
+        qd::for_each_launch(l.batch, g_per_launch, [&](int clip0, int nb) {
+            a.clip0 = clip0;
+            qd_emu::launch(dim3(gx, nb, 1), dim3(32 * qd::QD_XO_WARPS), 0, [&] { qd::crossover_kernel(a); });
+        });
         write_all(argv[10], lo);
         write_all(argv[11], hi);
         return 0;
