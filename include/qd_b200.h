@@ -260,6 +260,18 @@ int qd_distort_device(const float *x, float *y, int64_t count, int32_t mode, dou
  */
 int qd_spectral_peaks_device(const float *x, int64_t batch, int32_t n_samples, int32_t n_fft, int32_t topn,
                              double min_mag, int32_t precision, int16_t *bins, void *stream);
+/*
+ * The same on a ragged batch, packed as in qd_render_device_varlen: clip c occupies x[starts[c] - starts[0] ... +
+ * lengths[c]) (device arrays, never read on the host; the caller validates them), max_samples is the longest clip and
+ * sizes the grid.  Clip c has T_c = 1 + lengths[c] / hop frames, as alone (hop = n_fft / 4; a zero-length clip has one
+ * frame, all -1), and frame t of clip c is row (starts[c] - starts[0]) / hop + c + t of bins[rows][topn].  Rows of
+ * consecutive clips do not overlap, so span / hop + batch rows hold any batch (span = starts[batch-1] - starts[0] +
+ * lengths[batch-1]); rows no clip owns are not written.  Every clip's bins equal those of the clip alone.
+ */
+int qd_spectral_peaks_device_varlen(const float *x, const int64_t *starts /* device */,
+                                    const int32_t *lengths /* device */, int64_t batch, int32_t max_samples,
+                                    int32_t n_fft, int32_t topn, double min_mag, int32_t precision,
+                                    int16_t *bins, void *stream);
 
 /*
  * quantize_mode = "autotune_v1", the reference's default mode (dsp/autotune.py:426-447 behind dsp/pipeline.py:537-601):

@@ -94,6 +94,7 @@ def load() -> C.CDLL:
     lib.qd_crossover_device.argtypes = [vp, vp, vp, i64, i64, C.POINTER((dbl * 6) * 2), C.POINTER((dbl * 6) * 2), vp]
     lib.qd_distort_device.argtypes = [vp, vp, i64, i32, dbl, dbl, flt, flt, vp]
     lib.qd_spectral_peaks_device.argtypes = [vp, i64, i32, i32, i32, dbl, i32, vp, vp]
+    lib.qd_spectral_peaks_device_varlen.argtypes = [vp, vp, vp, i64, i32, i32, i32, dbl, i32, vp, vp]
     lib.qd_autotune_workspace_bytes.argtypes = [vp, i64]
     lib.qd_autotune_workspace_bytes.restype = C.c_size_t
     lib.qd_autotune_render_device.argtypes = [vp, vp, vp, i64, vp, vp, vp, C.c_size_t, vp]

@@ -57,10 +57,57 @@ def scale_cents_table(freqs: np.ndarray, key: str, scale: str) -> np.ndarray:
     return out
 
 
+def peak_rows(starts, lengths, hop: int) -> Tuple[np.ndarray, np.ndarray, int]:
+    """Rows of a ragged batch in the bins of qd_spectral_peaks_device_varlen (include/qd_b200.h): clip c's
+    T_c = 1 + n_c // hop frames start at row (starts[c] - starts[0]) // hop + c.  Returns (row0, frames, n_rows) with
+    n_rows = span // hop + batch, which holds every clip's rows without overlap."""
+    st = np.asarray(starts, dtype=np.int64).reshape(-1)
+    ln = np.asarray(lengths, dtype=np.int64).reshape(-1)
+    if st.size == 0:
+        return st, ln, 0
+    rel = st - st[0]
+    return rel // hop + np.arange(st.size, dtype=np.int64), 1 + ln // hop, int((rel[-1] + ln[-1]) // hop + st.size)
+
+
+def _ragged_peak_rows(clips, n_fft: int, topn: int, min_db: float, precision: str):
+    """The bins of a list of 1-D clips in one device call: (bins [n_rows, topn] int16 on the device, row0, frames,
+    is_np, cuda), rows as in ``peak_rows``."""
+    from .pipeline import clip_list_kind, pack_clips
+    is_np, cuda = clip_list_kind(clips)   # ValueError before any device check
+    prec = {"float32": 0, "float64": 1}[precision]
+    import torch
+    if not clips:
+        return torch.zeros((0, topn), dtype=torch.int16), np.zeros(0, np.int64), np.zeros(0, np.int64), is_np, cuda
+    if not torch.cuda.is_available():
+        raise _lib.QdError("no CUDA device visible: quantumdistortion_b200 has no CPU fallback")
+    lib = _lib.load()
+    xf, starts, span = pack_clips(clips, cuda)
+    lengths = np.array([int(c.shape[0]) for c in clips], dtype=np.int64)
+    row0, frames, n_rows = peak_rows(starts, lengths, int(n_fft) // 4)
+    xd = xf.cuda(non_blocking=True) if span else torch.zeros(1, device="cuda")   # all clips empty: x is never read
+    d_starts = torch.from_numpy(starts).cuda(non_blocking=True)
+    d_lengths = torch.from_numpy(lengths.astype(np.int32)).cuda(non_blocking=True)
+    bins = torch.empty((n_rows, topn), dtype=torch.int16, device="cuda")
+    _lib.check(lib.qd_spectral_peaks_device_varlen(xd.data_ptr(), d_starts.data_ptr(), d_lengths.data_ptr(), len(clips),
+                                                   int(lengths.max()), int(n_fft), int(topn),
+                                                   float(10.0 ** (min_db / 20.0)), prec, bins.data_ptr(),
+                                                   torch.cuda.current_stream().cuda_stream))
+    return bins, row0, frames, is_np, cuda
+
+
 def spectral_peak_bins(x, n_fft: int = 2048, topn: int = 3, min_db: float = -60.0, precision: str = "float64"):
     """Strongest ``topn`` bins per STFT frame of every clip: x [B, n] (CUDA tensor, CPU tensor or NumPy) ->
-    int16 [B, 1 + n // (n_fft/4), topn] on the same kind of container, -1 where fewer bins reach ``min_db``."""
+    int16 [B, 1 + n // (n_fft/4), topn] on the same kind of container, -1 where fewer bins reach ``min_db``.
+
+    ``x`` may also be a list or tuple of 1-D clips of any lengths: all NumPy arrays, all CPU tensors or all CUDA tensors,
+    each cast to float32.  They are packed into one buffer and run in one call (qd_spectral_peaks_device_varlen); the
+    result is a list of the same kind, clip c's int16 [1 + n_c // (n_fft/4), topn], equal to the clip run alone."""
     import torch
+    if isinstance(x, (list, tuple)):
+        bins, row0, frames, is_np, cuda = _ragged_peak_rows(list(x), n_fft, topn, min_db, precision)
+        if not cuda:
+            bins = bins.cpu().numpy() if is_np else bins.cpu()
+        return [bins[r:r + f] for r, f in zip(row0.tolist(), frames.tolist())]
     if not torch.cuda.is_available():
         raise _lib.QdError("no CUDA device visible: quantumdistortion_b200 has no CPU fallback")
     lib = _lib.load()
@@ -83,23 +130,36 @@ def spectral_peak_bins(x, n_fft: int = 2048, topn: int = 3, min_db: float = -60.
     return bins.cpu().numpy() if is_np else bins.cpu()
 
 
+def _cents_per_clip(bins: np.ndarray, row0: np.ndarray, frames: np.ndarray, table: np.ndarray):
+    """(avgs, per-clip |cents| arrays) from bins [rows, topn], clip c owning rows row0[c] .. + frames[c]: one table
+    lookup over every owned row, then a split by clip."""
+    b = len(row0)
+    owned = np.repeat(row0 - np.cumsum(frames) + frames, frames) + np.arange(int(frames.sum()), dtype=np.int64)
+    flat = bins[owned].reshape(-1)
+    owner = np.repeat(np.arange(b), frames * bins.shape[1])
+    keep = flat >= 0
+    cents = table[flat[keep].astype(np.int64)]
+    owner = owner[keep]
+    fin = np.isfinite(cents)
+    cents, owner = cents[fin].astype(float), owner[fin]
+    per_clip = np.split(cents, np.cumsum(np.bincount(owner, minlength=b))[:-1]) if b else []
+    avgs = np.array([float(np.mean(c)) if c.size else np.nan for c in per_clip], dtype=float)
+    return avgs, per_clip
+
+
 def avg_cents_offset_batch(x, sr: int, key: str, scale: str, frame_length: int = 2048, topn_peaks: int = 3,
                            min_db: float = -60.0, precision: str = "float64") -> Tuple[np.ndarray, List[np.ndarray]]:
     """The metric for every clip of a batch: (avg_abs_cents [B] (NaN for a silent clip), per-clip arrays of
-    per-peak |cents| in the reference's order: frame by frame, strongest bin first)."""
+    per-peak |cents| in the reference's order: frame by frame, strongest bin first).  ``x`` is [B, n] or a list of
+    1-D clips of any lengths (see ``spectral_peak_bins``); each clip gets the values it gets alone."""
+    table = scale_cents_table(np.fft.rfftfreq(frame_length, d=1.0 / sr), key, scale)
+    if isinstance(x, (list, tuple)):
+        bins, row0, frames, _, _ = _ragged_peak_rows(list(x), frame_length, topn_peaks, min_db, precision)
+        return _cents_per_clip(bins.cpu().numpy(), row0, frames, table)
     bins = spectral_peak_bins(x, n_fft=frame_length, topn=topn_peaks, min_db=min_db, precision=precision)
     bins = bins.cpu().numpy() if hasattr(bins, "cpu") else np.asarray(bins)
-    table = scale_cents_table(np.fft.rfftfreq(frame_length, d=1.0 / sr), key, scale)
-    avgs = np.full(bins.shape[0], np.nan)
-    per_clip: List[np.ndarray] = []
-    for i in range(bins.shape[0]):
-        flat = bins[i].reshape(-1)
-        c = table[flat[flat >= 0]]
-        c = c[np.isfinite(c)]
-        per_clip.append(c.astype(float))
-        if c.size:
-            avgs[i] = float(np.mean(c))
-    return avgs, per_clip
+    b, t = bins.shape[0], bins.shape[1]
+    return _cents_per_clip(bins.reshape(b * t, bins.shape[2]), np.arange(b, dtype=np.int64) * t, np.full(b, t, np.int64), table)
 
 
 def avg_cents_offset_from_scale(audio: np.ndarray, sr: int, key: str, scale: str, frame_length: int = 2048,

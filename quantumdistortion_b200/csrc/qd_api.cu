@@ -355,8 +355,8 @@ int launch_peaks_t(qd::PeaksArgsT<T> a, int64_t batch, cudaStream_t st) {
     static std::atomic<uint64_t> attr_mask{0};  // devices this instantiation was opted in on
     auto kern = qd::peaks_kernel<T, NC>;
     if (int rc_ = ensure_dyn_smem(kern, attr_mask, 227 * 1024)) return rc_;
-    const size_t per_warp = (size_t)qd::buf_slots<NC>() * sizeof(qd::V2<T>) + (size_t)2 * NC * sizeof(float);
-    const int nw = (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / per_warp));
+    constexpr size_t per_warp = qd::peaks_warp_smem<T, NC>();
+    constexpr int nw = qd::peaks_warps<T, NC>();
     const unsigned gx = (unsigned)((a.n_frames + nw - 1) / nw);
     qd::for_each_launch(batch, qd::QD_GRID_Y_MAX, [&](int clip0, int nb) {
         qd::PeaksArgsT<T> c = a;
@@ -367,15 +367,17 @@ int launch_peaks_t(qd::PeaksArgsT<T> a, int64_t batch, cudaStream_t st) {
     return QD_OK;
 }
 
+// Uniform batches pass null starts / lengths (n = the clip length); ragged ones their device arrays (n = the longest clip).
 template <class T>
-int launch_peaks(const float *x, int64_t batch, int n, int n_fft, int topn, double min_mag, int16_t *bins, cudaStream_t st) {
+int launch_peaks(const float *x, const int64_t *starts, const int32_t *lengths, int64_t batch, int n, int n_fft, int topn,
+                 double min_mag, int16_t *bins, cudaStream_t st) {
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) { cudaGetLastError(); return fail(QD_ERR_NO_DEVICE, "no CUDA device: libqd_b200 has no CPU path"); }
     PeakTables pt;
     int rc = peak_tables<T>(dev, n_fft, &pt);
     if (rc != QD_OK) return rc;
     qd::PeaksArgsT<T> a{};
-    a.x = x; a.bins = bins; a.n = n; a.topn = topn;
+    a.x = x; a.bins = bins; a.starts = starts; a.lengths = lengths; a.n = n; a.topn = topn;
     a.n_frames = 1 + n / (n_fft / 4);
     a.min_mag2 = (T)(min_mag * min_mag);
     a.wtab = reinterpret_cast<const qd::V2<T> *>(pt.wtab);
@@ -417,9 +419,22 @@ int qd_spectral_peaks_device(const float *x, int64_t batch, int32_t n_samples, i
     if (topn < 1 || topn > qd::QD_PEAKS_MAX) return fail(QD_ERR_INVALID_ARG, "topn must be 1..8");
     if (batch == 0) return QD_OK;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    if (precision == QD_PRECISION_F64) return launch_peaks<double>(x, batch, n_samples, n_fft, topn, min_mag, bins, st);
-    if (precision == QD_PRECISION_F32) return launch_peaks<float>(x, batch, n_samples, n_fft, topn, min_mag, bins, st);
+    if (precision == QD_PRECISION_F64) return launch_peaks<double>(x, nullptr, nullptr, batch, n_samples, n_fft, topn, min_mag, bins, st);
+    if (precision == QD_PRECISION_F32) return launch_peaks<float>(x, nullptr, nullptr, batch, n_samples, n_fft, topn, min_mag, bins, st);
     return fail(QD_ERR_INVALID_ARG, "bad precision");
+}
+
+int qd_spectral_peaks_device_varlen(const float *x, const int64_t *starts, const int32_t *lengths, int64_t batch,
+                                    int32_t max_samples, int32_t n_fft, int32_t topn, double min_mag, int32_t precision,
+                                    int16_t *bins, void *stream) {
+    if (!x || !starts || !lengths || !bins || batch < 0 || max_samples < 0) return fail(QD_ERR_INVALID_ARG, "null / negative argument");
+    if (batch > INT32_MAX) return fail(QD_ERR_INVALID_ARG, "batch of more than 2^31 - 1 clips");
+    if (topn < 1 || topn > qd::QD_PEAKS_MAX) return fail(QD_ERR_INVALID_ARG, "topn must be 1..8");
+    if (precision != QD_PRECISION_F64 && precision != QD_PRECISION_F32) return fail(QD_ERR_INVALID_ARG, "bad precision");
+    if (batch == 0) return QD_OK;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    if (precision == QD_PRECISION_F64) return launch_peaks<double>(x, starts, lengths, batch, max_samples, n_fft, topn, min_mag, bins, st);
+    return launch_peaks<float>(x, starts, lengths, batch, max_samples, n_fft, topn, min_mag, bins, st);
 }
 
 int qd_plan_create(const qd_params *params, const qd_tables *tables, qd_plan **out) {

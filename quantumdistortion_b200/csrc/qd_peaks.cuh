@@ -18,14 +18,29 @@ constexpr int QD_PEAKS_MAX = 8;
 
 template <class T>
 struct PeaksArgsT {
-    const float *x;       // [batch, n]
-    int16_t *bins;        // [batch, n_frames, topn]: bin index, -1 = no (further) bin above the threshold
-    int n, n_frames, topn;
+    const float *x;       // uniform: [batch, n]; ragged: packed, clip c at starts[c] - starts[0] (clip_loc)
+    int16_t *bins;        // rows of topn bin indices, -1 = no (further) bin above the threshold (see peaks_kernel)
+    const int64_t *starts;   // ragged batch: per-clip sample offsets and lengths; null = uniform
+    const int32_t *lengths;
+    int n, n_frames, topn;   // n: the clip length (uniform) or the longest clip (ragged); n_frames = 1 + n / hop
     int clip0;            // clip of blockIdx.y == 0 (launch splits advance it, see for_each_launch)
     T min_mag2;           // (10^(min_db/20))^2
     const V2<T> *wtab, *tw1, *tw2, *wsplit;
 };
 
+// Launch geometry: one warp per frame, as many warps per CTA (<= 8) as 200 KB of shared memory hold.
+template <class T, int NC>
+__host__ __device__ constexpr size_t peaks_warp_smem() { return (size_t)buf_slots<NC>() * sizeof(V2<T>) + (size_t)2 * NC * sizeof(float); }
+template <class T, int NC>
+__host__ __device__ constexpr int peaks_warps() {
+    constexpr size_t fit = (200 * 1024) / peaks_warp_smem<T, NC>();
+    return fit >= 8 ? 8 : fit < 1 ? 1 : (int)fit;
+}
+
+// Grid: x covers the frames of the longest clip, y the clips.  Clip c has its own T_c = 1 + n_c / hop frames (hop =
+// n_fft / 4 = NC / 2), the frame count it has alone; warps past it exit.  Output rows: uniform batches put frame t of
+// clip c at row c * n_frames + t; ragged batches at (starts[c] - starts[0]) / hop + c + t, the rule of at_row0 (no
+// scan, valid for sub-ranges, consecutive clips cannot overlap), so span / hop + batch rows hold any ragged batch.
 template <class T, int NC>
 __global__ void __launch_bounds__(256)
 peaks_kernel(const PeaksArgsT<T> a) {
@@ -33,17 +48,18 @@ peaks_kernel(const PeaksArgsT<T> a) {
     constexpr int ROWS = (NC + 1 + 31) / 32;
     QD_DYN_SMEM(smem);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-    const size_t per_warp = (size_t)BUF * sizeof(V2<T>) + (size_t)2 * NC * sizeof(float);
+    constexpr size_t per_warp = peaks_warp_smem<T, NC>();
     V2<T> *buf = reinterpret_cast<V2<T> *>(smem + (size_t)warp * per_warp);
     float *stage = reinterpret_cast<float *>(smem + (size_t)warp * per_warp + (size_t)BUF * sizeof(V2<T>));
-    const int clip = a.clip0 + (int)blockIdx.y;
+    constexpr int HOP = NC / 2;
+    const ClipLoc c = clip_loc(a, (int)blockIdx.y);
     const int t = blockIdx.x * nw + warp;
-    if (t >= a.n_frames) return;
-    const float *x = a.x + (size_t)clip * a.n;
-    const long long s0 = (long long)t * (NC / 2) - NC;   // centre padding of n_fft/2 (dsp/stft_utils.py:59-62)
+    if (t > c.n / HOP) return;
+    const float *x = a.x + c.base;
+    const long long s0 = (long long)t * HOP - NC;   // centre padding of n_fft/2 (dsp/stft_utils.py:59-62)
     for (int i = lane; i < 2 * NC; i += 32) {
         const long long s = s0 + i;
-        stage[i] = (s >= 0 && s < a.n) ? x[s] : 0.0f;
+        stage[i] = (s >= 0 && s < c.n) ? x[s] : 0.0f;   // outside the clip: zeros, as alone; gaps are never read
     }
     __syncwarp();
     SpecArgsT<T> sa{};
@@ -72,7 +88,8 @@ peaks_kernel(const PeaksArgsT<T> a) {
             }
         }
     }
-    int16_t *out = a.bins + ((size_t)clip * a.n_frames + t) * a.topn;
+    const long long row = (a.starts ? c.base / HOP + c.idx : (long long)c.idx * a.n_frames) + t;
+    int16_t *out = a.bins + row * a.topn;
     for (int r = 0; r < a.topn; ++r) {
         T best = bv[0];
         int bidx = bi[0] >= 0 ? bi[0] : 0x7fffffff;

@@ -133,6 +133,48 @@ def pack_layout(lengths: Sequence[int], itemsize: int = 4) -> Tuple[np.ndarray, 
     return starts, int(starts[-1] + n[-1])
 
 
+def clip_list_kind(clips: Sequence[Any]) -> Tuple[bool, bool]:
+    """(is_numpy, on_cuda) of a list of 1-D clips: all NumPy arrays, all CPU tensors or all CUDA tensors; anything else
+    raises ValueError.  Needs no device."""
+    import torch
+    if all(isinstance(c, np.ndarray) for c in clips):
+        is_np, cuda = True, False
+    elif all(isinstance(c, torch.Tensor) for c in clips):
+        is_np, cuda = False, bool(clips and clips[0].is_cuda)
+        if any(bool(c.is_cuda) != cuda for c in clips):
+            raise ValueError("a list of clips must be all CUDA or all CPU tensors")
+    else:
+        raise ValueError("a list of clips must be all NumPy arrays or all tensors")
+    if any(c.ndim != 1 for c in clips):
+        raise ValueError("a list of clips holds 1-D (mono) clips")
+    return is_np, cuda
+
+
+def pack_clips(clips: Sequence[Any], cuda: bool, pcm: bool = False):
+    """One buffer holding the clips in the ``pack_layout`` layout, zero in the gaps: CUDA clips with one concatenation on
+    the device (cast to float32), host clips copied once into page-locked memory (float32, or int16 for PCM16), which
+    is the H2D staging.  Returns (buffer, starts, span); at least one clip."""
+    torch = _torch()
+    lengths = np.array([int(c.shape[0]) for c in clips], dtype=np.int64)
+    starts, span = pack_layout(lengths, 2 if pcm else 4)
+    ends = starts + lengths
+    if cuda:   # one concatenation on the device: clips and the zero gaps that align the next start
+        zero = torch.zeros(4, dtype=torch.float32, device="cuda")
+        pieces = []
+        for k, c in enumerate(clips):
+            pieces.append(c.float())
+            if k + 1 < len(clips) and starts[k + 1] > ends[k]:
+                pieces.append(zero[:int(starts[k + 1] - ends[k])])
+        return torch.cat(pieces), starts, span
+    xf = torch.empty(span, dtype=torch.int16 if pcm else torch.float32, pin_memory=True)
+    xn = xf.numpy()
+    for k, c in enumerate(clips):
+        xn[starts[k]:ends[k]] = c if isinstance(c, np.ndarray) else c.numpy()
+        if k + 1 < len(clips):
+            xn[ends[k]:starts[k + 1]] = 0
+    return xf, starts, span
+
+
 def check_layout(starts, lengths, max_samples: int) -> None:
     """The rules of qd_render_*_varlen (include/qd_b200.h) on host arrays: starts non-decreasing, clips not
     overlapping, 0 <= length <= max_samples.  Raises ValueError; the device entry point does not check them."""
@@ -567,16 +609,7 @@ def make_renderer(n_samples: int, sr: int = DEFAULT_SAMPLE_RATE, n_fft: int = N_
 def _ragged_batch(clips: List[Any], sr: int, n_fft: int, return_taps: bool, chunk_clips: int, seeds, kwargs):
     """process_batch on a list of 1-D clips of any lengths (see there)."""
     torch = _torch()
-    if all(isinstance(c, np.ndarray) for c in clips):
-        is_np, cuda = True, False
-    elif all(isinstance(c, torch.Tensor) for c in clips):
-        is_np, cuda = False, bool(clips and clips[0].is_cuda)
-        if any(bool(c.is_cuda) != cuda for c in clips):
-            raise ValueError("a list of clips must be all CUDA or all CPU tensors")
-    else:
-        raise ValueError("a list of clips must be all NumPy arrays or all tensors")
-    if any(c.ndim != 1 for c in clips):
-        raise ValueError("a list of clips holds 1-D (mono) clips")
+    is_np, cuda = clip_list_kind(clips)
     pcm_of = (lambda c: c.dtype == np.int16) if is_np else (lambda c: c.dtype == torch.int16)  # noqa: E731
     pcm = bool(clips) and pcm_of(clips[0])
     if any(pcm_of(c) != pcm for c in clips):
@@ -607,24 +640,9 @@ def _ragged_batch(clips: List[Any], sr: int, n_fft: int, return_taps: bool, chun
         hop = int(n_fft) // 4
         r.set_fx_seeds(len(live), [seeds[i] for i in live] if isinstance(seeds, list) else seeds,
                        frames=[1 + int(n) // hop for n in n_live])
-        starts, span = pack_layout(n_live, 2 if pcm else 4)
+        xf, starts, span = pack_clips([clips[i] for i in live], cuda, pcm)
         max_n = int(n_live.max())
         ends = starts + n_live
-        if cuda:   # one concatenation on the device: clips and the zero gaps that align the next start
-            zero = torch.zeros(4, dtype=torch.float32, device="cuda")
-            pieces = []
-            for k, i in enumerate(live):
-                pieces.append(clips[i].float())
-                if k + 1 < len(live) and starts[k + 1] > ends[k]:
-                    pieces.append(zero[:int(starts[k + 1] - ends[k])])
-            xf = torch.cat(pieces)
-        else:      # packed once into page-locked memory: this copy is the H2D staging
-            xf = torch.empty(span, dtype=torch.int16 if pcm else torch.float32, pin_memory=True)
-            xn = xf.numpy()
-            for k, i in enumerate(live):
-                xn[starts[k]:ends[k]] = clips[i] if is_np else clips[i].numpy()
-                if k + 1 < len(live):
-                    xn[ends[k]:starts[k + 1]] = 0
         if cuda or return_taps:
             d_starts = torch.from_numpy(starts).cuda()
             d_lengths = torch.from_numpy(n_live.astype(np.int32)).cuda()
