@@ -205,7 +205,6 @@ QD_DEV V2<T> hann_pair(V2<T> wc, V2<T> ws, int q) {
 // the others are products w_k = w_{k - lowbit(k)} w_{lowbit(k)} (at most log2(R) - 1 multiplications deep), because the
 // pass is bound by shared-memory wavefronts, not by arithmetic.  `cur[j]` = latest w whose index has >= j trailing zeros.
 template <int K> struct KConst { static constexpr int value = K; };
-template <bool B> struct KBool { static constexpr bool value = B; };
 template <class T, int R, int K, class F>
 QD_DEV void twiddle_step(const V2<T> (&pw)[qd_log2(R)], V2<T> (&cur)[qd_log2(R) + 1], F &body) {
     if constexpr (K < R) {
@@ -976,34 +975,30 @@ struct SpecSmem {
     }
 };
 
+// the wavefold in float32 arithmetic: exact when bias == 0 and fold is a power of two (see epilogue_apply)
+QD_DEV float wavefold_f32(float v, float fold) {
+    float y = v * fold;
+    if (y > 1.0f) y = 2.0f - y;
+    if (y < -1.0f) y = -2.0f - y;
+    return fminf(fmaxf(y, -1.0f), 1.0f);
+}
+
 // wavefold / tube on the float32 iSTFT sample (dsp/distortion.py:18-90)
-// EF ("epilogue float"): the caller guarantees that the epilogue is none or a wavefold that is exact in float32 (no
-// bias, power-of-two gain -- the reference defaults); no tanh either.  The float64 branch below is only a dozen instructions, but the overlap-add loop
-// around it is unrolled NW + 3 times in the headline kernel, whose code already fills the instruction cache: with the
-// branch compiled in, that kernel ran 3 % slower even though the branch was never taken (measured, A/B on one box).
-template <bool EF>
 QD_DEV float epilogue_apply(float v, int mode, double fold, double bias, int exact_f32, float tg, float tn) {
     if (mode == 1) {
         // dsp/distortion.py:37-58 computes in float64 and rounds to float32 once; the negative fold is tested on the
         // already folded value (:44-56).  (x + bias) * fold reaches several units before it is folded back, so float32
         // arithmetic would carry the rounding error of the large intermediate (~2e-7) into the small result -- and the
         // second spectral pass amplifies its input error.  With bias == 0 and fold a power of two float32 is exact.
-        if constexpr (!EF) {
-            if (!exact_f32) {
-                double y = ((double)v + bias) * fold;
-                if (y > 1.0) y = 2.0 - y;
-                if (y < -1.0) y = -2.0 - y;
-                return (float)fmin(fmax(y, -1.0), 1.0);
-            }
+        if (!exact_f32) {
+            double y = ((double)v + bias) * fold;
+            if (y > 1.0) y = 2.0 - y;
+            if (y < -1.0) y = -2.0 - y;
+            return (float)fmin(fmax(y, -1.0), 1.0);
         }
-        float y = v * (float)fold;
-        if (y > 1.0f) y = 2.0f - y;
-        if (y < -1.0f) y = -2.0f - y;
-        return fminf(fmaxf(y, -1.0f), 1.0f);
+        return wavefold_f32(v, (float)fold);
     }
-    if constexpr (!EF) {
-        if (mode == 2) return tanhf(tg * v) * tn;
-    }
+    if (mode == 2) return tanhf(tg * v) * tn;
     return v;
 }
 
@@ -1196,20 +1191,52 @@ spec_pass_kernel(const SpecArgsT<T> a) {
         group_sync<NG, 32 * NW>(grp);
         // ---- overlap-add in frame order; blocks tb .. tb+NW-1 are now complete.  A thread owns one
         //      column of sample pairs: slice sl of warp w's frame sits at bufs[w][sl*HPP + pidx(c)].
-        //      The hop loop is unrolled only in the EF kernel (small epilogue): elsewhere NW + 3 copies of the store path
-        //      cost more instruction-cache misses than the loop overhead they save.
+        // An interior batch: every output hop j = tb .. tb+NW-1 lies in [j0, j1) and is covered by four frames of the
+        // clip (3 <= j <= n_frames - 1), so each takes row (0,3) of invw and ends inside the clip (hop j ends at sample
+        // (j-1)*HOP - 1 < (n_frames-1)*HOP <= n).  The same for the whole group; all batches of a clip but the first and
+        // the last one or two are interior.
+        const bool interior = tb >= 3 && tb >= j0 && tb + NW <= j1 && tb + NW <= n_frames;
         for (int c = tid; c < HP; c += nthreads) {
             const int pc = pidx(c);
-            // one output hop of this thread's column; FAST = float32-only epilogue, 8-byte stores, no tap
-            auto hop = [&](int h, auto fast_tag) {
-                constexpr bool FAST = decltype(fast_tag)::value;
-                V2<T> v = (h < 3) ? tail[h * HP + c] : mk2<T>(0.0f, 0.0f);   // partial sums carried from the last batch
+            // partial sum of hop h of this column: the sums carried from the last batch, then the frames in frame order
+            auto ola = [&](int h) {
+                V2<T> v = (h < 3) ? tail[h * HP + c] : mk2<T>(0.0f, 0.0f);
                 const int w0 = h - 3 > 0 ? h - 3 : 0, w1 = h < NW - 1 ? h : NW - 1;
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
                     const int w = w0 + k;
                     if (w <= w1) v = padd(v, bufs[(size_t)w * L::BUF + (h - w) * HPP + pc]);
                 }
+                return v;
+            };
+            if constexpr (EF) {
+                // EF ("epilogue float"): the caller guarantees that the epilogue is none or a wavefold that is exact
+                // in float32 (no bias, power-of-two gain -- the reference defaults).  On an interior batch with 8-byte
+                // stores and no tap, the hops of a column differ only by constant offsets: one base pointer, one
+                // 1/sum(w^2) pair, one fold factor and one epilogue test per column, and the hop loop unrolled.
+                if (interior && vec2 && !tap) {
+                    float2 *yc = reinterpret_cast<float2 *>(y + (tb - 2) * HOP) + c;
+                    const float2 inv = __ldg(reinterpret_cast<const float2 *>(a.invw + 3 * HOP) + c);   // row (0,3)
+                    const bool fold = a.epilogue == 1;
+                    const float fk = (float)a.fold;
+#pragma unroll
+                    for (int h = 0; h < NW + 3; ++h) {
+                        const float2 v = ola(h);
+                        if (h >= NW) {
+                            tail[(h - NW) * HP + c] = v;   // see the general hop below
+                            continue;
+                        }
+                        const float2 o = pmul(v, inv);
+                        const float2 r = fold ? make_float2(wavefold_f32(o.x, fk), wavefold_f32(o.y, fk)) : o;
+                        yc[h * HP] = r;
+                        out_peak = fmaxf(out_peak, fmaxf(fabsf(r.x), fabsf(r.y)));
+                    }
+                    continue;
+                }
+            }
+            // one output hop of this thread's column, any batch and epilogue
+            auto hop = [&](int h) {
+                const V2<T> v = ola(h);
                 if (h >= NW) {
                     tail[(h - NW) * HP + c] = v;  // partial sums of the next three blocks (slot h - NW < h: already read)
                     return;
@@ -1225,10 +1252,10 @@ spec_pass_kernel(const SpecArgsT<T> a) {
                 if (sl_a <= sl_b) inv = __ldg(reinterpret_cast<const V2<T> *>(a.invw + (sl_a * 4 + sl_b) * HOP) + c);
                 const V2<T> vi = pmul(v, inv);
                 const float2 o = make_float2((float)vi.x, (float)vi.y);  // float32 like istft_mono
-                const float2 r = make_float2(epilogue_apply<FAST>(o.x, a.epilogue, a.fold, a.bias, a.fold_exact_f32, a.tube_gain, a.tube_norm),
-                                             epilogue_apply<FAST>(o.y, a.epilogue, a.fold, a.bias, a.fold_exact_f32, a.tube_gain, a.tube_norm));
-                if (FAST || vec2) {  // nidx is even and n is even, so nidx + 1 < n
-                    if (!FAST && tap) *reinterpret_cast<float2 *>(tap + nidx) = o;
+                const float2 r = make_float2(epilogue_apply(o.x, a.epilogue, a.fold, a.bias, a.fold_exact_f32, a.tube_gain, a.tube_norm),
+                                             epilogue_apply(o.y, a.epilogue, a.fold, a.bias, a.fold_exact_f32, a.tube_gain, a.tube_norm));
+                if (vec2) {  // nidx is even and n is even, so nidx + 1 < n
+                    if (tap) *reinterpret_cast<float2 *>(tap + nidx) = o;
                     *reinterpret_cast<float2 *>(y + nidx) = r;
                     out_peak = fmaxf(out_peak, fmaxf(fabsf(r.x), fabsf(r.y)));
                 } else {
@@ -1242,17 +1269,12 @@ spec_pass_kernel(const SpecArgsT<T> a) {
                     }
                 }
             };
-            // The kernel's code fills the instruction cache, so only the EF kernel unrolls the hop loop, and only with
-            // the compact hop (no tanh, no float64, no scalar stores, no tap: the reference defaults on aligned clips);
-            // every other case runs the general hop in a rolled loop -- NW + 3 copies of it cost more in instruction
-            // fetch than the loop overhead they save (measured: 60.1 -> 56.2 ms per render of 4096 clips).
-            if (EF && vec2 && !tap) {
-#pragma unroll
-                for (int h = 0; h < NW + 3; ++h) hop(h, KBool<EF>{});
-            } else {
+            // The kernel's code fills the instruction cache, so only the EF kernel unrolls a hop loop, the compact one
+            // of interior batches above; every other case runs the general hop in a rolled loop -- NW + 3 copies of it
+            // cost more in instruction fetch than the loop overhead they save (measured: 60.1 -> 56.2 ms per render
+            // of 4096 clips).
 #pragma unroll 1
-                for (int h = 0; h < NW + 3; ++h) hop(h, KBool<false>{});
-            }
+            for (int h = 0; h < NW + 3; ++h) hop(h);
         }
         group_sync<NG, 32 * NW>(grp);
     }

@@ -526,8 +526,8 @@ spec_pass_team_kernel(const SpecArgsT<T> a, const TeamGather tg) {
                 if (sl_a <= sl_b) inv = __ldg(reinterpret_cast<const V2<T> *>(a.invw + (sl_a * 4 + sl_b) * HOP) + c);
                 const V2<T> vi = pmul(v, inv);
                 const float2 o = make_float2((float)vi.x, (float)vi.y);
-                const float2 r = make_float2(epilogue_apply<false>(o.x, a.epilogue, a.fold, a.bias, a.fold_exact_f32, a.tube_gain, a.tube_norm),
-                                             epilogue_apply<false>(o.y, a.epilogue, a.fold, a.bias, a.fold_exact_f32, a.tube_gain, a.tube_norm));
+                const float2 r = make_float2(epilogue_apply(o.x, a.epilogue, a.fold, a.bias, a.fold_exact_f32, a.tube_gain, a.tube_norm),
+                                             epilogue_apply(o.y, a.epilogue, a.fold, a.bias, a.fold_exact_f32, a.tube_gain, a.tube_norm));
                 if (vec2) {
                     if (tap) *reinterpret_cast<float2 *>(tap + nidx) = o;
                     *reinterpret_cast<float2 *>(y + nidx) = r;
